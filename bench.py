@@ -2,6 +2,7 @@
 """bench.py -- bzip2 level-9 compress throughput (BASELINE.json metric) on N B200s.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--level 9] [--mb 100] [--mode compress|decompress]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" = one pass of the hot path (Bzip2.compressFile at level 9) over one 100 MB batch of synthetic enwik8-like text
@@ -21,6 +22,11 @@ scaling, no collective on the data path -- per-shard scalars travel through shar
 
 --impl reference times that CPU port with all host threads on the same config/metric.
 --mode decompress makes decompression the headline value of the line (compress figures are then reported alongside).
+--dump-outputs DIR writes what the last timed device-resident compress and decompress steps produced (one process only):
+  compress_stream.npy / decompress_output.npy   the bytes as float32: all of them up to 4 Mi bytes, else the bytes at
+                                                4 Mi sorted positions drawn with seed 0 from the output's length
+  compress_stream_len.npy / decompress_output_len.npy   the output length in bytes (float64)
+The inputs are seeded, so two builds run with the same arguments can be compared file by file.
 """
 import argparse
 import ctypes
@@ -36,8 +42,10 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
+sys.dont_write_bytecode = True   # the benchmark leaves the tree it runs from untouched (it may be read-only)
 
 UNIT = "MB/s"
+DUMP_VALUES = 4 << 20   # bytes kept per dumped output: 16 MiB as float32, 32 MiB for the two outputs
 
 
 def metric_name(level, mode):
@@ -177,6 +185,19 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
+def dump_output(out_dir, name, d_bytes):
+    """a uint8 device tensor as out_dir/<name>.npy (float32, the seeded sample described in the module docstring) and its
+    length as out_dir/<name>_len.npy"""
+    import numpy as np
+    import torch
+    n = d_bytes.numel()
+    if n > DUMP_VALUES:
+        idx = np.sort(np.random.default_rng(0).integers(0, n, DUMP_VALUES))
+        d_bytes = d_bytes[torch.from_numpy(idx).to(d_bytes.device)]
+    np.save(os.path.join(out_dir, name + ".npy"), d_bytes.cpu().numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, name + "_len.npy"), np.array([n], dtype=np.float64))
+
+
 def gen_range(lo, hi, seed=8):
     """bytes [lo, hi) of the synthetic corpus (chunks of 1 MB are generated independently)"""
     from compressjs_flattened_b200.corpus import CHUNK, gen_text
@@ -204,7 +225,12 @@ def main():
     ap.add_argument("--lanes", type=int, default=1, help="lanes per rank of the N>1 host-call leg (measured best at 8 ranks: 1, plan [25, 75] MB)")
     ap.add_argument("--plan-first-mb", type=float, default=0.0)
     ap.add_argument("--plan-growth", type=float, default=0.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed steps to DIR (see above)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs: the b200 implementation in one process only")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -293,6 +319,9 @@ def main():
     wall_ms = (t1 - t0) * 1e3
     clocks = sampler.stop(t0, t1) if rank == 0 else None
     st_last = eng.stats()
+    if args.dump_outputs:   # before anything else writes d_out
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        dump_output(args.dump_outputs, "compress_stream", d_out[:out_len])
 
     if args.profile_only:
         print(json.dumps({"profile_only": True, "ms_per_step": round(dev_ms / args.steps, 3), "launches_per_step": launches // args.steps}), flush=True)
@@ -400,7 +429,7 @@ def main():
         out_len = eng.compress_device(d_in[0].data_ptr(), nbytes, level, d_out.data_ptr(), d_out.numel())
 
     # ---------------- decompress ----------------
-    dec_steps = max(1, min(args.steps, 5))
+    dec_steps = args.steps
     dec = {}
     if world == 1:
         last_in = (args.steps - 1) % 2
@@ -414,6 +443,8 @@ def main():
             got = eng.decompress_device(comp.data_ptr(), out_len, False, d_back.data_ptr(), d_back.numel())
             dec_ms += eng.stats().ms_total
         roundtrip_ok = bool(got == nbytes and torch.equal(d_back[:nbytes], d_in[last_in][:nbytes]))
+        if args.dump_outputs:
+            dump_output(args.dump_outputs, "decompress_output", d_back[:got])
         comp_host = comp.cpu().pin_memory()
         def dec_host():
             rc = L.bz2b200_decompress(eng._ctx, comp_host.data_ptr(), out_len, 0, ctypes.byref(out_p), ctypes.byref(out_n))
