@@ -7,9 +7,13 @@
   -d  decompress the FIRST stream of the input, stream flavour (bz2b200_dstream_*); --multistream decodes all of them
       (an extension: the reference's command line never passes the flag, NPM/bin/compressjs:166)
   -b  with -d: extract the single block whose signature starts at bit <bits> (Bzip2.decompressBlock)
+  --recover  write what survives of a damaged file (every block that decodes and matches its CRC, all streams); one line per
+      damaged region on stderr; exit status 0 when everything was intact, 2 when anything was lost
 If <infile> is omitted, reads from stdin; if <outfile> is omitted, writes to stdout.  Needs a CUDA device: no CPU fallback."""
 import argparse
 import sys
+
+from .bzip2 import NO_SIGNATURE, Err
 
 
 def main(argv=None, engine=None):
@@ -26,7 +30,19 @@ def main(argv=None, engine=None):
                         help="Fastest/largest compression" if lv == 1 else "Slowest/smallest compression" if lv == 9 else argparse.SUPPRESS)
     ap.add_argument("infile", nargs="?", default=None)
     ap.add_argument("outfile", nargs="?", default=None)
+    ap.add_argument("--recover", action="store_true", help="write the intact blocks of a damaged file, report the damage")
     a = ap.parse_args(argv)
+    if a.recover:
+        if a.compress:
+            print("--recover can only be used without -z", file=sys.stderr)
+            return 1
+        if a.block >= 0:
+            print("--recover and --block can't be used together", file=sys.stderr)
+            return 1
+        if any(getattr(a, f"l{lv}") for lv in range(1, 10)):
+            print("Compression level has no effect when recovering.", file=sys.stderr)
+            return 1
+        a.decompress = True
     if not a.decompress:
         a.compress = True
     if a.decompress and a.compress:
@@ -54,8 +70,18 @@ def main(argv=None, engine=None):
     Bzip2 = engine
     src = open(a.infile, "rb") if a.infile else sys.stdin.buffer
     dst = open(a.outfile, "wb") if a.outfile else sys.stdout.buffer
+    status = 0
     try:
-        if a.decompress and a.block >= 0:
+        if a.recover:
+            data, regions = Bzip2.recover(src.read())
+            dst.write(data)
+            names = {v: k for k, v in vars(Err).items() if isinstance(v, int)}
+            for r in regions:
+                if r.status:
+                    sig = " (no signature)" if r.flags & NO_SIGNATURE else ""
+                    print(f"bits {r.bit_begin}-{r.bit_end}: {r.kind_name}{sig} {names.get(r.status, r.status)}", file=sys.stderr)
+                    status = 2
+        elif a.decompress and a.block >= 0:
             dst.write(Bzip2.decompressBlock(src.read(), a.block))
         elif a.decompress:
             Bzip2.decompressStream(src, dst, a.multistream)
@@ -68,7 +94,7 @@ def main(argv=None, engine=None):
             dst.close()
         else:
             dst.flush()
-    return 0
+    return status
 
 
 if __name__ == "__main__":

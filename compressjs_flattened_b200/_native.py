@@ -50,6 +50,11 @@ class RangeResult(C.Structure):
     _fields_ = [("part", C.POINTER(C.c_uint8)), ("bytes", C.c_uint64), ("out_offset", C.c_uint64), ("rc", C.c_int32), ("n_blocks", C.c_uint32)]
 
 
+class Region(C.Structure):
+    _fields_ = [("bit_begin", C.c_uint64), ("bit_end", C.c_uint64), ("out_offset", C.c_uint64), ("out_bytes", C.c_uint32),
+                ("crc", C.c_uint32), ("status", C.c_int32), ("kind", C.c_uint32), ("stream", C.c_uint32), ("flags", C.c_uint32)]
+
+
 def take_bytes(ptr, n):
     """n bytes at a ctypes pointer as a bytes object (ctypes.string_at takes an int-sized length: streams above 2 GiB)"""
     if not n:
@@ -78,6 +83,7 @@ class Library:
         L.bz2b200_decompress_block.argtypes = [vp, vp, C.c_size_t, C.c_uint64, u8pp, szp]
         L.bz2b200_table.argtypes = [vp, vp, C.c_size_t, C.c_int, C.POINTER(C.POINTER(C.c_uint64)),
                                     C.POINTER(C.POINTER(C.c_uint32)), szp]
+        L.bz2b200_recover.argtypes = [vp, vp, C.c_size_t, u8pp, szp, C.POINTER(C.POINTER(Region)), szp]
         L.bz2b200_free.argtypes = [vp]
         L.bz2b200_free.restype = None
         L.bz2b200_compress_device.argtypes = [vp, vp, C.c_size_t, C.c_int, vp, C.c_size_t, szp]

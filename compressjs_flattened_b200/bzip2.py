@@ -18,6 +18,7 @@ Errors: `Bzip2Error` (a TypeError, like the JS `_throw`, BJ:1384-1391) carrying 
 a bad level raises ValueError('Invalid block size multiplier') (JS: Error, BJ:2208).
 """
 import ctypes as C
+from collections import namedtuple
 
 import numpy as np
 
@@ -42,6 +43,15 @@ class Err:  # BJ:1365-1375
     OUT_OF_MEMORY = -6
     OBSOLETE_INPUT = -7
     END_OF_BLOCK = -8
+
+
+REGION_HEADER, REGION_BLOCK, REGION_END, REGION_UNKNOWN = 0, 1, 2, 3   # bz2b200_region.kind
+REGION_KINDS = ("HEADER", "BLOCK", "END", "UNKNOWN")
+NO_SIGNATURE = 1   # bz2b200_region.flags: a block parsed where its predecessor ends (its signature is damaged)
+
+# One region of Bzip2Engine.recover: input bits [bit_begin, bit_end), its kind (and kind_name), status (0 or an Err code),
+# where its bytes are in the recovered data, the stored CRC, the stream (END regions before it) and flags.
+Region = namedtuple("Region", "bit_begin bit_end kind kind_name status out_offset out_bytes crc stream flags")
 
 
 def _coerce_input(inp):
@@ -251,6 +261,24 @@ class Bzip2Engine:
         finally:
             self._L.bz2b200_free(pos)
             self._L.bz2b200_free(sz)
+
+    def recover(self, input):
+        """What survives of a damaged file (bzip2recover, without stopping at damage): the input is read as a sequence of
+        streams; returns (data, regions).  data = the bytes of every block that decodes and matches its CRC, in input
+        order; regions = list of Region tiling the input bits (include/bz2b200.h, bz2b200_recover).  Damage is reported in
+        the regions, never raised: only CUDA or argument errors raise."""
+        a = _coerce_input(input)
+        out, n = C.POINTER(C.c_uint8)(), C.c_size_t()
+        regs, nr = C.POINTER(_native.Region)(), C.c_size_t()
+        rc = self._L.bz2b200_recover(self._ctx, a.ctypes.data, a.size, C.byref(out), C.byref(n), C.byref(regs), C.byref(nr))
+        if rc:
+            self._raise(rc)
+        try:
+            regions = [Region(r.bit_begin, r.bit_end, r.kind, REGION_KINDS[r.kind], r.status, r.out_offset, r.out_bytes, r.crc,
+                              r.stream, r.flags) for r in (regs[i] for i in range(nr.value))]
+        finally:
+            self._L.bz2b200_free(regs)
+        return self._take(out, n.value), regions
 
     # -- extras used by bench.py / tests --
     def stats(self):

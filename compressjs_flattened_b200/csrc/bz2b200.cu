@@ -18,6 +18,7 @@
 #include <chrono>
 #include <condition_variable>
 #include <future>
+#include <map>
 #include <mutex>
 #include <thread>
 #include <cctype>

@@ -14,6 +14,7 @@
  *   Bzip2.decompressBlock(BJ:1797-1818)    bz2b200_decompress_block
  *   Bzip2.table          (BJ:1823-1863)    bz2b200_table
  *   Err / ErrorMessages  (BJ:1365-1383)    bz2b200_strerror
+ *   (bzip2recover: no counterpart in BJ)   bz2b200_recover
  */
 #ifndef BZ2B200_H
 #define BZ2B200_H
@@ -71,6 +72,31 @@ int bz2b200_decompress(bz2b200_ctx *ctx, const uint8_t *in, size_t n, int multis
 int bz2b200_decompress_block(bz2b200_ctx *ctx, const uint8_t *in, size_t n, uint64_t bitpos, uint8_t **out, size_t *out_len);
 int bz2b200_table(bz2b200_ctx *ctx, const uint8_t *in, size_t n, int multistream, uint64_t **bitpos, uint32_t **sizes, size_t *count);
 void bz2b200_free(void *p);
+
+/* Recovery of a damaged file (what bzip2recover + bunzip2 of its pieces do, without stopping at damage).  The input is
+ * read as a sequence of streams (like multistream = 1).  *out = the bytes of every RECOVERED block, in input order: a
+ * block that decodes without error, fits its stream's block size (BZh<level>; 9 if that header is damaged) and whose CRC
+ * equals the one in its header.  *regions tiles the input bits [0, 8n) in order:
+ *   HEADER   the 4 header bytes (looked for at byte 0 and after a recognised footer)
+ *   BLOCK    a block from its signature (or from where its predecessor ends) up to the next region
+ *   END      end-of-stream signature, stream CRC, padding; status 0 only if every block of the stream was recovered and
+ *            the stored CRC equals their fold
+ *   UNKNOWN  bits nothing recognised claims (garbage, bits after a damaged header up to the first signature)
+ * status = 0 or the BZ2B200_E_* code that condemned the region (a bad CRC or an oversized block: DATA_ERROR; UNKNOWN and
+ * damaged headers: NOT_BZIP_DATA).  A block whose signature is damaged is still parsed where the region before it ends
+ * if that region is a recovered block or an intact header: it is flagged BZ2B200_REGION_NO_SIGNATURE.  After a lost
+ * block the walk goes on at the next signature.  Returns 0 whenever the call ran, whatever was lost; both arrays are
+ * released with bz2b200_free.  bz2b200_last_stats: n_blocks = blocks recovered, out_bytes, ms_total. */
+enum { BZ2B200_REGION_HEADER = 0, BZ2B200_REGION_BLOCK = 1, BZ2B200_REGION_END = 2, BZ2B200_REGION_UNKNOWN = 3 };
+#define BZ2B200_REGION_NO_SIGNATURE 1u
+typedef struct {
+  uint64_t bit_begin, bit_end;   /* [bit_begin, bit_end) of the input */
+  uint64_t out_offset;           /* where the region's bytes are (or would be) in *out */
+  uint32_t out_bytes, crc;       /* bytes recovered from it; CRC stored in a BLOCK / END region */
+  int32_t status;
+  uint32_t kind, stream, flags;  /* stream = END regions before this one */
+} bz2b200_region;
+int bz2b200_recover(bz2b200_ctx *ctx, const uint8_t *in, size_t n, uint8_t **out, size_t *out_len, bz2b200_region **regions, size_t *n_regions);
 
 /* Device-resident entry points: input already in HBM (16-byte aligned), output written to a
  * caller-provided device buffer of out_cap bytes (multiple of 4).  Used for the roofline figure. */
