@@ -39,10 +39,11 @@ struct DecBlk {
   u64 endbit;      // first bit after the end-of-block symbol
   u32 target_crc;  // BJ:1440
   u32 orig_ptr;    // BJ:1448
-  u32 count;       // dbufCount: bytes of the L column
+  u32 count;       // dbufCount: bytes of the L column; with err: the symbols parsed before the error, then (k_sym_offsets)
+                   // the most bytes a size check saw among them
   int err;         // 0 or a negative Err code
   u32 kind;        // 0 = block magic, 1 = end-of-stream magic (then target_crc = stream CRC)
-  u32 nsym;        // symbols parsed, including end-of-block
+  u32 nsym;        // symbols parsed, including end-of-block (0 with err)
 };
 
 // ---- K-U1 -----------------------------------------------------------------------------------
@@ -507,7 +508,13 @@ __global__ void __launch_bounds__(PT) k_huff_parse(const u8 *__restrict__ in, u6
       u32 take = left < total ? left : total;
       bool fin = false;
       if (sm.first_eob < take) { take = sm.first_eob + 1; fin = true; }
-      if (sm.first_bad < take || sm.first_eof < take) { err = sm.first_eof < sm.first_bad ? BZ2B200_E_UNEXPECTED_INPUT_EOF : BZ2B200_E_DATA_ERROR; break; }
+      if (sm.first_bad < take || sm.first_eof < take) {
+        err = sm.first_eof < sm.first_bad ? BZ2B200_E_UNEXPECTED_INPUT_EOF : BZ2B200_E_DATA_ERROR;
+        take = sm.first_eof < sm.first_bad ? sm.first_eof : sm.first_bad;  // the codes before it are kept (k_sym_offsets)
+        if ((u32)lane < take) sm.stage[staged + lane] = (u16)(sm.csym[lane] & 0x7fffu);
+        staged += take;
+        break;
+      }
       if ((u32)lane < take) sm.stage[staged + lane] = (u16)(sm.csym[lane] & 0x7fffu);
       const u32 advance = sm.cend[take - 1];
       __syncthreads();  // csym / cend / adv / first_* are rewritten in the next step
@@ -526,7 +533,7 @@ __global__ void __launch_bounds__(PT) k_huff_parse(const u8 *__restrict__ in, u6
   }
   if (lane == 0) {
     res.err = err;
-    res.count = 0;  // filled by k_sym_offsets
+    res.count = err ? flushed : 0;  // with err the symbols before it; k_sym_offsets fills in the rest
     res.nsym = err ? 0 : flushed;
     res.endbit = cur_bit;
     out[k] = res;
@@ -760,7 +767,11 @@ __global__ void __launch_bounds__(DECW_PT) k_huff_parse_win(const u8 *__restrict
         advance = sm.eob_end;
         done = 1;
       }
-      if (fb < take || fo < take) { err = fo < fb ? BZ2B200_E_UNEXPECTED_INPUT_EOF : BZ2B200_E_DATA_ERROR; break; }
+      if (fb < take || fo < take) {
+        err = fo < fb ? BZ2B200_E_UNEXPECTED_INPUT_EOF : BZ2B200_E_DATA_ERROR;
+        flushed += fo < fb ? fo : fb;  // the codes before it are kept (k_sym_offsets)
+        break;
+      }
       flushed += take;
       P += advance;
       selector += (int)ngd;
@@ -773,7 +784,7 @@ __global__ void __launch_bounds__(DECW_PT) k_huff_parse_win(const u8 *__restrict
   }
   if (lane == 0) {
     res.err = err;
-    res.count = 0;  // filled by k_sym_offsets
+    res.count = err ? flushed : 0;  // with err the symbols before it; k_sym_offsets fills in the rest
     res.nsym = err ? 0 : flushed;
     res.endbit = cur_bit;
     out[k] = res;
@@ -782,12 +793,15 @@ __global__ void __launch_bounds__(DECW_PT) k_huff_parse_win(const u8 *__restrict
 
 // ---- K-U3b: RLE2^-1 offsets.  One CTA per candidate: the k-th RUNA/RUNB of a run stands for (sym+1) << k copies of
 // the current list front (BJ:1621-1652), a literal for one byte; exclusive scan -> position of every symbol's output.
+// A block whose parse failed gets the size the reference's checks saw before the failing code (count, see below): the
+// reference checks the size at every symbol, so a block that outgrew its stream's block size first is a Data error.
 __global__ void __launch_bounds__(1024) k_sym_offsets(DecBlk *__restrict__ blks, const u16 *__restrict__ dsym, u32 *__restrict__ doff, u32 dbuf_cap) {
   __shared__ int wsi[33];
   __shared__ u32 ws[33];
   const u32 k = blockIdx.x;
-  const u32 m = blks[k].nsym;
-  if (blks[k].kind != 0 || blks[k].err || m == 0) return;
+  const bool parsed = !blks[k].err;  // else: the m symbols before the parse error (the last one is no end-of-block)
+  const u32 m = parsed ? blks[k].nsym : blks[k].count;
+  if (blks[k].kind != 0 || m == 0) return;
   const u16 *Sk = dsym + (u64)k * DEC_SYM_STRIDE;
   u32 *Ok = doff + (u64)k * DEC_SYM_STRIDE;
   int carry_lit = -1;  // last non-run symbol so far
@@ -823,8 +837,23 @@ __global__ void __launch_bounds__(1024) k_sym_offsets(DecBlk *__restrict__ blks,
     if (carry > over) carry = over;  // saturate at once (only "too large" matters): carry + a chunk's total stays below 2^32
     if (tot_l > carry_lit) carry_lit = tot_l;
   }
+  if (!parsed) __syncthreads();  // Ok[] of every thread is read below
   if (threadIdx.x == 0) {
     Ok[m] = carry;
+    if (!parsed) {
+      // the sizes the reference checks before the failing code: t_run after every run digit (BJ:1647), the bytes before
+      // every literal + 1 (BJ:1663); the largest is that of the last literal or of the run after it
+      const u32 i0 = (u32)(carry_lit + 1);
+      u32 lit = i0 == 0 ? 0u : i0 == m ? Ok[m - 1] + 1 : Ok[i0];  // (a last literal was counted as end-of-block above)
+      lit = lit < over ? lit : over;
+      u32 run = 0;
+      for (u32 i = i0; i < m && run < over; i++) {  // at most 21 digits: (sym+1) << 20 > any block size
+        const u32 kk = i - i0, v = kk < 21 ? ((u32)Sk[i] + 1) << kk : over;
+        run = run + v < over ? run + v : over;
+      }
+      blks[k].count = lit > run ? lit : run;
+      return;
+    }
     // BJ:1647,1663 (dbuf overflow) and BJ:1677 (origPtr past the data) -> DATA_ERROR
     if (carry > dbuf_cap || blks[k].orig_ptr >= carry) { blks[k].err = BZ2B200_E_DATA_ERROR; blks[k].nsym = 0; carry = 0; }
     blks[k].count = carry;
