@@ -2,6 +2,8 @@
 (NPM/bin/compressjs:7-33,58,163-180):
 
   python -m compressjs_flattened_b200 -d|-z [-1 .. -9] [-b <bits>] [-t bzip2] [infile] [outfile]
+  python -m compressjs_flattened_b200 -d --list [--multistream] [infile]
+  python -m compressjs_flattened_b200 -d --range START:LEN [--index FILE] [--multistream] [infile] [outfile]
 
   -z  compress (the default), stream flavour: the input is read piece by piece (bz2b200_zstream_*), level 7 by default
   -d  decompress the FIRST stream of the input, stream flavour (bz2b200_dstream_*); --multistream decodes all of them
@@ -9,11 +11,16 @@
   -b  with -d: extract the single block whose signature starts at bit <bits> (Bzip2.decompressBlock)
   --recover  write what survives of a damaged file (every block that decodes and matches its CRC, all streams); one line per
       damaged region on stderr; exit status 0 when everything was intact, 2 when anything was lost
+  --list  print the block index (Bzip2Index.to_text: one line per block, stream, level, bit range, output range, CRC) to
+      stdout; with --multistream it covers every stream
+  --range START:LEN  write the decompressed bytes [START, START+LEN), clipped like a slice, decoding only the blocks that
+      hold them; --index FILE takes the index from --list output, otherwise it is built first (a full decode).  A negative
+      START (counted from the end, like a slice) must be written --range=START:LEN, since -1 .. -9 are flags
 If <infile> is omitted, reads from stdin; if <outfile> is omitted, writes to stdout.  Needs a CUDA device: no CPU fallback."""
 import argparse
 import sys
 
-from .bzip2 import NO_SIGNATURE, Err
+from .bzip2 import NO_SIGNATURE, Bzip2Index, Err
 
 
 def main(argv=None, engine=None):
@@ -31,7 +38,38 @@ def main(argv=None, engine=None):
     ap.add_argument("infile", nargs="?", default=None)
     ap.add_argument("outfile", nargs="?", default=None)
     ap.add_argument("--recover", action="store_true", help="write the intact blocks of a damaged file, report the damage")
+    ap.add_argument("--list", action="store_true", help="with -d: print the block index")
+    ap.add_argument("--range", default=None, metavar="START:LEN", help="with -d: write only these decompressed bytes")
+    ap.add_argument("--index", default=None, metavar="FILE", help="with --range: the block index (--list output)")
     a = ap.parse_args(argv)
+    for flag, on, verb in (("--list", a.list, "listing"), ("--range", a.range is not None, "reading a range")):
+        if not on:
+            continue
+        if a.compress:
+            print(f"{flag} can only be used without -z", file=sys.stderr)
+            return 1
+        if a.block >= 0:
+            print(f"{flag} and --block can't be used together", file=sys.stderr)
+            return 1
+        if a.recover:
+            print(f"{flag} and --recover can't be used together", file=sys.stderr)
+            return 1
+        if any(getattr(a, f"l{lv}") for lv in range(1, 10)):
+            print(f"Compression level has no effect when {verb}.", file=sys.stderr)
+            return 1
+        a.decompress = True
+    if a.list and a.range is not None:
+        print("--list and --range can't be used together", file=sys.stderr)
+        return 1
+    if a.index is not None and a.range is None:
+        print("--index can only be used with --range", file=sys.stderr)
+        return 1
+    if a.range is not None:
+        try:
+            start, length = (int(v) for v in a.range.split(":"))
+        except ValueError:
+            print(f"--range takes START:LEN, not {a.range}", file=sys.stderr)
+            return 1
     if a.recover:
         if a.compress:
             print("--recover can only be used without -z", file=sys.stderr)
@@ -81,6 +119,16 @@ def main(argv=None, engine=None):
                     sig = " (no signature)" if r.flags & NO_SIGNATURE else ""
                     print(f"bits {r.bit_begin}-{r.bit_end}: {r.kind_name}{sig} {names.get(r.status, r.status)}", file=sys.stderr)
                     status = 2
+        elif a.list:
+            dst.write(Bzip2.index(src.read(), a.multistream).to_text().encode())
+        elif a.range is not None:
+            data = src.read()
+            if a.index is not None:
+                with open(a.index) as fh:
+                    index = Bzip2Index.from_text(fh.read())
+            else:
+                index = Bzip2.index(data, a.multistream)
+            dst.write(Bzip2.decompressRange(data, index, start, length))
         elif a.decompress and a.block >= 0:
             dst.write(Bzip2.decompressBlock(src.read(), a.block))
         elif a.decompress:

@@ -55,6 +55,11 @@ class Region(C.Structure):
                 ("crc", C.c_uint32), ("status", C.c_int32), ("kind", C.c_uint32), ("stream", C.c_uint32), ("flags", C.c_uint32)]
 
 
+class BlockEntry(C.Structure):
+    _fields_ = [("bit_begin", C.c_uint64), ("bit_end", C.c_uint64), ("out_offset", C.c_uint64), ("out_bytes", C.c_uint32),
+                ("crc", C.c_uint32), ("stream", C.c_uint32), ("level", C.c_uint32)]
+
+
 def take_bytes(ptr, n):
     """n bytes at a ctypes pointer as a bytes object (ctypes.string_at takes an int-sized length: streams above 2 GiB)"""
     if not n:
@@ -84,6 +89,8 @@ class Library:
         L.bz2b200_table.argtypes = [vp, vp, C.c_size_t, C.c_int, C.POINTER(C.POINTER(C.c_uint64)),
                                     C.POINTER(C.POINTER(C.c_uint32)), szp]
         L.bz2b200_recover.argtypes = [vp, vp, C.c_size_t, u8pp, szp, C.POINTER(C.POINTER(Region)), szp]
+        L.bz2b200_index.argtypes = [vp, vp, C.c_size_t, C.c_int, C.POINTER(C.POINTER(BlockEntry)), szp]
+        L.bz2b200_decompress_ranges.argtypes = [vp, vp, C.c_size_t, vp, C.c_size_t, vp, vp, C.c_size_t, u8pp, szp]
         L.bz2b200_free.argtypes = [vp]
         L.bz2b200_free.restype = None
         L.bz2b200_compress_device.argtypes = [vp, vp, C.c_size_t, C.c_int, vp, C.c_size_t, szp]

@@ -5,6 +5,8 @@
     Bzip2.decompressBlock(input, bitpos, output=None)         BJ:1797-1818
     Bzip2.table(input, callback, multistream=False)           BJ:1823-1863
 
+Random access (no counterpart in the reference): Bzip2Engine.index, decompressRanges, decompressRange and open.
+
 Same names, argument meaning and error behaviour as the JavaScript API; the work is done by
 the CUDA library behind include/bz2b200.h.  Coercions follow Util.coerceInputStream /
 coerceOutputStream (BJ:178-272):
@@ -17,7 +19,11 @@ coerceOutputStream (BJ:178-272):
 Errors: `Bzip2Error` (a TypeError, like the JS `_throw`, BJ:1384-1391) carrying `.errorCode`;
 a bad level raises ValueError('Invalid block size multiplier') (JS: Error, BJ:2208).
 """
+import builtins
 import ctypes as C
+import io
+import mmap
+import os
 from collections import namedtuple
 
 import numpy as np
@@ -52,6 +58,105 @@ NO_SIGNATURE = 1   # bz2b200_region.flags: a block parsed where its predecessor 
 # One region of Bzip2Engine.recover: input bits [bit_begin, bit_end), its kind (and kind_name), status (0 or an Err code),
 # where its bytes are in the recovered data, the stored CRC, the stream (END regions before it) and flags.
 Region = namedtuple("Region", "bit_begin bit_end kind kind_name status out_offset out_bytes crc stream flags")
+
+
+# bz2b200_block_entry (include/bz2b200.h), field for field
+INDEX_DTYPE = np.dtype([("bit_begin", "<u8"), ("bit_end", "<u8"), ("out_offset", "<u8"), ("out_bytes", "<u4"), ("crc", "<u4"),
+                        ("stream", "<u4"), ("level", "<u4")])
+assert INDEX_DTYPE.itemsize == C.sizeof(_native.BlockEntry)
+LEVEL9_BLOCK = 900_000   # the largest block a stream can have: the buffer of Bzip2Engine.open
+
+
+class Bzip2Index:
+    """The blocks of a bzip2 file (Bzip2Engine.index): `entries` is a numpy structured array with the layout of
+    bz2b200_block_entry -- bit_begin, bit_end, out_offset, out_bytes, crc, stream, level -- one row per block in stream order."""
+    HEADER = "# bzip2 block index v1"
+    _TEXT_FIELDS = ("stream", "level", "bit_begin", "bit_end", "out_offset", "out_bytes", "crc")
+
+    def __init__(self, entries):
+        self.entries = np.ascontiguousarray(entries, dtype=INDEX_DTYPE)
+
+    @property
+    def total(self):
+        """decompressed bytes the index covers"""
+        if not len(self.entries):
+            return 0
+        last = self.entries[-1]
+        return int(last["out_offset"]) + int(last["out_bytes"])
+
+    def __len__(self):
+        return len(self.entries)
+
+    def to_text(self):
+        """One line per block under a header line: stream, level, bit_begin, bit_end, out_offset, out_bytes, crc (hex), tab-separated."""
+        lines = [self.HEADER]
+        for e in self.entries:
+            lines.append("\t".join([str(int(e[f])) for f in self._TEXT_FIELDS[:-1]] + [f"{int(e['crc']):08x}"]))
+        return "\n".join(lines) + "\n"
+
+    @classmethod
+    def from_text(cls, text):
+        """The inverse of to_text; ValueError on anything else."""
+        lines = text.splitlines()
+        if not lines or lines[0] != cls.HEADER:
+            raise ValueError(f"not a block index: the first line must be {cls.HEADER!r}")
+        rows = []
+        for no, line in enumerate(lines[1:], 2):
+            parts = line.split("\t")
+            if len(parts) != len(cls._TEXT_FIELDS):
+                raise ValueError(f"line {no}: {len(parts)} fields, expected {len(cls._TEXT_FIELDS)}")
+            vals = []
+            for name, p in zip(cls._TEXT_FIELDS, parts):
+                digits = "0123456789abcdefABCDEF" if name == "crc" else "0123456789"
+                if not p or any(ch not in digits for ch in p):
+                    raise ValueError(f"line {no}: bad {name} {p!r}")
+                v = int(p, 16 if name == "crc" else 10)
+                if v >= 1 << (INDEX_DTYPE[name].itemsize * 8):
+                    raise ValueError(f"line {no}: {name} {p} out of range")
+                vals.append(v)
+            rec = dict(zip(cls._TEXT_FIELDS, vals))
+            rows.append(tuple(rec[f] for f in INDEX_DTYPE.names))
+        return cls(np.array(rows, dtype=INDEX_DTYPE))
+
+
+class _RangeReader(io.RawIOBase):
+    """Raw side of Bzip2Engine.open: every readinto is one decompressRanges call."""
+
+    def __init__(self, eng, data, index):
+        super().__init__()
+        self._eng, self._data, self._index = eng, data, index
+        self._total, self._pos = index.total, 0
+
+    def readable(self):
+        return True
+
+    def seekable(self):
+        return True
+
+    def tell(self):
+        return self._pos
+
+    def seek(self, offset, whence=io.SEEK_SET):
+        base = {io.SEEK_SET: 0, io.SEEK_CUR: self._pos, io.SEEK_END: self._total}.get(whence)
+        if base is None:
+            raise ValueError(f"invalid whence ({whence})")
+        if base + offset < 0:
+            raise ValueError(f"negative seek position {base + offset}")
+        self._pos = base + offset
+        return self._pos
+
+    def readinto(self, b):
+        mv = memoryview(b).cast("B")
+        n = max(0, min(len(mv), self._total - self._pos))
+        if n:
+            mv[:n] = self._eng.decompressRange(self._data, self._index, self._pos, n)
+            self._pos += n
+        return n
+
+    def readall(self):
+        data = self._eng.decompressRange(self._data, self._index, self._pos, max(0, self._total - self._pos))
+        self._pos += len(data)
+        return data
 
 
 def _coerce_input(inp):
@@ -279,6 +384,57 @@ class Bzip2Engine:
         finally:
             self._L.bz2b200_free(regs)
         return self._take(out, n.value), regions
+
+    # -- random access (include/bz2b200.h, bz2b200_index / bz2b200_decompress_ranges) --
+    def index(self, input, multistream=False):
+        """The block index of `input` (a Bzip2Index): the same walk as table(), and the same errors."""
+        a = _coerce_input(input)
+        ptr, n = C.POINTER(_native.BlockEntry)(), C.c_size_t()
+        rc = self._L.bz2b200_index(self._ctx, a.ctypes.data, a.size, int(bool(multistream)), C.byref(ptr), C.byref(n))
+        if rc:
+            self._raise(rc)
+        try:
+            raw = _native.take_bytes(C.cast(ptr, C.POINTER(C.c_uint8)), n.value * INDEX_DTYPE.itemsize)
+        finally:
+            self._L.bz2b200_free(ptr)
+        return Bzip2Index(np.frombuffer(raw, dtype=INDEX_DTYPE))
+
+    def decompressRanges(self, input, index, ranges):
+        """The bytes of every (start, length) of the decompressed output, as a list in request order.  Each range is clipped
+        to the output the way slicing clips output[start:start + length].  One call decodes every block that covers a
+        range, once, and nothing else; the stream CRC is not checked (include/bz2b200.h)."""
+        a = _coerce_input(input)
+        ix = index.entries
+        total = index.total
+        se = [slice(int(s), int(s) + int(ln)).indices(total)[:2] for s, ln in ranges]
+        starts = np.array([s for s, _ in se], dtype=np.uint64)
+        lens = np.array([max(0, e - s) for s, e in se], dtype=np.uint64)
+        out, n = C.POINTER(C.c_uint8)(), C.c_size_t()
+        rc = self._L.bz2b200_decompress_ranges(self._ctx, a.ctypes.data, a.size, ix.ctypes.data, len(ix), starts.ctypes.data,
+                                               lens.ctypes.data, len(se), C.byref(out), C.byref(n))
+        if rc:
+            self._raise(rc)
+        data = self._take(out, n.value)
+        ends = np.cumsum(lens, dtype=np.uint64).tolist()
+        return [data[e - int(ln):e] for e, ln in zip(ends, lens.tolist())]
+
+    def decompressRange(self, input, index, start, length):
+        """decompressRanges for one range: output[start:start + length]"""
+        return self.decompressRanges(input, index, [(start, length)])[0]
+
+    def open(self, input, index=None, multistream=False):
+        """A seekable, read-only binary file over the decompressed bytes of `input` (bytes-like, or a path, which is
+        memory-mapped).  Every read decodes only the blocks it needs.  Without `index` one is built first: that is a full
+        decode of the input.  The buffer holds one level-9 block, so small sequential reads do not decode a block each;
+        read() to the end is one call."""
+        if isinstance(input, (str, os.PathLike)):
+            with builtins.open(input, "rb") as fh:
+                size = os.fstat(fh.fileno()).st_size
+                input = np.frombuffer(mmap.mmap(fh.fileno(), 0, access=mmap.ACCESS_READ), dtype=np.uint8) if size else b""
+        a = _coerce_input(input)
+        if index is None:
+            index = self.index(a, multistream)
+        return io.BufferedReader(_RangeReader(self, a, index), buffer_size=LEVEL9_BLOCK)
 
     # -- extras used by bench.py / tests --
     def stats(self):

@@ -115,6 +115,7 @@ struct Ctx {
   DevBuf recs_cand, cand_first, out2, recs_all, blksort, r2_status, hfreq, hlens, hplen, hcodes, hsel, hcost, hgoff, hblk;
   // decode-side buffers
   DevBuf d_in, cand, ncand, dmeta, dsyms, dL, dtt, dwalk, dblk, dout, dmisc, dsel, doff, dperm, dmap;
+  DevBuf dpieces, dgather;  // range reads: the pieces and the packed bytes
   // last compress, for debug_fetch
   struct Pipe {
     const u8 *d_in = nullptr;
@@ -161,7 +162,8 @@ struct Ctx {
                      &Lcol, &ranks, &lastocc, &A, &freq, &meta, &W, &bit_off, &scrc, &out, &out_len, &used_bits,
                      &rs_tiles, &gbounds, &key2, &big_cnt, &big_old, &big_rank, &big_tile0, &big_tblk, &totals2,
                      &recs_cand, &cand_first, &out2, &recs_all, &blksort, &r2_status, &hfreq, &hlens, &hplen, &hcodes, &hsel, &hcost, &hgoff, &hblk,
-                     &d_in, &cand, &ncand, &dmeta, &dsyms, &dL, &dtt, &dwalk, &dblk, &dout, &dmisc, &dsel, &doff, &dperm, &dmap};
+                     &d_in, &cand, &ncand, &dmeta, &dsyms, &dL, &dtt, &dwalk, &dblk, &dout, &dmisc, &dsel, &doff, &dperm, &dmap,
+                     &dpieces, &dgather};
     for (DevBuf *b : all) pool.push_back(b);
   }
 };

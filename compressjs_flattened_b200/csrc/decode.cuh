@@ -1285,3 +1285,52 @@ __global__ void k_dec_crc_recs(const u64 *__restrict__ out_off, int nb, BlockRec
   r.s = (i64)out_off[p]; r.p = (i64)out_off[p + 1]; r.e_true = 0; r.Ge = 0; r.outR = 0; r.n = 0; r.crc = 0; r.orig_ptr = 0;
   recs[p] = r;
 }
+
+// ---- range reads (bz2b200_decompress_ranges) --------------------------------------------------------------------------
+// Packs pieces of the decoded blocks into one buffer: piece i = src[piece_src[i], +len) -> dst[piece_dst[i], +len), with
+// piece_dst the exclusive scan of the lengths (piece_dst[n_pieces] = total, every piece at least one byte long).  The work
+// is split by output bytes, GATHER_CHUNK per CTA: thread 0 finds the piece that holds the CTA's first byte by binary
+// search, then the CTA copies every piece that meets its chunk together -- 16-byte stores on 16-byte-aligned destination
+// addresses, the source read as aligned words and shifted into place when it is not aligned alike.  The source buffer
+// must be readable for 4 bytes after a piece's end (a decode sink keeps 64 bytes of slack).
+#define GATHER_CHUNK 8192u
+#define GATHER_THREADS 256
+__global__ void __launch_bounds__(GATHER_THREADS) k_gather_ranges(const u8 *__restrict__ src, const u64 *__restrict__ piece_src,
+                                                                  const u64 *__restrict__ piece_dst, u32 n_pieces, u64 total, u8 *__restrict__ dst) {
+  __shared__ u32 first;
+  const u64 c0 = (u64)blockIdx.x * GATHER_CHUNK;
+  const u64 c1 = c0 + GATHER_CHUNK < total ? c0 + GATHER_CHUNK : total;
+  if (threadIdx.x == 0) {  // piece_dst[lo] <= c0 < piece_dst[hi]
+    u32 lo = 0, hi = n_pieces;
+    while (hi - lo > 1) {
+      const u32 mid = (lo + hi) >> 1;
+      if (piece_dst[mid] <= c0) lo = mid; else hi = mid;
+    }
+    first = lo;
+  }
+  __syncthreads();
+  for (u32 p = first; p < n_pieces && piece_dst[p] < c1; p++) {
+    const u64 a = piece_dst[p] > c0 ? piece_dst[p] : c0, e = piece_dst[p + 1] < c1 ? piece_dst[p + 1] : c1;
+    const u8 *s = src + piece_src[p] + (a - piece_dst[p]);
+    u8 *d = dst + a;
+    const u32 len = (u32)(e - a);  // at most GATHER_CHUNK
+    const u32 head = min((u32)((16u - ((uintptr_t)d & 15u)) & 15u), len);
+    const u32 nvec = (len - head) >> 4;
+    if (threadIdx.x < head) d[threadIdx.x] = s[threadIdx.x];
+    const u8 *sv = s + head;
+    uint4 *dv = reinterpret_cast<uint4 *>(d + head);
+    if (((uintptr_t)sv & 15u) == 0) {
+      for (u32 v = threadIdx.x; v < nvec; v += GATHER_THREADS) dv[v] = reinterpret_cast<const uint4 *>(sv)[v];
+    } else {
+      const u32 *w0 = reinterpret_cast<const u32 *>((uintptr_t)sv & ~(uintptr_t)3);
+      const u32 sh = 8u * (u32)((uintptr_t)sv & 3u);
+      for (u32 v = threadIdx.x; v < nvec; v += GATHER_THREADS) {
+        const u32 *w = w0 + 4 * v;
+        const u32 x0 = w[0], x1 = w[1], x2 = w[2], x3 = w[3], x4 = sh ? w[4] : 0u;
+        dv[v] = make_uint4(__funnelshift_r(x0, x1, sh), __funnelshift_r(x1, x2, sh), __funnelshift_r(x2, x3, sh), __funnelshift_r(x3, x4, sh));
+      }
+    }
+    const u32 t0 = head + 16 * nvec;
+    if (threadIdx.x < len - t0) d[t0 + threadIdx.x] = s[t0 + threadIdx.x];
+  }
+}

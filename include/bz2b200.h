@@ -15,6 +15,7 @@
  *   Bzip2.table          (BJ:1823-1863)    bz2b200_table
  *   Err / ErrorMessages  (BJ:1365-1383)    bz2b200_strerror
  *   (bzip2recover: no counterpart in BJ)   bz2b200_recover
+ *   (random access: no counterpart in BJ)  bz2b200_index / bz2b200_decompress_ranges
  */
 #ifndef BZ2B200_H
 #define BZ2B200_H
@@ -97,6 +98,34 @@ typedef struct {
   uint32_t kind, stream, flags;  /* stream = END regions before this one */
 } bz2b200_region;
 int bz2b200_recover(bz2b200_ctx *ctx, const uint8_t *in, size_t n, uint8_t **out, size_t *out_len, bz2b200_region **regions, size_t *n_regions);
+
+/* Random access to the decompressed bytes.  bz2b200_index walks the input like bz2b200_table (same batches, same error
+ * codes) and returns one entry per block in stream order; *entries is released with bz2b200_free.
+ * bz2b200_decompress_ranges returns the bytes [starts[i], starts[i] + lens[i]) of the decompressed output (streams
+ * concatenated), for every i, concatenated in request order: *out_len = sum of lens.  Ranges may overlap, repeat, come in
+ * any order or be empty.  Only the blocks that cover a range are decoded, each once, and only their compressed bytes are
+ * uploaded (one span per run of consecutive covering blocks, from byte bit_begin / 8 to byte (bit_end + 7) / 8); a block
+ * of a later stream decodes at its entry's level.  BZ2B200_E_ARG: a range outside [0, total) (total = out_offset +
+ * out_bytes of the last entry), entries not sorted by bit_begin or overlapping, out_offset not contiguous from 0, a
+ * level outside 1..9, a bit_end not above bit_begin or past 8n.  Otherwise the first failing covering block in index
+ * order decides: no signature at bit_begin -> NOT_BZIP_DATA (like decompress_block); a parse error or a block larger
+ * than its level allows -> that code (also a stale index whose block runs on into the next uploaded span); a bad block
+ * CRC -> DATA_ERROR; an end bit or size that differs from the entry, or a parse that runs past the uploaded bytes where
+ * the input goes on -> DATA_ERROR "index does not match the input" (a stale index).  The stream CRC is NOT checked: a
+ * partial read cannot see every block of a stream.  bz2b200_last_stats: n_blocks = blocks decoded, in_bytes = bytes
+ * uploaded, out_bytes, ms_total (device time up to the packed result; its copy to the host is not included). */
+typedef struct {
+  uint64_t bit_begin;    /* first bit of the block signature (what bz2b200_table reports) */
+  uint64_t bit_end;      /* first bit after the block (next signature or end-of-stream signature) */
+  uint64_t out_offset;   /* first decoded byte of the block in the decompressed output (streams concatenated) */
+  uint32_t out_bytes;    /* decoded bytes (bz2b200_table's size) */
+  uint32_t crc;          /* stored block CRC */
+  uint32_t stream;       /* 0-based stream the block belongs to */
+  uint32_t level;        /* that stream's BZh level, 1..9 */
+} bz2b200_block_entry;
+int bz2b200_index(bz2b200_ctx *ctx, const uint8_t *in, size_t n, int multistream, bz2b200_block_entry **entries, size_t *count);
+int bz2b200_decompress_ranges(bz2b200_ctx *ctx, const uint8_t *in, size_t n, const bz2b200_block_entry *index, size_t count,
+                              const uint64_t *starts, const uint64_t *lens, size_t n_ranges, uint8_t **out, size_t *out_len);
 
 /* Device-resident entry points: input already in HBM (16-byte aligned), output written to a
  * caller-provided device buffer of out_cap bytes (multiple of 4).  Used for the roofline figure. */
