@@ -577,6 +577,14 @@ class Bzip2Engine:
         raw = self.debug_fetch(4, 0, C.sizeof(_native.BlockMeta) * nb)
         return (_native.BlockMeta * nb).from_buffer_copy(raw.tobytes()) if nb else []
 
+    def block_huffman(self, k):
+        """tests only: (selectors, code lengths) of block k of the last batch of the last compress call: the table index
+        of every group of 50 symbols (n_sel of them) and the lengths as a (6, 260) array (n_groups x alphabet + 2 used)"""
+        sel = self.debug_fetch(5, k, 1 << 15)   # raises for a block outside the batch; a block has at most 18 000 selectors
+        sz = C.sizeof(_native.BlockMeta)
+        meta = _native.BlockMeta.from_buffer_copy(self.debug_fetch(4, 0, sz * (k + 1))[sz * k:].tobytes())
+        return sel[:meta.n_sel], self.debug_fetch(6, k, 6 * 260).reshape(6, 260)
+
 
 class _Lazy:
     """`Bzip2` global of the reference (BJ:2198-2255): created on first use."""

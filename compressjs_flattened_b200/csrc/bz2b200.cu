@@ -150,7 +150,7 @@ struct Ctx {
   i64 cand_s[64];
   bool recs_batched = false;  // the last call ran in batches: the full block table is in recs_all
   int last_nb = 0;
-  i64 last_bs = 0, last_as = 0;
+  i64 last_bs = 0, last_as = 0, last_ss = 0;
   cudaEvent_t ev[10]{};
   bool ev_ok = false;
   std::vector<cudaEvent_t> dom_ev;  // start/stop pairs around the dominant kernel's launches
@@ -637,6 +637,7 @@ int pipe_stages(Ctx *c) {
     const u32 max_nsel = (B + 1 + BZ_GROUP - 1) / BZ_GROUP;
     HufArrays ha;
     ha.sel_stride = round_up((i64)max_nsel + 1, 16);
+    c->last_ss = ha.sel_stride;
     ENS(c->hfreq, 4 * (size_t)nb * BZ_MAX_GROUPS * BZ_MAX_SYMS);
     ENS(c->hlens, (size_t)nb * BZ_MAX_GROUPS * HUF_LSTRIDE);
     ENS(c->hplen, 8 * (size_t)nb * BZ_MAX_SYMS);
@@ -1167,6 +1168,8 @@ long long bz2b200_debug_fetch(bz2b200_ctx *ctx, int what, int blk, void *dst, si
     case 2: src = P<u8>(c->Lcol) + (i64)blk * c->last_bs; bytes = (size_t)c->last_bs; break;
     case 3: src = P<u16>(c->A) + (i64)blk * c->last_as; bytes = 2 * (size_t)c->last_as; break;
     case 4: src = c->meta.p; bytes = sizeof(BlockMeta) * (size_t)nb; break;
+    case 5: src = P<u8>(c->hsel) + (i64)blk * c->last_ss; bytes = (size_t)c->last_ss; break;
+    case 6: src = P<u8>(c->hlens) + (i64)blk * BZ_MAX_GROUPS * HUF_LSTRIDE; bytes = BZ_MAX_GROUPS * HUF_LSTRIDE; break;
     default: return BZ2B200_E_ARG;
   }
   if (bytes > cap) bytes = cap;

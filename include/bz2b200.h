@@ -276,7 +276,10 @@ int bz2b200_last_stats(bz2b200_ctx *ctx, bz2b200_stats *st);
 
 /* Stage dumps for the parity tests (tests/ only): after a compress call, copy an intermediate
  * of block `blk` to host.  what: 0 = BlockRec table (all blocks), 1 = RLE1'd block bytes,
- * 2 = BWT L column, 3 = MTF/RLE2 symbols (u16), 4 = BlockMeta table (all blocks).
+ * 2 = BWT L column, 3 = MTF/RLE2 symbols (u16), 4 = BlockMeta table (all blocks),
+ * 5 = selectors: the table of every group of 50 symbols (u8 x n_sel), 6 = code lengths
+ * (u8 [6][260]: table t, symbol s at t * 260 + s; n_groups tables of alphabet + 2 used).
+ * Kinds 1-6 describe the last batch of the last compress call (see debug_set_batch_blocks).
  * Returns the number of bytes written to dst (<= cap) or a negative error. */
 long long bz2b200_debug_fetch(bz2b200_ctx *ctx, int what, int blk, void *dst, size_t cap);
 /* tests/ only: override the block capacity B (0 = level*100000-19) to stress the cut-point logic. */
