@@ -4,6 +4,8 @@
   python -m compressjs_flattened_b200 -d|-z [-1 .. -9] [-b <bits>] [-t bzip2] [infile] [outfile]
   python -m compressjs_flattened_b200 -d --list [--multistream] [infile]
   python -m compressjs_flattened_b200 -d --range START:LEN [--index FILE] [--multistream] [infile] [outfile]
+  python -m compressjs_flattened_b200 -d --grep PATTERN [--grep PATTERN ...] [--ignore-case] [--line-number] [--count]
+      [--multistream] [infile] [outfile]
 
   -z  compress (the default), stream flavour: the input is read piece by piece (bz2b200_zstream_*), level 7 by default
   -d  decompress the FIRST stream of the input, stream flavour (bz2b200_dstream_*); --multistream decodes all of them
@@ -16,11 +18,16 @@
   --range START:LEN  write the decompressed bytes [START, START+LEN), clipped like a slice, decoding only the blocks that
       hold them; --index FILE takes the index from --list output, otherwise it is built first (a full decode).  A negative
       START (counted from the end, like a slice) must be written --range=START:LEN, since -1 .. -9 are flags
+  --grep PATTERN  write the lines of the decompressed output that contain PATTERN (a fixed string, UTF-8; repeat the flag
+      for several), searched on the GPU (Bzip2Engine.search), like bzgrep -F; --ignore-case folds ASCII letters,
+      --line-number puts "N:" (1-based) before each line, --count prints the number of matching lines instead.  Exit
+      status 0 when a line matched, 1 when none did, as with grep
+Usage errors (flags that contradict each other) exit with status 1.
 If <infile> is omitted, reads from stdin; if <outfile> is omitted, writes to stdout.  Needs a CUDA device: no CPU fallback."""
 import argparse
 import sys
 
-from .bzip2 import NO_SIGNATURE, Bzip2Index, Err
+from .bzip2 import MATCH_FIRST_IN_LINE, NO_SIGNATURE, Bzip2Index, Err
 
 
 def main(argv=None, engine=None):
@@ -41,8 +48,16 @@ def main(argv=None, engine=None):
     ap.add_argument("--list", action="store_true", help="with -d: print the block index")
     ap.add_argument("--range", default=None, metavar="START:LEN", help="with -d: write only these decompressed bytes")
     ap.add_argument("--index", default=None, metavar="FILE", help="with --range: the block index (--list output)")
+    ap.add_argument("--grep", action="append", default=None, metavar="PATTERN", help="with -d: write the lines that contain PATTERN")
+    ap.add_argument("--ignore-case", action="store_true", help="with --grep: ASCII letters match either case")
+    ap.add_argument("--line-number", action="store_true", help="with --grep: prefix each line with its 1-based number and ':'")
+    ap.add_argument("--count", action="store_true", help="with --grep: print the number of matching lines")
     a = ap.parse_args(argv)
-    for flag, on, verb in (("--list", a.list, "listing"), ("--range", a.range is not None, "reading a range")):
+    for flag, on in (("--ignore-case", a.ignore_case), ("--line-number", a.line_number), ("--count", a.count)):
+        if on and not a.grep:
+            print(f"{flag} can only be used with --grep", file=sys.stderr)
+            return 1
+    for flag, on, verb in (("--list", a.list, "listing"), ("--range", a.range is not None, "reading a range"), ("--grep", bool(a.grep), "searching")):
         if not on:
             continue
         if a.compress:
@@ -61,6 +76,10 @@ def main(argv=None, engine=None):
     if a.list and a.range is not None:
         print("--list and --range can't be used together", file=sys.stderr)
         return 1
+    for flag, on in (("--list", a.list), ("--range", a.range is not None)):
+        if on and a.grep:
+            print(f"{flag} and --grep can't be used together", file=sys.stderr)
+            return 1
     if a.index is not None and a.range is None:
         print("--index can only be used with --range", file=sys.stderr)
         return 1
@@ -129,6 +148,17 @@ def main(argv=None, engine=None):
             else:
                 index = Bzip2.index(data, a.multistream)
             dst.write(Bzip2.decompressRange(data, index, start, length))
+        elif a.grep:
+            r = Bzip2.search(src.read(), a.grep, ignore_case=a.ignore_case, max_matches=0 if a.count else None, multistream=a.multistream,
+                             lines=not a.count)
+            if a.count:
+                dst.write(f"{r.total_lines}\n".encode())
+            elif a.line_number:
+                numbers = r.matches["line"][(r.matches["flags"] & MATCH_FIRST_IN_LINE) != 0]
+                dst.write(b"".join(b"%d:%s\n" % (int(n) + 1, ln) for n, ln in zip(numbers, r.lines.split(b"\n"))))
+            else:
+                dst.write(r.lines)
+            status = 0 if r.total_lines else 1
         elif a.decompress and a.block >= 0:
             dst.write(Bzip2.decompressBlock(src.read(), a.block))
         elif a.decompress:

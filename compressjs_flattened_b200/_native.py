@@ -60,6 +60,15 @@ class BlockEntry(C.Structure):
                 ("crc", C.c_uint32), ("stream", C.c_uint32), ("level", C.c_uint32)]
 
 
+class Match(C.Structure):
+    _fields_ = [("offset", C.c_uint64), ("line", C.c_uint64), ("line_begin", C.c_uint64), ("line_end", C.c_uint64),
+                ("pattern", C.c_uint32), ("flags", C.c_uint32)]
+
+
+class SearchTotals(C.Structure):
+    _fields_ = [("matches", C.c_uint64), ("lines", C.c_uint64), ("out_bytes", C.c_uint64)]
+
+
 def take_bytes(ptr, n):
     """n bytes at a ctypes pointer as a bytes object (ctypes.string_at takes an int-sized length: streams above 2 GiB)"""
     if not n:
@@ -91,6 +100,8 @@ class Library:
         L.bz2b200_recover.argtypes = [vp, vp, C.c_size_t, u8pp, szp, C.POINTER(C.POINTER(Region)), szp]
         L.bz2b200_index.argtypes = [vp, vp, C.c_size_t, C.c_int, C.POINTER(C.POINTER(BlockEntry)), szp]
         L.bz2b200_decompress_ranges.argtypes = [vp, vp, C.c_size_t, vp, C.c_size_t, vp, vp, C.c_size_t, u8pp, szp]
+        L.bz2b200_search.argtypes = [vp, vp, C.c_size_t, C.c_int, vp, vp, C.c_size_t, C.c_uint, C.c_uint64, C.POINTER(C.POINTER(Match)), szp,
+                                     C.POINTER(SearchTotals), u8pp, szp]
         L.bz2b200_free.argtypes = [vp]
         L.bz2b200_free.restype = None
         L.bz2b200_compress_device.argtypes = [vp, vp, C.c_size_t, C.c_int, vp, C.c_size_t, szp]
@@ -107,6 +118,7 @@ class Library:
         L.bz2b200_debug_set_block_cap.argtypes = [vp, C.c_uint32]
         L.bz2b200_debug_set_batch_blocks.argtypes = [vp, C.c_uint32]
         L.bz2b200_debug_set_ignore_block_crc.argtypes = [vp, C.c_int]
+        L.bz2b200_debug_set_search_tile.argtypes = [vp, C.c_uint32]
         L.bz2b200_debug_huffman_lengths.argtypes = [vp, vp, C.c_int, C.c_int]
         L.bz2b200_shard_begin.argtypes = [vp, vp, C.c_size_t, C.c_int, C.c_int]
         L.bz2b200_shard_cut.argtypes = [vp, C.c_uint64, C.c_uint64, C.c_int, C.POINTER(ShardInfo)]

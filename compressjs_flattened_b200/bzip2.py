@@ -6,6 +6,7 @@
     Bzip2.table(input, callback, multistream=False)           BJ:1823-1863
 
 Random access (no counterpart in the reference): Bzip2Engine.index, decompressRanges, decompressRange and open.
+Search (bzgrep -F, no counterpart in the reference): Bzip2Engine.search.
 
 Same names, argument meaning and error behaviour as the JavaScript API; the work is done by
 the CUDA library behind include/bz2b200.h.  Coercions follow Util.coerceInputStream /
@@ -64,7 +65,31 @@ Region = namedtuple("Region", "bit_begin bit_end kind kind_name status out_offse
 INDEX_DTYPE = np.dtype([("bit_begin", "<u8"), ("bit_end", "<u8"), ("out_offset", "<u8"), ("out_bytes", "<u4"), ("crc", "<u4"),
                         ("stream", "<u4"), ("level", "<u4")])
 assert INDEX_DTYPE.itemsize == C.sizeof(_native.BlockEntry)
-LEVEL9_BLOCK = 900_000   # the largest block a stream can have: the buffer of Bzip2Engine.open
+LEVEL9_BLOCK = 900_000
+
+# bz2b200_match (include/bz2b200.h), field for field
+MATCH_DTYPE = np.dtype([("offset", "<u8"), ("line", "<u8"), ("line_begin", "<u8"), ("line_end", "<u8"), ("pattern", "<u4"), ("flags", "<u4")])
+assert MATCH_DTYPE.itemsize == C.sizeof(_native.Match)
+SEARCH_IGNORE_CASE = 1   # bz2b200_search flags
+MATCH_FIRST_IN_LINE = 1  # bz2b200_match.flags: the first match of its line
+SEARCH_MAX_PATTERNS = SEARCH_MAX_LEN = 256
+
+# Bzip2Engine.search: matches (numpy array of MATCH_DTYPE, sorted by offset then pattern), the exact totals whatever
+# max_matches cut, the decoded size, and the lines (bytes, or None when not asked for)
+SearchResult = namedtuple("SearchResult", "matches total_matches total_lines out_bytes lines")
+
+
+def _patterns(patterns):
+    """bytes / str (one pattern) or an iterable of them -> list of bytes, within the limits of bz2b200_search"""
+    if isinstance(patterns, (bytes, bytearray, memoryview, str)):
+        patterns = [patterns]
+    pats = [p.encode() if isinstance(p, str) else bytes(p) for p in patterns]
+    if not 1 <= len(pats) <= SEARCH_MAX_PATTERNS:
+        raise ValueError(f"search takes 1..{SEARCH_MAX_PATTERNS} patterns, not {len(pats)}")
+    for i, p in enumerate(pats):
+        if not 1 <= len(p) <= SEARCH_MAX_LEN:
+            raise ValueError(f"pattern {i}: length must be 1..{SEARCH_MAX_LEN}, not {len(p)}")
+    return pats   # the largest block a stream can have: the buffer of Bzip2Engine.open
 
 
 class Bzip2Index:
@@ -435,6 +460,43 @@ class Bzip2Engine:
         if index is None:
             index = self.index(a, multistream)
         return io.BufferedReader(_RangeReader(self, a, index), buffer_size=LEVEL9_BLOCK)
+
+    # -- search (include/bz2b200.h, bz2b200_search) --
+    def search(self, input, patterns, ignore_case=False, max_matches=None, multistream=False, lines=False):
+        """Every occurrence of every fixed-string pattern in the decompressed output, found on the GPU where the decode
+        leaves the bytes (what bzgrep -F does).  patterns: one bytes / str (UTF-8) or an iterable of them, 1..256 patterns
+        of 1..256 bytes (ValueError otherwise).  ignore_case folds ASCII A-Z only.  Returns a SearchResult: `matches`
+        holds the first max_matches (None: all) in (offset, pattern) order; total_matches and total_lines count them all.
+        lines=True also returns the distinct lines holding a returned match, each ending in '\n' (grep -F's output).
+        Decode errors raise Bzip2Error as decompressFile does."""
+        pats = _patterns(patterns)
+        if max_matches is None:
+            max_matches = (1 << 64) - 1
+        elif max_matches < 0:
+            raise ValueError("max_matches must not be negative")
+        max_matches = min(int(max_matches), (1 << 64) - 1)
+        a = _coerce_input(input)
+        packed = np.frombuffer(b"".join(pats), dtype=np.uint8)
+        lens = np.array([len(p) for p in pats], dtype=np.uint32)
+        mp, nm, tot = C.POINTER(_native.Match)(), C.c_size_t(), _native.SearchTotals()
+        lp, nl = C.POINTER(C.c_uint8)(), C.c_size_t()
+        rc = self._L.bz2b200_search(self._ctx, a.ctypes.data, a.size, int(bool(multistream)), packed.ctypes.data, lens.ctypes.data, len(pats),
+                                    SEARCH_IGNORE_CASE if ignore_case else 0, int(max_matches), C.byref(mp), C.byref(nm), C.byref(tot),
+                                    C.byref(lp) if lines else None, C.byref(nl) if lines else None)
+        if rc:
+            self._raise(rc)
+        try:
+            raw = _native.take_bytes(C.cast(mp, C.POINTER(C.c_uint8)), nm.value * MATCH_DTYPE.itemsize)
+        finally:
+            self._L.bz2b200_free(mp)
+        text = self._take(lp, nl.value) if lines else None
+        return SearchResult(np.frombuffer(raw, dtype=MATCH_DTYPE), tot.matches, tot.lines, tot.out_bytes, text)
+
+    def debug_set_search_tile(self, nbytes):
+        """tests only: bytes per search tile (a multiple of 256 up to 8192; 0 restores the default)"""
+        rc = self._L.bz2b200_debug_set_search_tile(self._ctx, nbytes)
+        if rc:
+            self._raise(rc)
 
     # -- extras used by bench.py / tests --
     def stats(self):

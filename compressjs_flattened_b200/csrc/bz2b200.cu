@@ -12,6 +12,7 @@
 #include "mtf.cuh"
 #include "huff.cuh"
 #include "decode.cuh"
+#include "search.cuh"
 
 #include <algorithm>
 #include <atomic>
@@ -115,7 +116,8 @@ struct Ctx {
   DevBuf recs_cand, cand_first, out2, recs_all, blksort, r2_status, hfreq, hlens, hplen, hcodes, hsel, hcost, hgoff, hblk;
   // decode-side buffers
   DevBuf d_in, cand, ncand, dmeta, dsyms, dL, dtt, dwalk, dblk, dout, dmisc, dsel, doff, dperm, dmap;
-  DevBuf dpieces, dgather;  // range reads: the pieces and the packed bytes
+  DevBuf dpieces, dgather;  // range reads: the pieces and the packed bytes (search: the lines)
+  DevBuf dspat, dstile, dsbase, dstsum, dsmatch, dspart, dstot;  // search: patterns and filter, per-tile and per-thread summaries, matches
   // last compress, for debug_fetch
   struct Pipe {
     const u8 *d_in = nullptr;
@@ -145,6 +147,7 @@ struct Ctx {
   u32 cap_override = 0;    // tests only
   u32 batch_override = 0;  // tests only: blocks per batch
   u32 dec_batch = 0;       // tests only: candidates per decode batch (0 = DEC_BATCH)
+  u32 search_tile = 0;     // tests only: bytes per search tile (0 = SEARCH_TILE_DEFAULT)
   u64 shard_bits = 0;      // bit length of the last shard segment (phase 0 in `out`)
   int cand_n = 0, cand_max_blocks = 0, cand_nb[64];  // speculated cut walks of the last shard_cut_g
   i64 cand_s[64];
@@ -163,7 +166,7 @@ struct Ctx {
                      &rs_tiles, &gbounds, &key2, &big_cnt, &big_old, &big_rank, &big_tile0, &big_tblk, &totals2,
                      &recs_cand, &cand_first, &out2, &recs_all, &blksort, &r2_status, &hfreq, &hlens, &hplen, &hcodes, &hsel, &hcost, &hgoff, &hblk,
                      &d_in, &cand, &ncand, &dmeta, &dsyms, &dL, &dtt, &dwalk, &dblk, &dout, &dmisc, &dsel, &doff, &dperm, &dmap,
-                     &dpieces, &dgather};
+                     &dpieces, &dgather, &dspat, &dstile, &dsbase, &dstsum, &dsmatch, &dspart, &dstot};
     for (DevBuf *b : all) pool.push_back(b);
   }
 };
@@ -1208,6 +1211,13 @@ int bz2b200_debug_set_block_cap(bz2b200_ctx *ctx, uint32_t cap) {
   Ctx *c = reinterpret_cast<Ctx *>(ctx);
   if (!c || (cap && cap < 8) || cap > 899981) return BZ2B200_E_ARG;
   c->cap_override = cap;
+  return BZ2B200_OK;
+}
+
+int bz2b200_debug_set_search_tile(bz2b200_ctx *ctx, uint32_t bytes) {
+  Ctx *c = reinterpret_cast<Ctx *>(ctx);
+  if (!c || bytes % SEARCH_THREADS || bytes > SEARCH_TILE_MAX) return BZ2B200_E_ARG;
+  c->search_tile = bytes;
   return BZ2B200_OK;
 }
 

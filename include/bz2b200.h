@@ -16,6 +16,7 @@
  *   Err / ErrorMessages  (BJ:1365-1383)    bz2b200_strerror
  *   (bzip2recover: no counterpart in BJ)   bz2b200_recover
  *   (random access: no counterpart in BJ)  bz2b200_index / bz2b200_decompress_ranges
+ *   (bzgrep: no counterpart in BJ)         bz2b200_search
  */
 #ifndef BZ2B200_H
 #define BZ2B200_H
@@ -126,6 +127,36 @@ typedef struct {
 int bz2b200_index(bz2b200_ctx *ctx, const uint8_t *in, size_t n, int multistream, bz2b200_block_entry **entries, size_t *count);
 int bz2b200_decompress_ranges(bz2b200_ctx *ctx, const uint8_t *in, size_t n, const bz2b200_block_entry *index, size_t count,
                               const uint64_t *starts, const uint64_t *lens, size_t n_ranges, uint8_t **out, size_t *out_len);
+
+/* Fixed-string search of the decompressed output (what bzgrep -F does, without bringing the decoded bytes back).  The
+ * input is decoded exactly as bz2b200_decompress(ctx, in, n, multistream) decodes it -- same walk, CRC checks and error
+ * codes; on an error nothing is returned.  patterns: n_patterns byte strings packed one after the other, pattern_lens[i]
+ * bytes each; any byte is allowed ('\n' and NUL too).  1 <= n_patterns <= 256 and 1 <= length <= 256, otherwise
+ * BZ2B200_E_ARG (bz2b200_last_error says which).  flags: BZ2B200_SEARCH_IGNORE_CASE.
+ * Every occurrence of every pattern is a match: overlapping ones, each occurrence of a pattern listed twice, and matches
+ * across block or stream boundaries.  Matches are sorted by offset, then by pattern; *matches holds the first
+ * min(total, max_matches) of them (max_matches = 0: counts only).  totals->matches counts all matches and totals->lines
+ * the distinct lines in which a match starts, exact whatever max_matches is; totals->out_bytes is the decoded size.
+ * lines (NULL: skipped): the distinct lines that hold the start of a returned match, in order, each followed by one '\n'
+ * (for patterns without '\n', what grep -F prints, -i with IGNORE_CASE in the C locale).  *matches and *lines are
+ * released with bz2b200_free.  bz2b200_last_stats: n_blocks, in_bytes and out_bytes as bz2b200_decompress; ms_total =
+ * device time up to the packed results (their copy to the host is not included); ms_stage[5] = device time of the
+ * search kernels and the line gather alone. */
+#define BZ2B200_SEARCH_IGNORE_CASE 1u      /* ASCII: A-Z equal a-z; every other byte compares as it is */
+#define BZ2B200_MATCH_FIRST_IN_LINE 1u     /* bz2b200_match.flags */
+typedef struct {
+  uint64_t offset;      /* first byte of the match in the decompressed output (streams concatenated) */
+  uint64_t line;        /* '\n' bytes before offset: the 0-based line number */
+  uint64_t line_begin;  /* first byte of that line */
+  uint64_t line_end;    /* the '\n' that ends the line, or the output's length when the last line has none */
+  uint32_t pattern;     /* index of the pattern in the request */
+  uint32_t flags;       /* BZ2B200_MATCH_FIRST_IN_LINE: the first match of its line in the order above (no match starts
+                           earlier in the line, and none at the same offset has a lower pattern index) */
+} bz2b200_match;
+typedef struct { uint64_t matches, lines, out_bytes; } bz2b200_search_totals;
+int bz2b200_search(bz2b200_ctx *ctx, const uint8_t *in, size_t n, int multistream, const uint8_t *patterns, const uint32_t *pattern_lens,
+                   size_t n_patterns, unsigned flags, uint64_t max_matches, bz2b200_match **matches, size_t *n_matches,
+                   bz2b200_search_totals *totals, uint8_t **lines, size_t *lines_len);
 
 /* Device-resident entry points: input already in HBM (16-byte aligned), output written to a
  * caller-provided device buffer of out_cap bytes (multiple of 4).  Used for the roofline figure. */
@@ -287,6 +318,9 @@ int bz2b200_debug_set_block_cap(bz2b200_ctx *ctx, uint32_t cap);
 /* tests/ only: run the per-block stages in batches of at most `blocks` blocks (0 = as many as fit the
  * 31-bit index space and 70 % of the free device memory).  Stage dumps then show the last batch. */
 int bz2b200_debug_set_batch_blocks(bz2b200_ctx *ctx, uint32_t blocks);
+/* tests/ only: bytes per tile of the search kernels, a multiple of 256 up to 8192 (0 = 8192), so that small outputs
+ * span many tiles. */
+int bz2b200_debug_set_search_tile(bz2b200_ctx *ctx, uint32_t bytes);
 /* tests/ only: skip the block-CRC comparison of the decoder (BJ:1756-1761), so that what a damaged stream decodes TO
  * can be compared with the oracle.  Not reachable from the environment. */
 int bz2b200_debug_set_ignore_block_crc(bz2b200_ctx *ctx, int on);
