@@ -61,6 +61,8 @@ __global__ void k_seg_init(const BlockRec *__restrict__ recs, int nb, u32 *__res
 }
 
 // ---- key construction ------------------------------------------------------------------------
+#define KEY_BITS 44   // bits of the first sort key: 5 radix passes of 9 bits (36 bits, four passes, measured slower)
+#define KEY_SLACK 2   // depth limit of the round-0 code tree above ceil(log2 alphabet)
 // The first sort covers as many symbols as fit 44 bits.  Round 1 gave every symbol of a block the same number of bits
 // (dense codes, b = ceil(log2 alphabet): 6 symbols of text).  Now the bytes get an ORDER-PRESERVING PREFIX-FREE code
 // whose lengths follow the symbol frequencies (an alphabetic tree built by weight-balanced bisection, depth limited to
@@ -102,7 +104,7 @@ __global__ void __launch_bounds__(256) k_sym_used(const u8 *__restrict__ blk, i6
   if (tot) atomicAdd(&bs[p].cnt[threadIdx.x], tot);
 }
 // nb CTAs of 256 threads (thread = byte value): the code of every byte value, L
-__global__ void __launch_bounds__(256) k_sym_tab(BlkSort *__restrict__ bs, u32 key_bits, u32 slack) {
+__global__ void __launch_bounds__(256) k_sym_tab(BlkSort *__restrict__ bs) {
   __shared__ u32 ws[33];
   __shared__ u32 P[257];     // P[r] = occurrences of the first r used symbols (by value)
   __shared__ u32 wmax[8];
@@ -122,7 +124,7 @@ __global__ void __launch_bounds__(256) k_sym_tab(BlkSort *__restrict__ bs, u32 k
     else {
       u32 lb = 1;
       while ((1u << lb) < alpha) lb++;
-      const u32 lmax = lb + (alpha > 2 ? slack : 0u);  // depth limit of the tree (slack = 2: at most 8 + 3 = 11 bits)
+      const u32 lmax = lb + (alpha > 2 ? KEY_SLACK : 0u);  // depth limit of the tree (at most 8 + 2 = 10 bits)
       u32 lo = 0, hi = alpha;                       // the node: used symbols [lo, hi)
       while (hi - lo > 1) {
         const u32 cap = 1u << (lmax - len - 1);     // leaves a child may still hold
@@ -154,10 +156,10 @@ __global__ void __launch_bounds__(256) k_sym_tab(BlkSort *__restrict__ bs, u32 k
     u32 m = 1;
     for (int w = 0; w < 8; w++) if (wmax[w] > m) m = wmax[w];
     B.maxlen = m;
-    B.L = key_bits / m;
+    B.L = KEY_BITS / m;
   }
 }
-// the first key_bits (44, or 36: one radix pass less) bits of the code string of each rotation, from bit 20 up; rotation
+// the first KEY_BITS bits of the code string of each rotation, from bit 20 up; rotation
 // index in the low 20 bits.  The tile's bytes (+ 43 more, cyclically: a key never needs more than 44 symbols) are staged
 // in shared memory.  A thread owns 16 CONSECUTIVE rotations and slides a bit window over their code string (drop the
 // first symbol's code, append codes at the end): ~2 table look-ups per rotation instead of one per covered symbol.  The
@@ -165,20 +167,19 @@ __global__ void __launch_bounds__(256) k_sym_tab(BlkSort *__restrict__ bs, u32 k
 // 20..28) is counted on the way, so pass 0 needs no k_rs_hist.
 __global__ void __launch_bounds__(SEG_THREADS) k_keys_init(const u8 *__restrict__ blk, i64 blk_stride, const BlockRec *__restrict__ recs,
                                                            const u32 *__restrict__ seg_tile0, const u32 *__restrict__ tile_blk,
-                                                           const BlkSort *__restrict__ bs, u64 *__restrict__ keys, u32 *__restrict__ hist0,
-                                                           u32 tile_base, u32 key_bits) {
+                                                           const BlkSort *__restrict__ bs, u64 *__restrict__ keys, u32 *__restrict__ hist0) {
   __shared__ u32 cw[256];  // length << 16 | code
   __shared__ u8 sc[SORT_TILE + 48];
   __shared__ u32 h[512];
   __shared__ u64 sk[SORT_TILE];
-  u32 tile = blockIdx.x + tile_base, p = tile_blk[tile];
+  u32 tile = blockIdx.x, p = tile_blk[tile];
   u32 n = recs[p].n;
   cw[threadIdx.x] = ((u32)bs[p].clen[threadIdx.x] << 16) | bs[p].cval[threadIdx.x];
   for (int i = threadIdx.x; i < 512; i += SEG_THREADS) h[i] = 0;
   __syncthreads();
   const u8 *T = blk + (i64)p * blk_stride;
   u32 l0 = (tile - seg_tile0[p]) * SORT_TILE;
-  u64 g0 = (u64)(tile - tile_base) * SORT_TILE;  // keys and per-tile histograms are local to the group of blocks being sorted
+  u64 g0 = (u64)tile * SORT_TILE;
   const u32 m = n - l0 < SORT_TILE ? n - l0 : SORT_TILE;
   for (u32 j = threadIdx.x; j < m + 43; j += SEG_THREADS) {
     u32 x = l0 + j;
@@ -193,12 +194,12 @@ __global__ void __launch_bounds__(SEG_THREADS) k_keys_init(const u8 *__restrict_
     for (u32 e = 0; e < SEG_E; e++) {
       const u32 j = j0 + e;
       if (j >= m) break;
-      while (bits < key_bits) {  // at most 43 + 9 bits are ever held
+      while (bits < KEY_BITS) {  // at most 43 + 10 bits are ever held
         const u32 w = cw[sc[kk++]], l = w >> 16;
         buf |= (u64)(w & 0xffffu) << (64 - bits - l);
         bits += l;
       }
-      const u64 key = ((buf >> (64 - key_bits)) << 20) | (l0 + j);
+      const u64 key = ((buf >> (64 - KEY_BITS)) << 20) | (l0 + j);
       sk[j] = key;
       atomicAdd(&h[(u32)(key >> 20) & 511u], 1u);
       const u32 lj = cw[sc[j]] >> 16;  // the window moves on by the first symbol's code
@@ -208,19 +209,19 @@ __global__ void __launch_bounds__(SEG_THREADS) k_keys_init(const u8 *__restrict_
   }
   __syncthreads();
   for (u32 j = threadIdx.x; j < m; j += SEG_THREADS) keys[g0 + j] = sk[j];
-  for (int i = threadIdx.x; i < 512; i += SEG_THREADS) hist0[(u64)(tile - tile_base) * 512 + i] = h[i];
+  for (int i = threadIdx.x; i < 512; i += SEG_THREADS) hist0[(u64)tile * 512 + i] = h[i];
 }
 // ---- one LSD radix pass (BITS-bit digit, 8 or 9), batched over blocks ---------------------------
 // seg_base (optional): slot at which segment p starts; default = seg_tile0[p] * SORT_TILE (block layout)
 template <int BITS>
 __global__ void __launch_bounds__(SORT_THREADS) k_rs_hist(const u64 *__restrict__ keys, const u32 *__restrict__ seg_cnt,
                                                           const u32 *__restrict__ seg_tile0, const u32 *__restrict__ tile_blk, int shift,
-                                                          u32 *__restrict__ hist, const u32 *__restrict__ seg_base, u32 tile_base = 0) {
+                                                          u32 *__restrict__ hist, const u32 *__restrict__ seg_base) {
   constexpr int NB = 1 << BITS;
   __shared__ u32 h[NB];
-  u32 tile = blockIdx.x + tile_base, p = tile_blk[tile];
+  u32 tile = blockIdx.x, p = tile_blk[tile];
   u32 cnt = seg_cnt[p], l0 = (tile - seg_tile0[p]) * SORT_TILE;
-  u64 g0 = seg_base ? (u64)seg_base[p] + l0 : (u64)(tile - tile_base) * SORT_TILE;
+  u64 g0 = seg_base ? (u64)seg_base[p] + l0 : (u64)tile * SORT_TILE;
   for (int i = threadIdx.x; i < NB; i += SORT_THREADS) h[i] = 0;
   __syncthreads();
   u64 k[SORT_E];
@@ -235,20 +236,19 @@ __global__ void __launch_bounds__(SORT_THREADS) k_rs_hist(const u64 *__restrict_
     if (l0 + o < cnt) atomicAdd(&h[(u32)(k[e] >> shift) & (NB - 1)], 1u);
   }
   __syncthreads();
-  for (int i = threadIdx.x; i < NB; i += SORT_THREADS) hist[(u64)(tile - tile_base) * NB + i] = h[i];
+  for (int i = threadIdx.x; i < NB; i += SORT_THREADS) hist[(u64)tile * NB + i] = h[i];
 }
 // per block: column-wise exclusive prefix over its tiles (in place) and the digit totals.  grid (nb, NB / 32), 512
 // threads: a CTA owns 32 digits (lane = digit), its 16 warps split the block's tiles into contiguous ranges: sum of
 // the own range, exclusive scan over the warps in shared memory, then the prefixes of the own range.
 #define RSS_WARPS 16
 template <int BITS>
-__global__ void __launch_bounds__(RSS_WARPS * 32) k_rs_scan(u32 *__restrict__ hist, const u32 *__restrict__ seg_tile0, u32 *__restrict__ digit_tot,
-                                                            u32 p_base = 0, u32 tile_base = 0) {
+__global__ void __launch_bounds__(RSS_WARPS * 32) k_rs_scan(u32 *__restrict__ hist, const u32 *__restrict__ seg_tile0, u32 *__restrict__ digit_tot) {
   constexpr int NB = 1 << BITS;
   __shared__ u32 part[RSS_WARPS][32];
-  const u32 p = blockIdx.x + p_base, d = blockIdx.y * 32 + lane_id();
+  const u32 p = blockIdx.x, d = blockIdx.y * 32 + lane_id();
   const int w = warp_id();
-  const u32 t0 = seg_tile0[p] - tile_base, t1 = seg_tile0[p + 1] - tile_base, nt = t1 - t0;
+  const u32 t0 = seg_tile0[p], t1 = seg_tile0[p + 1], nt = t1 - t0;
   const u32 per = (nt + RSS_WARPS - 1) / RSS_WARPS;
   const u32 a = t0 + (u32)w * per < t1 ? t0 + (u32)w * per : t1, b = a + per < t1 ? a + per : t1;
   u32 sum = 0;
@@ -268,13 +268,13 @@ template <int BITS>
 __global__ void __launch_bounds__(SORT_THREADS, 3) k_rs_scatter(const u64 *__restrict__ keys_in, u64 *__restrict__ keys_out,
                                                              const u32 *__restrict__ seg_cnt, const u32 *__restrict__ seg_tile0,
                                                              const u32 *__restrict__ tile_blk, int shift, const u32 *__restrict__ hist,
-                                                             const u32 *__restrict__ digit_tot, const u32 *__restrict__ seg_base, u32 tile_base = 0) {
+                                                             const u32 *__restrict__ digit_tot, const u32 *__restrict__ seg_base) {
   constexpr int NB = 1 << BITS;
   __shared__ u16 wcnt[SORT_THREADS / 32][NB];  // a warp ranks 256 keys: counts fit 16 bits
   __shared__ u32 base[NB];
-  u32 tile = blockIdx.x + tile_base, p = tile_blk[tile];
+  u32 tile = blockIdx.x, p = tile_blk[tile];
   u32 cnt = seg_cnt[p], l0 = (tile - seg_tile0[p]) * SORT_TILE;
-  u64 gp = seg_base ? (u64)seg_base[p] : (u64)(seg_tile0[p] - tile_base) * SORT_TILE, g0 = gp + l0;
+  u64 gp = seg_base ? (u64)seg_base[p] : (u64)seg_tile0[p] * SORT_TILE, g0 = gp + l0;
   int lane = lane_id(), w = warp_id();
   for (int i = threadIdx.x; i < (SORT_THREADS / 32) * NB / 2; i += SORT_THREADS) reinterpret_cast<u32 *>(&wcnt[0][0])[i] = 0;
   {  // base of digit d = keys of the block with a smaller digit (scan of the totals) + keys with digit d in earlier tiles
@@ -282,7 +282,7 @@ __global__ void __launch_bounds__(SORT_THREADS, 3) k_rs_scatter(const u64 *__res
     __shared__ u32 ws[33];
     u32 tot_d = threadIdx.x < NB ? digit_tot[(u64)p * NB + threadIdx.x] : 0u, tot;
     u32 ex = block_excl_sum<u32>(tot_d, tot, ws);
-    if (threadIdx.x < NB) base[threadIdx.x] = ex + hist[(u64)(tile - tile_base) * NB + threadIdx.x];
+    if (threadIdx.x < NB) base[threadIdx.x] = ex + hist[(u64)tile * NB + threadIdx.x];
   }
   __syncthreads();
   u64 key[SORT_E];
@@ -395,7 +395,7 @@ __global__ void __launch_bounds__(R0_THREADS) k_rank0(const u64 *__restrict__ ke
                                                       const u32 *__restrict__ seg_tile0, const u32 *__restrict__ tile_blk,
                                                       u32 *__restrict__ isa, i64 stride, u32 *__restrict__ act_idx, u32 *__restrict__ act_rank,
                                                       u64 *__restrict__ status, u32 *__restrict__ ticket, u32 *__restrict__ n_act_out, u32 ntiles,
-                                                      const u8 *__restrict__ T, u8 *__restrict__ L, BlockRec *__restrict__ recs, u32 tile_base) {
+                                                      const u8 *__restrict__ T, u8 *__restrict__ L, BlockRec *__restrict__ recs) {
   __shared__ u64 sk[SORT_TILE + 2];  // sk[1 + i] = key of tile slot i; sk[0] / sk[m + 1] = the neighbours
   __shared__ int wlast[R0_THREADS / 32];
   __shared__ u32 wkeep[R0_THREADS / 32];
@@ -406,7 +406,7 @@ __global__ void __launch_bounds__(R0_THREADS) k_rank0(const u64 *__restrict__ ke
   __syncthreads();
   const u32 tile = sh_tile, p = tile_blk[tile];
   const u32 cnt = seg_cnt[p], l0 = (tile - seg_tile0[p]) * SORT_TILE;
-  const u64 gp = (u64)(seg_tile0[p] - tile_base) * SORT_TILE;  // the ticket runs over all tiles of the batch, the keys are the group's
+  const u64 gp = (u64)seg_tile0[p] * SORT_TILE;
   const u32 m = cnt - l0 < SORT_TILE ? cnt - l0 : SORT_TILE;
   for (u32 i = threadIdx.x; i < m + 2; i += R0_THREADS) {
     i64 j = (i64)l0 - 1 + i;

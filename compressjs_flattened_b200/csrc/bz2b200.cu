@@ -8,7 +8,6 @@
 #include "rle1.cuh"
 #include "bwt.cuh"
 #include "refine.cuh"
-#include "rsort2.cuh"
 #include "mtf.cuh"
 #include "huff.cuh"
 #include "decode.cuh"
@@ -111,7 +110,7 @@ struct Ctx {
   DevBuf isa, keysA, keysB, valsB, actI0, actI1, actR0, actR1, lb_status, lbm, hist, digit_base;
   DevBuf seg_cnt, seg_tile0, tile_blk, tile_i0, tile_i1, totals;
   DevBuf Lcol, ranks, lastocc, A, freq, meta, W, bit_off, scrc, out, out_len, used_bits;
-  DevBuf rs_tiles, gbounds;
+  DevBuf gbounds;
   DevBuf key2, big_cnt, big_old, big_rank, big_tile0, big_tblk, totals2;
   DevBuf recs_cand, cand_first, out2, recs_all, blksort, r2_status, hfreq, hlens, hplen, hcodes, hsel, hcost, hgoff, hblk;
   // decode-side buffers
@@ -128,11 +127,6 @@ struct Ctx {
   } pipe;
   bool trace = false;      // BZ2B200_TRACE
   int sms = 148;           // multiprocessors of the device
-  unsigned ibwt_s = 64;    // splitter spacing of the inverse-BWT list ranking (BZ2B200_IBWT_S overrides: 64..1024)
-  u32 r0_tiles = 1u << 30; // tiles per group of the round-0 sort (BZ2B200_R0_TILES; default: all blocks at once -- L2-sized groups were slower)
-  u32 key_slack = 2;       // depth limit of the code tree above ceil(log2 alphabet) (BZ2B200_KEY_SLACK=0..3)
-  u32 key_bits = 44;       // bits of the first sort key (BZ2B200_KEY_BITS=36: four radix passes instead of five, shallower keys)
-  bool rs2 = false;        // BZ2B200_RS2=1: the TMA-pipelined scatter passes of rsort2.cuh (measured 0.15-0.25 ms per step slower: profiles/r02_scatter_variants.md)
   int parse_mode = 0;      // BZ2B200_PARSE: 0 = by block count, 1 = k_huff_parse, 2 = k_huff_parse_win (development aid)
   std::vector<cudaEvent_t> trace_ev, trace_pool;
   std::vector<const char *> trace_names;
@@ -163,7 +157,7 @@ struct Ctx {
                      &isa, &keysA, &keysB, &valsB, &actI0, &actI1, &actR0, &actR1, &lb_status, &lbm, &hist, &digit_base,
                      &seg_cnt, &seg_tile0, &tile_blk, &tile_i0, &tile_i1, &totals,
                      &Lcol, &ranks, &lastocc, &A, &freq, &meta, &W, &bit_off, &scrc, &out, &out_len, &used_bits,
-                     &rs_tiles, &gbounds, &key2, &big_cnt, &big_old, &big_rank, &big_tile0, &big_tblk, &totals2,
+                     &gbounds, &key2, &big_cnt, &big_old, &big_rank, &big_tile0, &big_tblk, &totals2,
                      &recs_cand, &cand_first, &out2, &recs_all, &blksort, &r2_status, &hfreq, &hlens, &hplen, &hcodes, &hsel, &hcost, &hgoff, &hblk,
                      &d_in, &cand, &ncand, &dmeta, &dsyms, &dL, &dtt, &dwalk, &dblk, &dout, &dmisc, &dsel, &doff, &dperm, &dmap,
                      &dpieces, &dgather, &dspat, &dstile, &dsbase, &dstsum, &dsmatch, &dspart, &dstot};
@@ -447,12 +441,7 @@ int pipe_stages(Ctx *c) {
 
     // ---- S2 BWT ----
     size_t slots = 0;
-    std::vector<u32> tiles_of((size_t)nb), tile_first((size_t)nb);
-    for (int b = 0; b < nb; b++) {
-      tile_first[(size_t)b] = (u32)(slots / SORT_TILE);
-      tiles_of[(size_t)b] = (u32)(round_up(hrecs[(size_t)b].n, SORT_TILE) / SORT_TILE);
-      slots += (size_t)tiles_of[(size_t)b] * SORT_TILE;
-    }
+    for (auto &r : hrecs) slots += (size_t)round_up(r.n, SORT_TILE);
     const size_t tiles0 = slots / SORT_TILE;
     if ((u64)nb * (u64)BS >= (1ull << 31)) { c->err = "too many bytes for one call (block table * stride must stay below 2^31)"; return BZ2B200_E_ARG; }
     const size_t big_tiles = 5 * tiles0 + 16;                // big groups have > RF_T0 slots each
@@ -482,14 +471,12 @@ int pipe_stages(Ctx *c) {
     ENS(c->blksort, sizeof(BlkSort) * (size_t)nb);
     CK(cudaMemsetAsync(c->blksort.p, 0, sizeof(BlkSort) * (size_t)nb, c->stream));
     LAUNCH(k_sym_used, dim3(32, (unsigned)nb), 256, 0, P<u8>(c->blk), BS, P<BlockRec>(c->recs), P<BlkSort>(c->blksort));
-    LAUNCH(k_sym_tab, (unsigned)nb, 256, 0, P<BlkSort>(c->blksort), c->key_bits, c->key_slack);
-    ENS(c->rs_tiles, sizeof(RsTile) * (size_t)(Ta + 1));
-    if (Ta) LAUNCH(k_rs_tiles, (Ta + 255) / 256, 256, 0, seg_cnt, tile0, tblk, (u32)Ta, P<RsTile>(c->rs_tiles));
+    LAUNCH(k_sym_tab, (unsigned)nb, 256, 0, P<BlkSort>(c->blksort));
     u64 total_n = 0;
     for (auto &r : hrecs) total_n += r.n;
     c->dom_used = 0;
     auto timed_scatter = [&](bool bits9, unsigned grid, const u64 *ki, u64 *ko, const u32 *scnt, const u32 *st0, const u32 *stb, int shift,
-                             const u32 *sbase, u64 slots_now, u32 tile_base) -> int {
+                             const u32 *sbase, u64 slots_now) -> int {
       if (c->ev_ok) {
         if (c->dom_used + 2 > c->dom_ev.size()) {
           cudaEvent_t a, b2;
@@ -498,64 +485,31 @@ int pipe_stages(Ctx *c) {
         }
         CK(cudaEventRecord(c->dom_ev[c->dom_used], c->stream));
       }
-      if (bits9) LAUNCH(k_rs_scatter<9>, grid, SORT_THREADS, 0, ki, ko, scnt, st0, stb, shift, P<u32>(c->hist), P<u32>(c->digit_base), sbase, tile_base);
-      else LAUNCH(k_rs_scatter<8>, grid, SORT_THREADS, 0, ki, ko, scnt, st0, stb, shift, P<u32>(c->hist), P<u32>(c->digit_base), sbase, tile_base);
+      if (bits9) LAUNCH(k_rs_scatter<9>, grid, SORT_THREADS, 0, ki, ko, scnt, st0, stb, shift, P<u32>(c->hist), P<u32>(c->digit_base), sbase);
+      else LAUNCH(k_rs_scatter<8>, grid, SORT_THREADS, 0, ki, ko, scnt, st0, stb, shift, P<u32>(c->hist), P<u32>(c->digit_base), sbase);
       if (c->ev_ok) { CK(cudaEventRecord(c->dom_ev[c->dom_used + 1], c->stream)); c->dom_used += 2; }
       c->st.dom_launches++;
       c->st.dom_bytes += 16ull * slots_now;
       return 0;
     };
     u32 hv[4] = {0, 0, 0, 0};
-    // ---- round 0: 5-byte prefix, batched global radix sort (5 passes), then groups + ISA + active list ----
-    // The blocks are sorted in GROUPS of a few blocks: the two key buffers of a group (2 x 8 B per slot, r0_tiles tiles) are the
-    // same memory for every group and stay in the L2 cache through all five passes, so the passes move their 16 B per key
-    // through L2 instead of HBM.  k_rank0 keeps one ticket / look-back chain over all groups (the active list is global).
+    // ---- round 0: first keys, batched global radix sort (5 passes), then groups + ISA + active list ----
+    // All blocks of the batch are sorted at once (L2-sized groups of blocks were measured slower: profiles/r02_round0_l2_groups.log).
     {
       c->st.sort_rounds++;
       c->st.sort_slots += (u64)Ta * SORT_TILE;
       CK(cudaMemsetAsync(lbm, 0, 16, c->stream));
       CK(cudaMemsetAsync(status, 0, 8 * (size_t)Ta, c->stream));
-      for (int b0 = 0; b0 < nb;) {
-        u32 gt = 0;
-        int b1 = b0;
-        u64 gn = 0;
-        while (b1 < nb && (b1 == b0 || gt + tiles_of[b1] <= c->r0_tiles)) { gt += tiles_of[b1]; gn += hrecs[(size_t)b1].n; b1++; }
-        const u32 tb = tile_first[b0];
-        const unsigned gb = (unsigned)(b1 - b0);
-        LAUNCH(k_keys_init, gt, SEG_THREADS, 0, P<u8>(c->blk), BS, P<BlockRec>(c->recs), tile0, tblk, P<BlkSort>(c->blksort), kA, P<u32>(c->hist), tb, c->key_bits);
-        u64 *ki = kA, *ko = kB;
-        const int npass = (int)(c->key_bits + 8) / 9;
-        for (int pass = 0; pass < npass; pass++) {  // bits 20 .. 20 + key_bits, 9 bits a pass
-          if (pass) LAUNCH(k_rs_hist<9>, gt, SORT_THREADS, 0, ki, seg_cnt, tile0, tblk, 20 + pass * 9, P<u32>(c->hist), (const u32 *)nullptr, tb);  // pass 0: k_keys_init
-          if (c->rs2 && tb == 0 && gt == Ta) {  // whole batch at once: table of absolute positions + pipelined scatter (rsort2.cuh)
-#if RS2_SCAN1
-            LAUNCH(k_rs_scan<9>, dim3((unsigned)nb, 512 / 32), RSS_WARPS * 32, 0, P<u32>(c->hist), tile0, P<u32>(c->digit_base), 0u, 0u);
-#else
-            LAUNCH(k_rs_bases, (unsigned)nb, 512, 0, P<u32>(c->hist), tile0);
-#endif
-            if (c->ev_ok) {
-              if (c->dom_used + 2 > c->dom_ev.size()) {
-                cudaEvent_t a, b2;
-                CK(cudaEventCreate(&a)); CK(cudaEventCreate(&b2));
-                c->dom_ev.push_back(a); c->dom_ev.push_back(b2);
-              }
-              CK(cudaEventRecord(c->dom_ev[c->dom_used], c->stream));
-            }
-            const unsigned g2 = gt < (unsigned)(2 * c->sms) ? gt : (unsigned)(2 * c->sms);
-            LAUNCH(k_rs_scatter2, g2, RS2_THREADS, sizeof(Rs2Smem), ki, ko, P<u32>(c->hist), P<RsTile>(c->rs_tiles), gt, 20 + pass * 9, P<u32>(c->digit_base));
-            if (c->ev_ok) { CK(cudaEventRecord(c->dom_ev[c->dom_used + 1], c->stream)); c->dom_used += 2; }
-            c->st.dom_launches++;
-            c->st.dom_bytes += 16ull * gn;
-          } else {
-            LAUNCH(k_rs_scan<9>, dim3(gb, 512 / 32), RSS_WARPS * 32, 0, P<u32>(c->hist), tile0, P<u32>(c->digit_base), (u32)b0, tb);
-            if ((rc = timed_scatter(true, gt, ki, ko, seg_cnt, tile0, tblk, 20 + pass * 9, nullptr, gn, tb))) return rc;
-          }
-          u64 *tk = ki; ki = ko; ko = tk;
-        }
-        LAUNCH(k_rank0, gt, R0_THREADS, 0, ki, seg_cnt, tile0, tblk, P<u32>(c->isa), BS, actI[0], actR[0], status, lbm, lbm + 1, (u32)Ta, P<u8>(c->blk),
-               P<u8>(c->Lcol), P<BlockRec>(c->recs), tb);
-        b0 = b1;
+      LAUNCH(k_keys_init, Ta, SEG_THREADS, 0, P<u8>(c->blk), BS, P<BlockRec>(c->recs), tile0, tblk, P<BlkSort>(c->blksort), kA, P<u32>(c->hist));
+      u64 *ki = kA, *ko = kB;
+      for (int pass = 0; pass * 9 < KEY_BITS; pass++) {  // bits 20 .. 20 + KEY_BITS, 9 bits a pass
+        if (pass) LAUNCH(k_rs_hist<9>, Ta, SORT_THREADS, 0, ki, seg_cnt, tile0, tblk, 20 + pass * 9, P<u32>(c->hist), (const u32 *)nullptr);  // pass 0: k_keys_init
+        LAUNCH(k_rs_scan<9>, dim3((unsigned)nb, 512 / 32), RSS_WARPS * 32, 0, P<u32>(c->hist), tile0, P<u32>(c->digit_base));
+        if ((rc = timed_scatter(true, Ta, ki, ko, seg_cnt, tile0, tblk, 20 + pass * 9, nullptr, total_n))) return rc;
+        u64 *tk = ki; ki = ko; ko = tk;
       }
+      LAUNCH(k_rank0, Ta, R0_THREADS, 0, ki, seg_cnt, tile0, tblk, P<u32>(c->isa), BS, actI[0], actR[0], status, lbm, lbm + 1, (u32)Ta, P<u8>(c->blk),
+             P<u8>(c->Lcol), P<BlockRec>(c->recs));
       RC(rb_add(c, hv, lbm, sizeof hv));
       RC(rb_sync(c));
     }
@@ -592,7 +546,7 @@ int pipe_stages(Ctx *c) {
         for (int pass = 0; pass < 3; pass++) {  // key2 < 2^20: bits 32..55
           LAUNCH(k_rs_hist<8>, Tb, SORT_THREADS, 0, ki, bcnt, bt0, btb, 32 + pass * 8, P<u32>(c->hist), bbase);
           LAUNCH(k_rs_scan<8>, dim3(n_big, 256 / 32), RSS_WARPS * 32, 0, P<u32>(c->hist), bt0, P<u32>(c->digit_base));
-          if ((rc = timed_scatter(false, Tb, ki, ko, bcnt, bt0, btb, 32 + pass * 8, bbase, t2[1], 0u))) return rc;
+          if ((rc = timed_scatter(false, Tb, ki, ko, bcnt, bt0, btb, 32 + pass * 8, bbase, t2[1]))) return rc;
           u64 *tk = ki; ki = ko; ko = tk;
         }
         LAUNCH(k_sub_heads, Tb, SEG_THREADS, 0, ki, bcnt, bt0, btb, P<int>(c->tile_i0), bbase, 32);
@@ -859,13 +813,11 @@ cudaError_t set_kernel_attributes() {
 #ifndef BZ_SIM
   cudaError_t e;
   if ((e = cudaFuncSetAttribute(k_sort_groups, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RfSmem))) != cudaSuccess) return e;
-  if ((e = cudaFuncSetAttribute(k_rs_scatter2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Rs2Smem))) != cudaSuccess) return e;
   if ((e = cudaFuncSetAttribute(k_mtf_ranks, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(MTR_WARPS * sizeof(MtrSmem)))) != cudaSuccess) return e;
   if ((e = cudaFuncSetAttribute(k_huf_init, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(HufBuildSmem))) != cudaSuccess) return e;
   if ((e = cudaFuncSetAttribute(k_huf_build, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(HufBuildSmem))) != cudaSuccess) return e;
   if ((e = cudaFuncSetAttribute(k_huff_parse_win, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(DecWinSmem))) != cudaSuccess) return e;
-  const size_t rank_smem = 12 * (size_t)((DEC_DBUF_MAX + 64 - 1) / 64 + 2);  // the smallest splitter spacing (64) needs the most
-  if ((e = cudaFuncSetAttribute(k_ibwt_rank, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rank_smem)) != cudaSuccess) return e;
+  if ((e = cudaFuncSetAttribute(k_ibwt_rank, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)IBWT_RANK_SMEM)) != cudaSuccess) return e;
 #endif
   return cudaSuccess;
 }
@@ -880,11 +832,6 @@ int ctx_new(int device, Ctx **out) {
   c->ev_ok = true;
   { const char *t = getenv("BZ2B200_TRACE"); c->trace = t && *t && *t != '0'; }
   { const char *t = getenv("BZ2B200_PARSE"); c->parse_mode = t ? atoi(t) : 0; }
-  { const char *t = getenv("BZ2B200_KEY_SLACK"); if (t && *t >= '0' && *t <= '3') c->key_slack = (u32)(*t - '0'); }
-  { const char *t = getenv("BZ2B200_KEY_BITS"); int v = t ? atoi(t) : 0; if (v == 36 || v == 44 || v == 27) c->key_bits = (u32)v; }
-  { const char *t = getenv("BZ2B200_RS2"); if (t && *t) c->rs2 = *t != '0'; }
-  { const char *t = getenv("BZ2B200_R0_TILES"); int v = t ? atoi(t) : 0; if (v > 0) c->r0_tiles = (u32)v; }
-  { const char *t = getenv("BZ2B200_IBWT_S"); int v = t ? atoi(t) : 0; if (v == 64 || v == 128 || v == 256 || v == 512 || v == 1024) c->ibwt_s = (unsigned)v; }
   { int v = 0; if (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, device) == cudaSuccess && v > 0) c->sms = v; }
   for (auto &e : c->ev) if (cudaEventCreate(&e) != cudaSuccess) c->ev_ok = false;
   if (set_kernel_attributes() != cudaSuccess) { ctx_delete(c); return BZ2B200_E_CUDA; }

@@ -32,7 +32,7 @@
 #define DEC_LUT_BAD 0xffffu  // LUT entry of a prefix the reference's walk rejects; 0 = code longer than the LUT
 #define DEC_MAX_SEL 32768
 #define DEC_DBUF_MAX 900000
-#define IBWT_S ibwt_s  // splitter spacing: a kernel parameter / host variable (power of two)
+#define IBWT_S 64u     // splitter spacing of the inverse-BWT list ranking (power of two)
 
 struct DecBlk {
   u64 bitpos;      // position of the 48-bit magic
@@ -1016,12 +1016,12 @@ __global__ void __launch_bounds__(SEG_THREADS) k_dec_extract(const u64 *__restri
 // ---- K-U4b: list ranking ----------------------------------------------------------------------
 // Splitters of block p: slots 0, S, 2S, ... plus one extra for the start slot pos0 = tt[origPtr].
 // spl arrays are laid out per block at offset spl0[p]; W_p = ceil(n/S) + 1.
-__device__ __forceinline__ bool ibwt_is_spl(u32 j, u32 pos0, u32 ibwt_s) { return (j & (IBWT_S - 1)) == 0 || j == pos0; }
-__device__ __forceinline__ u32 ibwt_spl_index(u32 j, u32 pos0, u32 W, u32 ibwt_s) { return j == pos0 ? W - 1 : j / IBWT_S; }
+__device__ __forceinline__ bool ibwt_is_spl(u32 j, u32 pos0) { return (j & (IBWT_S - 1)) == 0 || j == pos0; }
+__device__ __forceinline__ u32 ibwt_spl_index(u32 j, u32 pos0, u32 W) { return j == pos0 ? W - 1 : j / IBWT_S; }
 
 __global__ void __launch_bounds__(256) k_ibwt_walk1(const u32 *__restrict__ tt, const DecBlk *__restrict__ blks, const u32 *__restrict__ order,
                                                     const u32 *__restrict__ seg_tile0, const u32 *__restrict__ spl0, int nb,
-                                                    u32 *__restrict__ spl_next, u32 *__restrict__ spl_len, u32 p0, u32 ibwt_s) {
+                                                    u32 *__restrict__ spl_next, u32 *__restrict__ spl_len, u32 p0) {
   u32 p = p0 + blockIdx.y;  // launched in batches of blocks whose T-vectors fit the L2 together
   const DecBlk &b = blks[order[p]];
   u32 n = b.count;
@@ -1037,13 +1037,15 @@ __global__ void __launch_bounds__(256) k_ibwt_walk1(const u32 *__restrict__ tt, 
       continue;
     }
     u32 cur = start, len = 0;
-    do { cur = T[cur] >> 8; len++; } while (!ibwt_is_spl(cur, pos0, ibwt_s) && len < n);
-    spl_next[spl0[p] + s] = ibwt_spl_index(cur, pos0, W, ibwt_s);
+    do { cur = T[cur] >> 8; len++; } while (!ibwt_is_spl(cur, pos0) && len < n);
+    spl_next[spl0[p] + s] = ibwt_spl_index(cur, pos0, W);
     spl_len[spl0[p] + s] = len;
   }
 }
 #define IBWT_R 64      // sub-splitter spacing of the splitter chase
-#define IBWT_SUBS 256  // >= (900000 / 64 + 2) / IBWT_R + 2 sub-splitters
+#define IBWT_SUBS 256  // >= the sub-splitters NS of the largest block
+static_assert(((DEC_DBUF_MAX + IBWT_S - 1) / IBWT_S + 1 + IBWT_R - 1) / IBWT_R + 1 <= IBWT_SUBS, "IBWT_SUBS too small for IBWT_S");
+#define IBWT_RANK_SMEM (12 * (size_t)((DEC_DBUF_MAX + IBWT_S - 1) / IBWT_S + 2))  // >= 3 * W words for the largest block
 // one CTA per block: offsets of the splitters along the walk from pos0; period if the walk closes
 // one CTA per block: the splitter links are staged in shared memory, one thread chases them there (a few dozen cycles
 // per hop instead of a DRAM round trip), all threads write the offsets back.  Dynamic shared memory: 3 * W words.
@@ -1051,7 +1053,7 @@ __global__ void __launch_bounds__(256) k_ibwt_walk1(const u32 *__restrict__ tt, 
 // walk1 + walk2 + rank = 0.64 + 1.29 + 0.85 ms per 100 MB; 128: 1.26 + 1.70 + 0.43; 256: 2.27 + 2.64 + 0.22).
 __global__ void __launch_bounds__(256) k_ibwt_rank(const DecBlk *__restrict__ blks, const u32 *__restrict__ order, const u32 *__restrict__ spl0, int nb,
                                                    const u32 *__restrict__ spl_next, const u32 *__restrict__ spl_len, u32 *__restrict__ spl_off,
-                                                   u32 *__restrict__ period, u32 ibwt_s) {
+                                                   u32 *__restrict__ period) {
   DYN_SMEM(u32, sm);
   const int p = blockIdx.x;
   const u32 n = blks[order[p]].count;
@@ -1059,6 +1061,7 @@ __global__ void __launch_bounds__(256) k_ibwt_rank(const DecBlk *__restrict__ bl
   const u32 W = (n + IBWT_S - 1) / IBWT_S + 1, base = spl0[p];
   u64 *lk = reinterpret_cast<u64 *>(sm);  // (length << 32) | next splitter: one dependent read per hop
   u32 *of = sm + 2 * W;
+#pragma unroll 1  // unrolling these two copy loops only costs registers
   for (u32 s = threadIdx.x; s < W; s += blockDim.x) { lk[s] = ((u64)spl_len[base + s] << 32) | spl_next[base + s]; of[s] = 0xffffffffu; }
   __syncthreads();
   // the chase over W links is itself list ranking: every 64th link (and the start) is a sub-splitter, all threads walk
@@ -1104,13 +1107,14 @@ __global__ void __launch_bounds__(256) k_ibwt_rank(const DecBlk *__restrict__ bl
     } while (cur != W - 1 && (cur % IBWT_R) != 0);
   }
   __syncthreads();
+#pragma unroll 1
   for (u32 s = threadIdx.x; s < W; s += blockDim.x) spl_off[base + s] = of[s];
 }
 __global__ void __launch_bounds__(256) k_ibwt_walk2(const u32 *__restrict__ tt, const u8 *__restrict__ dL, i64 l_stride,
                                                     const DecBlk *__restrict__ blks, const u32 *__restrict__ order,
                                                     const u32 *__restrict__ seg_tile0, const u32 *__restrict__ spl0, int nb,
                                                     const u32 *__restrict__ spl_len, const u32 *__restrict__ spl_off,
-                                                    const u32 *__restrict__ period, u8 *__restrict__ blk_out, i64 b_stride, u32 p0, u32 ibwt_s) {
+                                                    const u32 *__restrict__ period, u8 *__restrict__ blk_out, i64 b_stride, u32 p0) {
   u32 p = p0 + blockIdx.y;
   const DecBlk &b = blks[order[p]];
   u32 n = b.count;

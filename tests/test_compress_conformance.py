@@ -18,7 +18,7 @@ import numpy as np
 import pytest
 
 B9, B1 = 899_981, 99_981
-KEY_BITS, KEY_SLACK = 44, 2
+KEY_BITS, KEY_SLACK = 44, 2  # KEY_BITS and KEY_SLACK of csrc/bwt.cuh
 CPUS = os.cpu_count() or 1
 
 
