@@ -31,6 +31,11 @@ class BlockMeta(C.Structure):
                 ("n_sel", C.c_uint32), ("bits", C.c_uint64), ("d1", C.c_uint32), ("pad", C.c_uint32)]
 
 
+class DecBlk(C.Structure):
+    _fields_ = [("bitpos", C.c_uint64), ("endbit", C.c_uint64), ("target_crc", C.c_uint32), ("orig_ptr", C.c_uint32),
+                ("count", C.c_uint32), ("err", C.c_int32), ("kind", C.c_uint32), ("nsym", C.c_uint32)]
+
+
 class ShardInfo(C.Structure):
     _fields_ = [("next_start", C.c_uint64), ("bits", C.c_uint64), ("n_blocks", C.c_uint32), ("crc_fold", C.c_uint32),
                 ("complete", C.c_uint32), ("bit_phase", C.c_uint32)]
@@ -147,6 +152,7 @@ class Library:
         L.bz2b200_pool_decompress_shards.argtypes = [vp, vp, C.POINTER(ShardJob), C.c_int, C.c_int, C.c_uint64, C.c_int, C.c_int, C.c_int,
                                                      C.POINTER(RangeResult)]
         L.bz2b200_debug_set_decode_batch.argtypes = [vp, vp, C.c_uint32]
+        L.bz2b200_debug_set_rle1_threads.argtypes = [vp, vp, C.c_uint32]
         for name in ("zstream", "dstream"):
             getattr(L, f"bz2b200_{name}_open").argtypes = [vp, C.c_int, C.c_size_t, C.POINTER(vp)]
             getattr(L, f"bz2b200_{name}_feed").argtypes = [vp, vp, C.c_size_t, u8pp, szp]

@@ -615,6 +615,39 @@ class Bzip2Engine:
         if rc:
             self._raise(rc)
 
+    def debug_set_decode_batch(self, candidates):
+        """tests only: signature candidates per decode batch (0 restores the default), so that neighbours fall in different batches"""
+        rc = self._L.bz2b200_debug_set_decode_batch(self._ctx, None, candidates)
+        if rc:
+            self._raise(rc)
+
+    def debug_set_rle1_threads(self, threads):
+        """tests only: threads per CTA of the RLE1 inverse, 512 or 1024 (0 restores the choice by block count)"""
+        rc = self._L.bz2b200_debug_set_rle1_threads(self._ctx, None, threads)
+        if rc:
+            self._raise(rc)
+
+    def decode_candidates(self):
+        """tests only: the DecBlk of every candidate of the last batch of the last decode call"""
+        sz = C.sizeof(_native.DecBlk)
+        raw = self.debug_fetch(7, 0, sz * (1 << 20)).tobytes()
+        return list((_native.DecBlk * (len(raw) // sz)).from_buffer_copy(raw))
+
+    def decode_stages(self, k, nsym=None):
+        """tests only: (symbols, offsets, L column) of candidate k of the last decode batch; nsym: read that many symbols
+        and offsets instead of the candidate's own count (which a block that failed the size checks has set to 0)"""
+        b = self.decode_candidates()[k]
+        nsym = b.nsym if nsym is None else nsym
+        syms = np.frombuffer(self.debug_fetch(8, k, 2 * nsym).tobytes(), dtype=np.uint16)
+        offs = np.frombuffer(self.debug_fetch(9, k, 4 * (nsym + 1)).tobytes(), dtype=np.uint32)
+        return syms, offs, self.debug_fetch(10, k, b.count)
+
+    def decode_inverted(self):
+        """tests only: [(candidate index, inverse-BWT output)] of the blocks the last decode batch inverted, in stream order"""
+        chain = np.frombuffer(self.debug_fetch(12, 0, 4 << 20).tobytes(), dtype=np.uint32)
+        cands = self.decode_candidates()
+        return [(int(k), self.debug_fetch(11, p, cands[k].count).tobytes()) for p, k in enumerate(chain)]
+
     def debug_huffman_lengths(self, sorted_freqs, maxlen):
         """tests only: HuffmanAllocator.allocateHuffmanCodeLengths (BJ:1275-1298) run by the device copy of the allocator"""
         a = np.asarray(sorted_freqs, dtype=np.int32).copy()

@@ -141,6 +141,12 @@ struct Ctx {
   u32 cap_override = 0;    // tests only
   u32 batch_override = 0;  // tests only: blocks per batch
   u32 dec_batch = 0;       // tests only: candidates per decode batch (0 = DEC_BATCH)
+  u32 rle1_threads = 0;    // tests only: CTA width of k_rle1_inv, 512 or 1024 (0 = by block count)
+  // the last decode batch, for the decode kinds of debug_fetch: candidates parsed, blocks inverted (indices into the
+  // candidates, stream order) and the stride of their inverse-BWT outputs
+  u32 dec_last_ncand = 0;
+  std::vector<u32> dec_last_chain;
+  i64 dec_last_bs = 0;
   u32 search_tile = 0;     // tests only: bytes per search tile (0 = SEARCH_TILE_DEFAULT)
   u64 shard_bits = 0;      // bit length of the last shard segment (phase 0 in `out`)
   int cand_n = 0, cand_max_blocks = 0, cand_nb[64];  // speculated cut walks of the last shard_cut_g
@@ -1108,7 +1114,15 @@ long long bz2b200_debug_fetch(bz2b200_ctx *ctx, int what, int blk, void *dst, si
   const void *src = nullptr;
   size_t bytes = 0;
   int nb = c->last_nb;
-  if (what != 0 && what != 4 && (blk < 0 || blk >= nb)) return BZ2B200_E_ARG;
+  if (what >= 1 && what <= 6 && what != 4 && (blk < 0 || blk >= nb)) return BZ2B200_E_ARG;
+  if (what >= 8 && what <= 10 && (blk < 0 || (u32)blk >= c->dec_last_ncand)) return BZ2B200_E_ARG;
+  if (what == 11 && (blk < 0 || (size_t)blk >= c->dec_last_chain.size())) return BZ2B200_E_ARG;
+  if (what == 12) {  // host copy
+    bytes = 4 * c->dec_last_chain.size();
+    if (bytes > cap) bytes = cap;
+    if (bytes) memcpy(dst, c->dec_last_chain.data(), bytes);
+    return (long long)bytes;
+  }
   switch (what) {
     case 0:
       if (c->recs_batched) { src = c->recs_all.p; bytes = sizeof(BlockRec) * (size_t)c->pipe.nb; }
@@ -1120,6 +1134,15 @@ long long bz2b200_debug_fetch(bz2b200_ctx *ctx, int what, int blk, void *dst, si
     case 4: src = c->meta.p; bytes = sizeof(BlockMeta) * (size_t)nb; break;
     case 5: src = P<u8>(c->hsel) + (i64)blk * c->last_ss; bytes = (size_t)c->last_ss; break;
     case 6: src = P<u8>(c->hlens) + (i64)blk * BZ_MAX_GROUPS * HUF_LSTRIDE; bytes = BZ_MAX_GROUPS * HUF_LSTRIDE; break;
+    case 7: src = c->dmeta.p; bytes = sizeof(DecBlk) * (size_t)c->dec_last_ncand; break;
+    case 8: src = P<u16>(c->dsyms) + (i64)blk * DEC_SYM_STRIDE; bytes = 2 * (size_t)DEC_SYM_STRIDE; break;
+    case 9: src = P<u32>(c->doff) + (i64)blk * DEC_SYM_STRIDE; bytes = 4 * (size_t)DEC_SYM_STRIDE; break;
+    case 10: {
+      const i64 LS = round_up(DEC_DBUF_MAX + 1024, 256);  // as in dec_parse
+      src = P<u8>(c->dL) + (i64)blk * LS; bytes = (size_t)LS;
+      break;
+    }
+    case 11: src = P<u8>(c->dblk) + (i64)blk * c->dec_last_bs; bytes = (size_t)c->dec_last_bs; break;
     default: return BZ2B200_E_ARG;
   }
   if (bytes > cap) bytes = cap;

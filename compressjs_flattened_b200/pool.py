@@ -147,6 +147,11 @@ class Bzip2Pool:
     def debug_decode_batch(self, candidates):
         self._L.bz2b200_debug_set_decode_batch(None, self._p, candidates)
 
+    def debug_rle1_threads(self, threads):
+        rc = self._L.bz2b200_debug_set_rle1_threads(None, self._p, threads)
+        if rc:
+            self._raise(rc)
+
     def decompress_shards(self, group, jobs, total_shards, total_n, first_level, multistream=False, keep_on_device=False, to_bytes=True):
         """This process's byte slices of a stream that spans the group.  jobs: dicts {src, n_readable, own_len, base, index,
         on_device}.  Returns [(bytes | pointer | None, out_offset, n_bytes, rc, n_blocks)] per job; the stream's status is

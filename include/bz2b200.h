@@ -280,6 +280,9 @@ int bz2b200_pool_compress_shards(bz2b200_pool *pool, bz2b200_group *grp, const b
 int bz2b200_pool_debug(bz2b200_pool *pool, uint32_t block_cap, uint32_t batch_blocks, size_t first_halo, int force_staging);
 /* tests/ only: candidates per decode batch (0 = 320) for a context / every lane of a pool */
 int bz2b200_debug_set_decode_batch(bz2b200_ctx *ctx, bz2b200_pool *pool, uint32_t candidates);
+/* tests/ only: threads per CTA of the RLE1 inverse, 512 or 1024 (0 = 1024 when the batch has no more blocks than the
+ * device has SMs, else 512) for a context / every lane of a pool, so that one input reaches both strip widths */
+int bz2b200_debug_set_rle1_threads(bz2b200_ctx *ctx, bz2b200_pool *pool, uint32_t threads);
 int bz2b200_debug_set_pool(bz2b200_ctx *ctx, size_t min_bytes, size_t shard_bytes, size_t first_halo, int force_staging);
 
 /* ---- the stream flavour (SURVEY.md 8f N2; csrc/stream_abi.inl) ----
@@ -311,6 +314,11 @@ int bz2b200_last_stats(bz2b200_ctx *ctx, bz2b200_stats *st);
  * 5 = selectors: the table of every group of 50 symbols (u8 x n_sel), 6 = code lengths
  * (u8 [6][260]: table t, symbol s at t * 260 + s; n_groups tables of alphabet + 2 used).
  * Kinds 1-6 describe the last batch of the last compress call (see debug_set_batch_blocks).
+ * Kinds 7-12 describe the last batch of the last decode call (see debug_set_decode_batch): 7 = the parsed candidates
+ * (DecBlk of csrc/decode.cuh, one per candidate), 8 = the symbols of candidate blk (u16, nsym of them, end-of-block
+ * last), 9 = its RLE2 inverse offsets (u32, nsym + 1: where each symbol's bytes start in the L column), 10 = its L
+ * column after the inverse MTF (count bytes), 11 = the inverse-BWT output (RLE1 bytes) of the blk-th inverted block,
+ * 12 = the inverted blocks as candidate indices (u32, stream order: entry blk is the candidate of kind 11's blk).
  * Returns the number of bytes written to dst (<= cap) or a negative error. */
 long long bz2b200_debug_fetch(bz2b200_ctx *ctx, int what, int blk, void *dst, size_t cap);
 /* tests/ only: override the block capacity B (0 = level*100000-19) to stress the cut-point logic. */

@@ -165,13 +165,23 @@ def make_block(content, used=None, ntab=2, lens=None, sel=None, sel_mtf=None, ns
     if orig == pidx:
         assert ibwt(L, pidx) == content
     stored = O.crc32(out if out is not None else b"") if crc is None else crc
+    bits, sym_end = write_block(A, used, orig, stored, lens, tables, raw)
+    return dict(bits=bits, crc=stored, out=out, A=A, sym_end=sym_end, n=len(content), used=used,
+                lens=lens, tables=tables, nsel=len(raw))
+
+
+def write_block(A, used, orig, stored, lens, tables, raw):
+    """The bits of one block: the symbols A (MTF/RLE2 over the byte map `used`, end-of-block last) coded with the code
+    lengths lens[tables[g]] in group g, raw selector MTF indices, origPtr and the stored CRC.  Returns the bits and the bit
+    offset where each symbol ends."""
+    m = len(A)
     hdr = [put(MAGIC_BLOCK, 48), put(stored, 32), put(0, 1), put(orig, 24)]
     groups = [any(b >> 4 == i for b in used) for i in range(16)]
     hdr.append(np.array(groups, dtype=np.uint8))
     for i in range(16):
         if groups[i]:
             hdr.append(np.array([(i << 4 | j) in used for j in range(16)], dtype=np.uint8))
-    hdr += [put(ntab, 3), put(len(raw), 15)]
+    hdr += [put(len(lens), 3), put(len(raw), 15)]
     r = np.array(raw, dtype=np.int64)
     sb = np.ones(int((r + 1).sum()), dtype=np.uint8)
     sb[np.cumsum(r + 1) - 1] = 0
@@ -190,8 +200,7 @@ def make_block(content, used=None, ntab=2, lens=None, sel=None, sel_mtf=None, ns
     k = np.arange(int(ends[-1])) - np.repeat(ends - ln, ln)
     data = ((np.repeat(codes, ln) >> (np.repeat(ln, ln) - 1 - k)) & 1).astype(np.uint8)
     head = np.concatenate(hdr)
-    return dict(bits=np.concatenate([head, data]), crc=stored, out=out, A=A, sym_end=len(head) + ends, n=len(content), used=used,
-                lens=lens, tables=tables, nsel=len(raw))
+    return np.concatenate([head, data]), len(head) + ends
 
 
 def make_stream(level, blocks):
