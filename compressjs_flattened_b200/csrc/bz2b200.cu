@@ -35,6 +35,29 @@
 
 namespace {
 
+// ---- bzip2 stream framing, host side (k_stream_ends writes the same header and footer on the device) ----------
+// header: "BZh" and the level digit (BJ:2223-2226)
+static void stream_header(u8 *h, int level) { h[0] = 'B'; h[1] = 'Z'; h[2] = 'h'; h[3] = (u8)('0' + level); }
+// the 4 bytes at h start with "BZh", whatever the level digit
+static bool stream_header_magic(const u8 *h) { return h[0] == 'B' && h[1] == 'Z' && h[2] == 'h'; }
+// the level of the 4-byte header at h, 0 if it is not a header (BJ:1408-1427)
+static int stream_header_level(const u8 *h) { return stream_header_magic(h) && h[3] >= '1' && h[3] <= '9' ? h[3] - '0' : 0; }
+// the combined CRC after `blocks` more blocks whose own combined CRC, counted from 0, is `fold` (BJ:2237)
+static u32 stream_crc_add(u32 crc, u32 blocks, u32 fold) {
+  const u32 m = blocks & 31u;
+  return (m ? (crc << m) | (crc >> (32 - m)) : crc) ^ fold;
+}
+// footer: the end-of-stream magic and the combined CRC, 80 bits ORed into dst from bit `bitpos` on (the caller clears
+// those bytes); returns the bit after it (BJ:2245-2247)
+static u64 stream_footer(u8 *dst, u64 bitpos, u32 crc) {
+  const u64 vals[2] = {BZ_MAGIC_END, (u64)crc};
+  const int lens[2] = {48, 32};
+  for (int q = 0; q < 2; q++)
+    for (int i = lens[q] - 1; i >= 0; i--, bitpos++)
+      if ((vals[q] >> i) & 1) dst[bitpos >> 3] |= (u8)(0x80u >> (bitpos & 7));
+  return bitpos;
+}
+
 // ---- results handed to the caller ------------------------------------------------------------
 // Large results live in page-locked memory (the device-to-host copy then runs at PCIe speed instead of through
 // the driver's pageable staging).  bz2b200_free() recognises them and keeps a few for reuse, so a caller that
@@ -763,8 +786,7 @@ int pipe_run(Ctx *c, u64 base_bits, bool whole, u32 *d_out, size_t out_cap, bool
     u32 foldb = 0;
     if ((rc = pipe_emit_part(c, running, b0 == 0, d_out, out_cap, &bits, &foldb))) return rc;
     CK(cudaMemcpyAsync(P<BlockRec>(c->recs_all) + b0, c->recs.p, sizeof(BlockRec) * (size_t)bn, cudaMemcpyDeviceToDevice, c->stream));
-    const u32 m = (u32)bn & 31u;
-    fold = (m ? ((fold << m) | (fold >> (32 - m))) : fold) ^ foldb;  // BJ:2237 over the batch's blocks
+    fold = stream_crc_add(fold, (u32)bn, foldb);
     running += bits;
     {
       std::vector<BlockMeta> hm((size_t)bn);
@@ -808,6 +830,19 @@ int compress_device(Ctx *c, const u8 *d_in, size_t n_, int level, u32 *d_out, si
   rc = pipe_run(c, 32, true, d_out, out_cap, own_out, out_len, nullptr, nullptr);
   trace_report(c);
   return rc;
+}
+
+// the segment of `bits` bits that pipe_run left in c->out, moved to start at bit `phase` of its first byte (into
+// c->out2 when phase > 0): *d_seg = its (phase + bits + 7) / 8 bytes on the device
+int seg_shift(Ctx *c, u64 bits, u32 phase, const u8 **d_seg) {
+  const u64 nsrc = (bits + 7) / 8;
+  *d_seg = P<u8>(c->out);
+  if (phase && bits) {
+    ENS(c->out2, nsrc + 16);
+    LAUNCH(k_shift_bytes, (unsigned)((nsrc + 256) / 256), 256, 0, P<u8>(c->out), nsrc, phase, P<u8>(c->out2));
+    *d_seg = P<u8>(c->out2);
+  }
+  return 0;
 }
 
 #include "decode_host.inl"
@@ -1012,14 +1047,10 @@ int bz2b200_shard_emit(bz2b200_ctx *ctx, int bit_phase, bz2b200_shard_info *info
   Ctx *c = reinterpret_cast<Ctx *>(ctx);
   if (!c || !info || !seg_bytes || bit_phase < 0 || bit_phase > 7) return BZ2B200_E_ARG;
   CK(cudaSetDevice(c->device));
-  const u64 bits = c->shard_bits, nsrc = (bits + 7) / 8;
+  const u64 bits = c->shard_bits;
   const size_t olen = (size_t)(((u64)bit_phase + bits + 7) / 8);
-  const u8 *d_seg = P<u8>(c->out);
-  if (bit_phase && bits) {
-    ENS(c->out2, nsrc + 16);
-    LAUNCH(k_shift_bytes, (unsigned)((nsrc + 256) / 256), 256, 0, P<u8>(c->out), nsrc, (u32)bit_phase, P<u8>(c->out2));
-    d_seg = P<u8>(c->out2);
-  }
+  const u8 *d_seg = nullptr;
+  RC(seg_shift(c, bits, (u32)bit_phase, &d_seg));
   CK(cudaStreamSynchronize(c->stream));
   info->bit_phase = (uint32_t)bit_phase;
   *seg_bytes = olen;
@@ -1041,7 +1072,7 @@ int bz2b200_stitch_shards(int level, int n_shards, const uint8_t *const *segs, c
   size_t nbytes = (size_t)((total_bits + 80 + 7) / 8);
   uint8_t *o = (uint8_t *)calloc(nbytes + 8, 1);
   if (!o) return BZ2B200_E_OUT_OF_MEMORY;
-  o[0] = 'B'; o[1] = 'Z'; o[2] = 'h'; o[3] = (uint8_t)('0' + level);  // BJ:2223-2226
+  stream_header(o, level);
   u64 bitpos = 32;
   u32 crc = 0;
   for (int r = 0; r < n_shards; r++) {
@@ -1052,14 +1083,9 @@ int bz2b200_stitch_shards(int level, int n_shards, const uint8_t *const *segs, c
       if (len > 1) memcpy(o + off + 1, segs[r] + 1, len - 1);
       bitpos += infos[r].bits;
     }
-    u32 m = infos[r].n_blocks & 31u;
-    crc = (m ? ((crc << m) | (crc >> (32 - m))) : crc) ^ infos[r].crc_fold;  // BJ:2237 over the shard's blocks
+    crc = stream_crc_add(crc, infos[r].n_blocks, infos[r].crc_fold);
   }
-  u64 vals[2] = {BZ_MAGIC_END, (u64)crc};  // BJ:2245-2247
-  int lens[2] = {48, 32};
-  for (int q = 0; q < 2; q++)
-    for (int i = lens[q] - 1; i >= 0; i--, bitpos++)
-      if ((vals[q] >> i) & 1) o[bitpos >> 3] |= (uint8_t)(0x80u >> (bitpos & 7));
+  bitpos = stream_footer(o, bitpos, crc);
   *out = o;
   *out_len = (size_t)((bitpos + 7) / 8);
   return BZ2B200_OK;

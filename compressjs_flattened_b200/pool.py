@@ -32,6 +32,23 @@ def bind_thread_to_device(device, library=None):
     return int(lib.L.bz2b200_bind_thread_to_device(int(device)))
 
 
+def _shard_jobs(jobs):
+    """jobs (dicts {src, n_readable, own_len, base, index, on_device}) as a bz2b200_shard_job array, and the host
+    arrays it points into (keep them alive for the call)."""
+    arr = (_native.ShardJob * max(len(jobs), 1))()
+    keep = []
+    for i, j in enumerate(jobs):
+        src = j["src"]
+        if j.get("on_device"):
+            ptr, nr = int(src), int(j["n_readable"])
+        else:
+            a = src if isinstance(src, np.ndarray) else _coerce_input(src)
+            keep.append(a)
+            ptr, nr = a.ctypes.data, int(j.get("n_readable", a.size))
+        arr[i] = _native.ShardJob(ptr, nr, int(j["own_len"]), int(j["base"]), int(j["index"]), int(bool(j.get("on_device"))))
+    return arr, keep
+
+
 class ShardGroup:
     def __init__(self, name, rank, world, timeout_ms=120_000, library=None):
         self._lib = library or _native.default_library()
@@ -157,17 +174,7 @@ class Bzip2Pool:
         on_device}.  Returns [(bytes | pointer | None, out_offset, n_bytes, rc, n_blocks)] per job; the stream's status is
         the first non-zero rc in slice order over ALL ranks."""
         n = len(jobs)
-        arr = (_native.ShardJob * max(n, 1))()
-        keep = []
-        for i, j in enumerate(jobs):
-            src = j["src"]
-            if j.get("on_device"):
-                ptr, nr = int(src), int(j["n_readable"])
-            else:
-                a = src if isinstance(src, np.ndarray) else _coerce_input(src)
-                keep.append(a)
-                ptr, nr = a.ctypes.data, int(j.get("n_readable", a.size))
-            arr[i] = _native.ShardJob(ptr, nr, int(j["own_len"]), int(j["base"]), int(j["index"]), int(bool(j.get("on_device"))))
+        arr, keep = _shard_jobs(jobs)
         res = (_native.RangeResult * max(n, 1))()
         rc = self._L.bz2b200_pool_decompress_shards(self._p, group._g if group is not None else None, arr, n, total_shards, int(total_n),
                                                     int(first_level), int(bool(multistream)), int(bool(keep_on_device)), res)
@@ -189,17 +196,7 @@ class Bzip2Pool:
         """jobs: list of dicts {src: bytes-like or device pointer (int), n_readable, own_len, base, index, on_device}.
         Returns a list of (segment, ShardResult): segment = bytes (to_bytes), a raw pointer, or None (keep_on_device)."""
         n = len(jobs)
-        arr = (_native.ShardJob * max(n, 1))()
-        keep = []
-        for i, j in enumerate(jobs):
-            src = j["src"]
-            if j.get("on_device"):
-                ptr, nr = int(src), int(j["n_readable"])
-            else:
-                a = src if isinstance(src, np.ndarray) else _coerce_input(src)
-                keep.append(a)
-                ptr, nr = a.ctypes.data, int(j.get("n_readable", a.size))
-            arr[i] = _native.ShardJob(ptr, nr, int(j["own_len"]), int(j["base"]), int(j["index"]), int(bool(j.get("on_device"))))
+        arr, keep = _shard_jobs(jobs)
         res = (_native.ShardResult * max(n, 1))()
         rc = self._L.bz2b200_pool_compress_shards(self._p, group._g if group is not None else None, arr, n, total_shards, level,
                                                   int(bool(keep_on_device)), res)
