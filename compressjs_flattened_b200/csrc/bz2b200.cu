@@ -135,7 +135,7 @@ struct Ctx {
   DevBuf Lcol, ranks, lastocc, A, freq, meta, W, bit_off, scrc, out, out_len, used_bits;
   DevBuf gbounds;
   DevBuf key2, big_cnt, big_old, big_rank, big_tile0, big_tblk, totals2;
-  DevBuf recs_cand, cand_first, out2, recs_all, blksort, r2_status, hfreq, hlens, hplen, hcodes, hsel, hcost, hgoff, hblk;
+  DevBuf recs_cand, cand_first, out2, blksort, r2_status, hfreq, hlens, hplen, hcodes, hsel, hcost, hgoff, hblk;
   // decode-side buffers
   DevBuf d_in, cand, ncand, dmeta, dsyms, dL, dtt, dwalk, dblk, dout, dmisc, dsel, doff, dperm, dmap;
   DevBuf dpieces, dgather;  // range reads: the pieces and the packed bytes (search: the lines)
@@ -174,7 +174,6 @@ struct Ctx {
   u64 shard_bits = 0;      // bit length of the last shard segment (phase 0 in `out`)
   int cand_n = 0, cand_max_blocks = 0, cand_nb[64];  // speculated cut walks of the last shard_cut_g
   i64 cand_s[64];
-  bool recs_batched = false;  // the last call ran in batches: the full block table is in recs_all
   int last_nb = 0;
   i64 last_bs = 0, last_as = 0, last_ss = 0;
   cudaEvent_t ev[10]{};
@@ -187,7 +186,7 @@ struct Ctx {
                      &seg_cnt, &seg_tile0, &tile_blk, &tile_i0, &tile_i1, &totals,
                      &Lcol, &ranks, &lastocc, &A, &freq, &meta, &W, &bit_off, &scrc, &out, &out_len, &used_bits,
                      &gbounds, &key2, &big_cnt, &big_old, &big_rank, &big_tile0, &big_tblk, &totals2,
-                     &recs_cand, &cand_first, &out2, &recs_all, &blksort, &r2_status, &hfreq, &hlens, &hplen, &hcodes, &hsel, &hcost, &hgoff, &hblk,
+                     &recs_cand, &cand_first, &out2, &blksort, &r2_status, &hfreq, &hlens, &hplen, &hcodes, &hsel, &hcost, &hgoff, &hblk,
                      &d_in, &cand, &ncand, &dmeta, &dsyms, &dL, &dtt, &dwalk, &dblk, &dout, &dmisc, &dsel, &doff, &dperm, &dmap,
                      &dpieces, &dgather, &dspat, &dstile, &dsbase, &dstsum, &dsmatch, &dspart, &dstot};
     for (DevBuf *b : all) pool.push_back(b);
@@ -340,8 +339,8 @@ int mark(Ctx *c, int i) {
 // ------------------------------------------------------------------------------ compress
 // The pipeline is split so that a multi-GPU caller can interleave it with the two scalar exchanges of
 // SURVEY section 8e: pipe_begin (tile summaries; independent of where the first block starts), pipe_cut
-// (the sequential cut walk from a known first-block offset), pipe_stages (everything per block) and
-// pipe_emit (bit-granular stitch at a given bit offset).
+// (the sequential cut walk from a known first-block offset) and pipe_run (pipe_stages, everything per block, then the
+// bit-granular stitch at a given bit offset, batch by batch).
 int pipe_begin(Ctx *c, const u8 *d_in, size_t n_, int level) {
   if (level < 1 || level > 9) return BZ2B200_E_LEVEL;
   c->st = bz2b200_stats{};
@@ -428,13 +427,14 @@ bool pipe_pick(Ctx *c, i64 s_local, i64 own_end, int &rc) {
   return false;
 }
 
-int pipe_stages(Ctx *c) {
+// the stages of blocks first .. first + nb - 1 of the block table
+int pipe_stages(Ctx *c, int first, int nb) {
   Ctx::Pipe &P_ = c->pipe;
   const i64 N = P_.N, T = P_.T;
   const u32 B = P_.B;
-  const int nb = P_.nb;
   const u8 *d_in = P_.d_in;
-  std::vector<BlockRec> &hrecs = P_.hrecs;
+  const BlockRec *hrecs = P_.hrecs.data() + first;
+  BlockRec *recs = P<BlockRec>(c->recs) + first;
   int rc;
   const i64 BS = round_up((i64)B + 1, 256);  // per-block stride of byte arrays (block, L, ranks)
   const i64 AS = round_up((i64)B + 2, 128);  // per-block stride of the u16 symbol array
@@ -448,12 +448,12 @@ int pipe_stages(Ctx *c) {
   if (nb) {
     // ---- S1 emit + CRC ----
     ENS(c->blk, (size_t)nb * BS);
-    const i64 t_first = hrecs.front().s / RLE_TILE, t_last = (hrecs.back().p + RLE_TILE - 1) / RLE_TILE;
+    const i64 t_first = hrecs[0].s / RLE_TILE, t_last = (hrecs[nb - 1].p + RLE_TILE - 1) / RLE_TILE;
     (void)T;
-    LAUNCH(k_rle_emit, (unsigned)(t_last - t_first), RLE_THREADS, 0, d_in, N, B, P<i64>(c->head_carry), P<u64>(c->g_tile), P<BlockRec>(c->recs), nb,
+    LAUNCH(k_rle_emit, (unsigned)(t_last - t_first), RLE_THREADS, 0, d_in, N, B, P<i64>(c->head_carry), P<u64>(c->g_tile), recs, nb,
            P<u8>(c->blk), BS, t_first);
     i64 max_len = 0;
-    for (auto &r : hrecs) { if (r.p - r.s > max_len) max_len = r.p - r.s; c->st.rle1_bytes += r.n; }
+    for (int k = 0; k < nb; k++) { const BlockRec &r = hrecs[k]; if (r.p - r.s > max_len) max_len = r.p - r.s; c->st.rle1_bytes += r.n; }
     int max_chunks = (int)((max_len + CRC_CHUNK - 1) / CRC_CHUNK);
     ENS(c->crcpart, 4 * (size_t)nb * max_chunks);
     if (!c->pow256.p) {
@@ -462,15 +462,15 @@ int pipe_stages(Ctx *c) {
       for (int j = 0; j < 256; j++) h[j] = crc_xpow(8ull * 256 * (u64)j);
       CK(cudaMemcpy(c->pow256.p, h, sizeof h, cudaMemcpyHostToDevice));
     }
-    LAUNCH(k_crc_chunks, dim3((unsigned)max_chunks, (unsigned)nb), 256, 0, d_in, P<BlockRec>(c->recs), P<u32>(c->pow256), P<u32>(c->crcpart),
+    LAUNCH(k_crc_chunks, dim3((unsigned)max_chunks, (unsigned)nb), 256, 0, d_in, recs, P<u32>(c->pow256), P<u32>(c->crcpart),
            max_chunks);
-    LAUNCH(k_crc_fold, (unsigned)((nb + 127) / 128), 128, 0, P<BlockRec>(c->recs), nb, P<u32>(c->crcpart), max_chunks,
+    LAUNCH(k_crc_fold, (unsigned)((nb + 127) / 128), 128, 0, recs, nb, P<u32>(c->crcpart), max_chunks,
            crc_xpow(8ull * CRC_CHUNK));
     if ((rc = mark(c, 1))) return rc;
 
     // ---- S2 BWT ----
     size_t slots = 0;
-    for (auto &r : hrecs) slots += (size_t)round_up(r.n, SORT_TILE);
+    for (int k = 0; k < nb; k++) slots += (size_t)round_up(hrecs[k].n, SORT_TILE);
     const size_t tiles0 = slots / SORT_TILE;
     if ((u64)nb * (u64)BS >= (1ull << 31)) { c->err = "too many bytes for one call (block table * stride must stay below 2^31)"; return BZ2B200_E_ARG; }
     const size_t big_tiles = 5 * tiles0 + 16;                // big groups have > RF_T0 slots each
@@ -494,15 +494,15 @@ int pipe_stages(Ctx *c) {
     u32 *lbm = P<u32>(c->lbm);  // [0] tile ticket, [1] length of the list being written, [2] big groups of the round
     u64 *status = P<u64>(c->lb_status);
     const u64 magic = ~0ull / (u64)BS + 1;  // gidx / BS == umul64hi(gidx, magic) for gidx < 2^32
-    LAUNCH(k_seg_init, (unsigned)((nb + 255) / 256), 256, 0, P<BlockRec>(c->recs), nb, seg_cnt);
+    LAUNCH(k_seg_init, (unsigned)((nb + 255) / 256), 256, 0, recs, nb, seg_cnt);
     LAUNCH(k_tilemap, 1, 1024, 0, seg_cnt, nb, tile0, tblk, P<u64>(c->totals));
     const unsigned Ta = (unsigned)tiles0;
     ENS(c->blksort, sizeof(BlkSort) * (size_t)nb);
     CK(cudaMemsetAsync(c->blksort.p, 0, sizeof(BlkSort) * (size_t)nb, c->stream));
-    LAUNCH(k_sym_used, dim3(32, (unsigned)nb), 256, 0, P<u8>(c->blk), BS, P<BlockRec>(c->recs), P<BlkSort>(c->blksort));
+    LAUNCH(k_sym_used, dim3(32, (unsigned)nb), 256, 0, P<u8>(c->blk), BS, recs, P<BlkSort>(c->blksort));
     LAUNCH(k_sym_tab, (unsigned)nb, 256, 0, P<BlkSort>(c->blksort));
     u64 total_n = 0;
-    for (auto &r : hrecs) total_n += r.n;
+    for (int k = 0; k < nb; k++) total_n += hrecs[k].n;
     c->dom_used = 0;
     auto timed_scatter = [&](bool bits9, unsigned grid, const u64 *ki, u64 *ko, const u32 *scnt, const u32 *st0, const u32 *stb, int shift,
                              const u32 *sbase, u64 slots_now) -> int {
@@ -529,7 +529,7 @@ int pipe_stages(Ctx *c) {
       c->st.sort_slots += (u64)Ta * SORT_TILE;
       CK(cudaMemsetAsync(lbm, 0, 16, c->stream));
       CK(cudaMemsetAsync(status, 0, 8 * (size_t)Ta, c->stream));
-      LAUNCH(k_keys_init, Ta, SEG_THREADS, 0, P<u8>(c->blk), BS, P<BlockRec>(c->recs), tile0, tblk, P<BlkSort>(c->blksort), kA, P<u32>(c->hist));
+      LAUNCH(k_keys_init, Ta, SEG_THREADS, 0, P<u8>(c->blk), BS, recs, tile0, tblk, P<BlkSort>(c->blksort), kA, P<u32>(c->hist));
       u64 *ki = kA, *ko = kB;
       for (int pass = 0; pass * 9 < KEY_BITS; pass++) {  // bits 20 .. 20 + KEY_BITS, 9 bits a pass
         if (pass) LAUNCH(k_rs_hist<9>, Ta, SORT_THREADS, 0, ki, seg_cnt, tile0, tblk, 20 + pass * 9, P<u32>(c->hist), (const u32 *)nullptr);  // pass 0: k_keys_init
@@ -538,13 +538,13 @@ int pipe_stages(Ctx *c) {
         u64 *tk = ki; ki = ko; ko = tk;
       }
       LAUNCH(k_rank0, Ta, R0_THREADS, 0, ki, seg_cnt, tile0, tblk, P<u32>(c->isa), BS, actI[0], actR[0], status, lbm, lbm + 1, (u32)Ta, P<u8>(c->blk),
-             P<u8>(c->Lcol), P<BlockRec>(c->recs));
+             P<u8>(c->Lcol), recs);
       RC(rb_add(c, hv, lbm, sizeof hv));
       RC(rb_sync(c));
     }
     // ---- rounds >= 1 (refine.cuh): list A (+ key2) -> sorted staging list B -> compacted list A ----
     u32 n_act = hv[1], round = 0;  // doubling round r compares h = L << r symbols further on (L per block)
-    if (n_act) LAUNCH(k_keys2, (n_act + 255) / 256, 256, 0, actI[0], n_act, P<BlockRec>(c->recs), P<u32>(c->isa), (u32)BS, magic, P<BlkSort>(c->blksort), round,
+    if (n_act) LAUNCH(k_keys2, (n_act + 255) / 256, 256, 0, actI[0], n_act, recs, P<u32>(c->isa), (u32)BS, magic, P<BlkSort>(c->blksort), round,
                       P<u32>(c->key2));
     while (n_act) {
       c->st.sort_rounds++;
@@ -557,7 +557,7 @@ int pipe_stages(Ctx *c) {
       LAUNCH(k_group_bounds, (ntiles + 1 + 7) / 8, 256, 0, actR[0], n_act, ntiles, gb_lo, gb_lo2, P<u32>(c->big_cnt), P<u32>(c->big_old), P<u32>(c->big_rank),
              lbm + 2, big_cap);
       LAUNCH(k_sort_groups, ntiles, RF_THREADS, sizeof(RfSmem), P<u32>(c->key2), actI[0], actR[0], n_act, P<u32>(c->isa), (u32)BS, magic, actI[1],
-             actR[1], P<u32>(c->big_cnt), P<u32>(c->big_old), P<u32>(c->big_rank), lbm + 2, big_cap, P<u8>(c->blk), P<u8>(c->Lcol), P<BlockRec>(c->recs),
+             actR[1], P<u32>(c->big_cnt), P<u32>(c->big_old), P<u32>(c->big_rank), lbm + 2, big_cap, P<u8>(c->blk), P<u8>(c->Lcol), recs,
              gb_lo, gb_lo2);
       RC(rb_add(c, hv, lbm, sizeof hv));
       RC(rb_sync(c));
@@ -581,10 +581,10 @@ int pipe_stages(Ctx *c) {
         LAUNCH(k_sub_heads, Tb, SEG_THREADS, 0, ki, bcnt, bt0, btb, P<int>(c->tile_i0), bbase, 32);
         LAUNCH(k_seg_scan, n_big, 256, 0, bt0, 0, P<int>(c->tile_i0), P<int>(c->tile_i1), (u32 *)nullptr);
         LAUNCH(k_big_apply, Tb, SEG_THREADS, 0, ki, bcnt, bt0, btb, bbase, P<u32>(c->big_rank), P<int>(c->tile_i1), P<u32>(c->isa), (u32)BS, magic,
-               actI[1], actR[1], P<u8>(c->blk), P<u8>(c->Lcol), P<BlockRec>(c->recs));
+               actI[1], actR[1], P<u8>(c->blk), P<u8>(c->Lcol), recs);
       }
       round = round < 30 ? round + 1 : round;
-      LAUNCH(k_compact_keys, ctiles, CK_THREADS, 0, actI[1], actR[1], n_act, P<BlockRec>(c->recs), P<u32>(c->isa), (u32)BS, magic, P<BlkSort>(c->blksort), round,
+      LAUNCH(k_compact_keys, ctiles, CK_THREADS, 0, actI[1], actR[1], n_act, recs, P<u32>(c->isa), (u32)BS, magic, P<BlkSort>(c->blksort), round,
              actI[0], actR[0],
              P<u32>(c->key2), status, lbm, lbm + 1, ctiles);
       RC(rb_add(c, hv, lbm, sizeof hv));
@@ -601,17 +601,17 @@ int pipe_stages(Ctx *c) {
     ENS(c->freq, 4 * BZ_MAX_SYMS * (size_t)nb);
     ENS(c->used_bits, 32 * (size_t)nb);
     CK(cudaMemsetAsync(c->used_bits.p, 0, 32 * (size_t)nb, c->stream));
-    LAUNCH(k_mtf_lastocc, dim3((unsigned)((nseg_max + 7) / 8), (unsigned)nb), 256, 0, P<u8>(c->Lcol), BS, P<BlockRec>(c->recs), P<int>(c->lastocc),
+    LAUNCH(k_mtf_lastocc, dim3((unsigned)((nseg_max + 7) / 8), (unsigned)nb), 256, 0, P<u8>(c->Lcol), BS, recs, P<int>(c->lastocc),
            nseg_max * 256, P<u32>(c->used_bits));
-    LAUNCH(k_mtf_scan, (unsigned)nb, 256, 0, P<BlockRec>(c->recs), P<int>(c->lastocc), nseg_max * 256, P<u32>(c->used_bits), P<BlockMeta>(c->meta));
+    LAUNCH(k_mtf_scan, (unsigned)nb, 256, 0, recs, P<int>(c->lastocc), nseg_max * 256, P<u32>(c->used_bits), P<BlockMeta>(c->meta));
     LAUNCH(k_mtf_ranks, dim3((unsigned)((nseg_max + MTR_WARPS - 1) / MTR_WARPS), (unsigned)nb), MTR_WARPS * 32, MTR_WARPS * sizeof(MtrSmem), P<u8>(c->Lcol),
-           BS, P<BlockRec>(c->recs), P<int>(c->lastocc), nseg_max * 256, P<u8>(c->ranks));
+           BS, recs, P<int>(c->lastocc), nseg_max * 256, P<u8>(c->ranks));
     {
       const i64 r2_tiles = (BS + R2_TILE - 1) / R2_TILE;
       ENS(c->r2_status, 8 * (size_t)nb * r2_tiles + 4 * (size_t)nb);
       CK(cudaMemsetAsync(c->r2_status.p, 0, 8 * (size_t)nb * r2_tiles + 4 * (size_t)nb, c->stream));
       CK(cudaMemsetAsync(c->freq.p, 0, 4 * BZ_MAX_SYMS * (size_t)nb, c->stream));
-      LAUNCH(k_mtf_rle2, dim3((unsigned)r2_tiles, (unsigned)nb), R2_THREADS, 0, P<BlockRec>(c->recs), P<u8>(c->ranks), BS, P<u16>(c->A), AS, P<u32>(c->freq),
+      LAUNCH(k_mtf_rle2, dim3((unsigned)r2_tiles, (unsigned)nb), R2_THREADS, 0, recs, P<u8>(c->ranks), BS, P<u16>(c->A), AS, P<u32>(c->freq),
              P<BlockMeta>(c->meta), P<u64>(c->r2_status), r2_tiles, reinterpret_cast<u32 *>(P<u64>(c->r2_status) + (size_t)nb * r2_tiles));
     }
     if ((rc = mark(c, 3))) return rc;
@@ -643,7 +643,7 @@ int pipe_stages(Ctx *c) {
       LAUNCH(k_huf_build, (unsigned)nb, HUF_BT, sizeof(HufBuildSmem), ha);
     }
     LAUNCH(k_huf_assign, ggrid, HUF_GT, 0, ha, P<u16>(c->A), AS, 1);  // BJ:2163
-    LAUNCH(k_huf_codes, (unsigned)nb, HUF_CT, 0, ha, P<BlockRec>(c->recs), P<BlockMeta>(c->meta), P<u32>(c->W), WS);
+    LAUNCH(k_huf_codes, (unsigned)nb, HUF_CT, 0, ha, recs, P<BlockMeta>(c->meta), P<u32>(c->W), WS);
     LAUNCH(k_huf_emit, ggrid, HUF_GT, 0, ha, P<u16>(c->A), AS, P<u32>(c->W), WS);
   } else {
     for (int i = 1; i <= 3; i++) if ((rc = mark(c, i))) return rc;
@@ -653,63 +653,10 @@ int pipe_stages(Ctx *c) {
   return BZ2B200_OK;
 }
 
-// base_bits: 32 for a whole stream (then header and footer are written too), 0..7 for a shard segment
-int pipe_emit(Ctx *c, u64 base_bits, bool whole, u32 *d_out, size_t out_cap, bool own_out, size_t *out_len, u64 *bits_out, u32 *crc_fold) {
-  Ctx::Pipe &P_ = c->pipe;
-  const int nb = P_.nb;
-  LAUNCH(k_stitch_offsets, 1, 1024, 0, P<BlockMeta>(c->meta), P<BlockRec>(c->recs), nb, P<u64>(c->bit_off), P<u32>(c->scrc), base_bits);
-  u64 end_bits = 0;
-  u32 fold = 0;
-  RC(rb_add(c, &end_bits, P<u64>(c->bit_off) + nb, 8));
-  RC(rb_add(c, &fold, c->scrc.p, 4));
-  RC(rb_sync(c));
-  if (bits_out) *bits_out = end_bits - base_bits;
-  if (crc_fold) *crc_fold = fold;
-  size_t need = (size_t)((end_bits + (whole ? 80 : 0) + 7) / 8);
-  size_t need_w = round_up((i64)need, 4) + 8;
-  if (own_out) {
-    ENS(c->out, need_w);
-    d_out = P<u32>(c->out);
-  } else if (out_cap < need_w) {
-    c->err = "output buffer too small";
-    return BZ2B200_E_UNEXPECTED_OUTPUT_EOF;
-  }
-  CK(cudaMemsetAsync(d_out, 0, need_w, c->stream));
-  if (nb) LAUNCH(k_stitch, dim3(32, (unsigned)nb), 256, 0, P<u32>(c->W), P_.WS, P<u64>(c->bit_off), d_out);
-  u64 olen = need;
-  if (whole) {
-    LAUNCH(k_stream_ends, 1, 32, 0, d_out, P<u64>(c->bit_off), nb, P<u32>(c->scrc), P_.level, P<u64>(c->out_len));
-    RC(rb_add(c, &olen, c->out_len.p, 8));
-  }
-  int rc;
-  if ((rc = mark(c, 5))) return rc;
-  RC(rb_sync(c));
-  CK(cudaGetLastError());
-  *out_len = (size_t)olen;
-  c->st.out_bytes = olen;
-  if (nb) {
-    std::vector<BlockMeta> hm((size_t)nb);
-    CK(cudaMemcpy(hm.data(), c->meta.p, sizeof(BlockMeta) * (size_t)nb, cudaMemcpyDeviceToHost));
-    c->st.mtf_syms = 0;
-    for (auto &m : hm) { c->st.mtf_syms += m.m; c->st.d1_triggered |= m.d1; }
-  }
-  if (c->ev_ok) {
-    for (int i = 0; i < 5; i++) CK(cudaEventElapsedTime(&c->st.ms_stage[i], c->ev[i], c->ev[i + 1]));
-    CK(cudaEventElapsedTime(&c->st.ms_total, c->ev[0], c->ev[5]));
-    c->st.dom_ms = 0;
-    for (size_t i = 0; i + 1 < c->dom_used; i += 2) {
-      float ms = 0;
-      CK(cudaEventElapsedTime(&ms, c->dom_ev[i], c->dom_ev[i + 1]));
-      c->st.dom_ms += ms;
-    }
-  }
-  return BZ2B200_OK;
-}
-
 // ---- batches of blocks --------------------------------------------------------------------------
 // The per-block state is ~45 bytes per input byte and global indices are 31 bits, so a call with more blocks than
-// fit is run as consecutive batches of whole blocks: the stages see one batch at a time (c->recs = its slice of the
-// block table) and every batch is stitched behind the previous one at the running bit offset.
+// fit is run as consecutive batches of whole blocks: the stages see one batch at a time (a slice of the block table)
+// and every batch is stitched behind the previous one at the running bit offset.
 int batch_limit(Ctx *c) {
   if (c->batch_override) return (int)c->batch_override;
   const i64 BS = round_up((i64)c->pipe.B + 1, 256);
@@ -730,96 +677,67 @@ int batch_limit(Ctx *c) {
   return (int)(lim < 1 ? 1 : lim);
 }
 
-// one batch: bit offsets from `base_bits`, the output words this batch touches are cleared (the word that holds
-// base_bits keeps the previous batch's bits unless this is the first batch), then the funnel-shift stitch
-int pipe_emit_part(Ctx *c, u64 base_bits, bool first, u32 *d_out, size_t out_cap, u64 *bits_out, u32 *crc_fold) {
-  Ctx::Pipe &P_ = c->pipe;
-  const int nb = P_.nb;
-  LAUNCH(k_stitch_offsets, 1, 1024, 0, P<BlockMeta>(c->meta), P<BlockRec>(c->recs), nb, P<u64>(c->bit_off), P<u32>(c->scrc), base_bits);
-  u64 end_bits = 0;
-  u32 fold = 0;
-  RC(rb_add(c, &end_bits, P<u64>(c->bit_off) + nb, 8));
-  RC(rb_add(c, &fold, c->scrc.p, 4));
-  RC(rb_sync(c));
-  *bits_out = end_bits - base_bits;
-  *crc_fold = fold;
-  const u64 w_first = first ? 0 : (base_bits >> 5) + 1, w_end = ((end_bits + 80 + 31) >> 5) + 2;  // room for the footer too
-  if (w_end * 4 > out_cap) { c->err = "output buffer too small"; return BZ2B200_E_UNEXPECTED_OUTPUT_EOF; }
-  if (w_end > w_first) CK(cudaMemsetAsync(d_out + w_first, 0, (size_t)(w_end - w_first) * 4, c->stream));
-  if (nb) LAUNCH(k_stitch, dim3(32, (unsigned)nb), 256, 0, P<u32>(c->W), P_.WS, P<u64>(c->bit_off), d_out);
-  int rc;
-  if ((rc = mark(c, 5))) return rc;
-  CK(cudaStreamSynchronize(c->stream));
-  CK(cudaGetLastError());
-  return BZ2B200_OK;
-}
-
-// stages + emission of every block in the table, in one batch or several
+// stages + emission of every block in the table, batch by batch.  base_bits: 32 for a whole stream (then header and
+// footer are written too), 0..7 for a shard segment.  The stats of the batches add up in c->st, which pipe_begin cleared.
 int pipe_run(Ctx *c, u64 base_bits, bool whole, u32 *d_out, size_t out_cap, bool own_out, size_t *out_len, u64 *bits_out, u32 *crc_fold) {
   Ctx::Pipe &P_ = c->pipe;
-  const int nb_total = P_.nb, maxb = batch_limit(c);
-  int rc;
-  c->recs_batched = false;
-  if (nb_total <= maxb) {
-    if ((rc = pipe_stages(c))) return rc;
-    return pipe_emit(c, base_bits, whole, d_out, out_cap, own_out, out_len, bits_out, crc_fold);
-  }
-  std::vector<BlockRec> all = P_.hrecs;
-  ENS(c->recs_all, sizeof(BlockRec) * (size_t)nb_total);
-  CK(cudaMemcpyAsync(c->recs_all.p, c->recs.p, sizeof(BlockRec) * (size_t)nb_total, cudaMemcpyDeviceToDevice, c->stream));
-  if (own_out) {
+  const int nb = P_.nb, maxb = batch_limit(c);
+  const bool batched = nb > maxb;
+  if (own_out && batched) {  // sized once: growing it later would drop the bits of the earlier batches
     out_cap = bz2b200_compress_bound((size_t)P_.N, P_.level) + 64;
     ENS(c->out, out_cap);
     d_out = P<u32>(c->out);
   }
-  u64 running = base_bits, mtf_syms = 0;
-  u32 fold = 0, d1 = 0;
-  float ms_stage[5] = {0, 0, 0, 0, 0}, ms_total = 0, dom_ms = 0;
-  for (int b0 = 0; b0 < nb_total; b0 += maxb) {
-    const int bn = nb_total - b0 < maxb ? nb_total - b0 : maxb;
-    CK(cudaMemcpyAsync(c->recs.p, P<BlockRec>(c->recs_all) + b0, sizeof(BlockRec) * (size_t)bn, cudaMemcpyDeviceToDevice, c->stream));
-    P_.hrecs.assign(all.begin() + b0, all.begin() + b0 + bn);
-    P_.nb = bn;
+  u64 end_bits = base_bits, olen = 0;
+  u32 fold = 0;  // combined CRC of the blocks so far
+  int rc, b0 = 0;
+  do {
+    const int bn = nb - b0 < maxb ? nb - b0 : maxb;
     if (b0) { if ((rc = mark(c, 0))) return rc; if ((rc = mark(c, 1))) return rc; }  // S1 of later batches: emit + CRC only, counted from here
-    if ((rc = pipe_stages(c))) return rc;
-    u64 bits = 0;
-    u32 foldb = 0;
-    if ((rc = pipe_emit_part(c, running, b0 == 0, d_out, out_cap, &bits, &foldb))) return rc;
-    CK(cudaMemcpyAsync(P<BlockRec>(c->recs_all) + b0, c->recs.p, sizeof(BlockRec) * (size_t)bn, cudaMemcpyDeviceToDevice, c->stream));
-    fold = stream_crc_add(fold, (u32)bn, foldb);
-    running += bits;
-    {
+    if ((rc = pipe_stages(c, b0, bn))) return rc;
+    const u64 base = end_bits;
+    LAUNCH(k_stitch_offsets, 1, 1024, 0, P<BlockMeta>(c->meta), P<BlockRec>(c->recs) + b0, bn, P<u64>(c->bit_off), P<u32>(c->scrc), base, fold);
+    RC(rb_add(c, &end_bits, P<u64>(c->bit_off) + bn, 8));
+    RC(rb_add(c, &fold, c->scrc.p, 4));
+    RC(rb_sync(c));
+    const size_t need = (size_t)((end_bits + (whole ? 80 : 0) + 7) / 8), need_w = round_up((i64)need, 4) + 8;
+    if (own_out && !batched) {
+      ENS(c->out, need_w);
+      d_out = P<u32>(c->out);
+    } else if (out_cap < need_w) {
+      c->err = "output buffer too small";
+      return BZ2B200_E_UNEXPECTED_OUTPUT_EOF;
+    }
+    // the words this batch touches are cleared; a later batch keeps the word that holds `base` (the earlier bits)
+    const size_t w_first = b0 ? (size_t)(base >> 5) + 1 : 0;
+    CK(cudaMemsetAsync(d_out + w_first, 0, need_w - 4 * w_first, c->stream));
+    if (bn) LAUNCH(k_stitch, dim3(32, (unsigned)bn), 256, 0, P<u32>(c->W), P_.WS, P<u64>(c->bit_off), d_out);
+    olen = need;
+    if (whole && b0 + bn == nb) {
+      LAUNCH(k_stream_ends, 1, 32, 0, d_out, P<u64>(c->bit_off), bn, P<u32>(c->scrc), P_.level, P<u64>(c->out_len));
+      RC(rb_add(c, &olen, c->out_len.p, 8));
+    }
+    if ((rc = mark(c, 5))) return rc;
+    RC(rb_sync(c));
+    CK(cudaGetLastError());
+    if (bn) {
       std::vector<BlockMeta> hm((size_t)bn);
       CK(cudaMemcpy(hm.data(), c->meta.p, sizeof(BlockMeta) * (size_t)bn, cudaMemcpyDeviceToHost));
-      for (auto &mm : hm) { mtf_syms += mm.m; d1 |= mm.d1; }
+      for (auto &m : hm) { c->st.mtf_syms += m.m; c->st.d1_triggered |= m.d1; }
     }
     if (c->ev_ok) {
-      for (int i = 0; i < 5; i++) { float t = 0; CK(cudaEventElapsedTime(&t, c->ev[i], c->ev[i + 1])); ms_stage[i] += t; ms_total += t; }
-      for (size_t i = 0; i + 1 < c->dom_used; i += 2) { float t = 0; CK(cudaEventElapsedTime(&t, c->dom_ev[i], c->dom_ev[i + 1])); dom_ms += t; }
+      float t = 0;
+      for (int i = 0; i < 5; i++) { CK(cudaEventElapsedTime(&t, c->ev[i], c->ev[i + 1])); c->st.ms_stage[i] += t; }
+      CK(cudaEventElapsedTime(&t, c->ev[0], c->ev[5]));
+      c->st.ms_total += t;
+      for (size_t i = 0; i + 1 < c->dom_used; i += 2) { CK(cudaEventElapsedTime(&t, c->dom_ev[i], c->dom_ev[i + 1])); c->st.dom_ms += t; }
     }
-  }
-  P_.hrecs = all;
-  P_.nb = nb_total;
-  c->recs_batched = true;
-  c->st.n_blocks = (u32)nb_total;
-  if (bits_out) *bits_out = running - base_bits;
+    b0 += bn;
+  } while (b0 < nb);
+  if (bits_out) *bits_out = end_bits - base_bits;
   if (crc_fold) *crc_fold = fold;
-  u64 olen = (running + 7) / 8;
-  if (whole) {
-    u64 endb = running;
-    CK(cudaMemcpyAsync(c->bit_off.p, &endb, 8, cudaMemcpyHostToDevice, c->stream));
-    CK(cudaMemcpyAsync(c->scrc.p, &fold, 4, cudaMemcpyHostToDevice, c->stream));
-    LAUNCH(k_stream_ends, 1, 32, 0, d_out, P<u64>(c->bit_off), 0, P<u32>(c->scrc), P_.level, P<u64>(c->out_len));
-    RC(rb_add(c, &olen, c->out_len.p, 8));
-    RC(rb_sync(c));
-  }
   *out_len = (size_t)olen;
   c->st.out_bytes = olen;
-  c->st.mtf_syms = mtf_syms;
-  c->st.d1_triggered = d1;
-  for (int i = 0; i < 5; i++) c->st.ms_stage[i] = ms_stage[i];
-  c->st.ms_total = ms_total;
-  c->st.dom_ms = dom_ms;
   return BZ2B200_OK;
 }
 
@@ -1150,10 +1068,7 @@ long long bz2b200_debug_fetch(bz2b200_ctx *ctx, int what, int blk, void *dst, si
     return (long long)bytes;
   }
   switch (what) {
-    case 0:
-      if (c->recs_batched) { src = c->recs_all.p; bytes = sizeof(BlockRec) * (size_t)c->pipe.nb; }
-      else { src = c->recs.p; bytes = sizeof(BlockRec) * (size_t)nb; }
-      break;
+    case 0: src = c->recs.p; bytes = sizeof(BlockRec) * (size_t)c->pipe.nb; break;
     case 1: src = P<u8>(c->blk) + (i64)blk * c->last_bs; bytes = (size_t)c->last_bs; break;
     case 2: src = P<u8>(c->Lcol) + (i64)blk * c->last_bs; bytes = (size_t)c->last_bs; break;
     case 3: src = P<u16>(c->A) + (i64)blk * c->last_as; bytes = 2 * (size_t)c->last_as; break;

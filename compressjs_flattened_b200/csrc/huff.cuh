@@ -589,9 +589,16 @@ __global__ void __launch_bounds__(HUF_GT) k_huf_emit(HufArrays ha, const u16 *__
 // ---- K-S6: bit-granular concatenation of the per-block streams --------------------------
 // Output bytes are produced as big-endian 32-bit words: bit 31 of word 0 is the first bit.
 // offsets: header is 32 bits, block k starts at 32 + sum(bits[0..k)).
+// A call in several batches passes the running bit offset as base_bits and the combined CRC of the earlier batches
+// as crc_in; stream_crc is then the combined CRC of every block so far.
 __global__ void __launch_bounds__(1024) k_stitch_offsets(const BlockMeta *__restrict__ meta, const BlockRec *__restrict__ recs, int nb,
-                                                         u64 *__restrict__ bit_off, u32 *__restrict__ stream_crc, u64 base_bits) {
+                                                         u64 *__restrict__ bit_off, u32 *__restrict__ stream_crc, u64 base_bits, u32 crc_in) {
   __shared__ u64 ws[33];
+  if (threadIdx.x == 0) {  // before the scan, so that crc_in does not hold a register through it
+    u32 c = crc_in;
+    for (int k = 0; k < nb; k++) c = ((c << 1) | (c >> 31)) ^ recs[k].crc;  // BJ:2237
+    *stream_crc = c;
+  }
   u64 carry = base_bits;  // 32 for a whole stream (after "BZh9"), the bit phase 0..7 for a shard segment
   for (int base = 0; base < nb; base += blockDim.x) {
     int k = base + threadIdx.x;
@@ -600,12 +607,7 @@ __global__ void __launch_bounds__(1024) k_stitch_offsets(const BlockMeta *__rest
     if (k < nb) bit_off[k] = carry + e;
     carry += tot;
   }
-  if (threadIdx.x == 0) {
-    bit_off[nb] = carry;
-    u32 c = 0;
-    for (int k = 0; k < nb; k++) c = ((c << 1) | (c >> 31)) ^ recs[k].crc;  // BJ:2237
-    *stream_crc = c;
-  }
+  if (threadIdx.x == 0) bit_off[nb] = carry;
 }
 __device__ __forceinline__ u32 bswap32(u32 v) { return __byte_perm(v, 0, 0x0123); }
 __global__ void __launch_bounds__(256) k_stitch(const u32 *__restrict__ W, i64 w_stride, const u64 *__restrict__ bit_off, u32 *__restrict__ out) {

@@ -60,7 +60,8 @@ def test_context_pool_equals_oracle(sim_lib, oracle, name):
 
 
 def test_pool_lanes_and_devices(sim_lib, oracle):
-    """an explicit pool: 2 'devices' x 2 lanes, several shard sizes, levels 1 and 9 at the real block sizes"""
+    """an explicit pool: 2 'devices' x 2 lanes, several shard sizes, levels 1 and 9 at the real block sizes; then small
+    blocks in batches of 1 and 3, so that every lane stitches its segment from several batches"""
     from compressjs_flattened_b200.pool import Bzip2Pool
     from compressjs_flattened_b200.corpus import gen_text
     data = gen_text(450_000, 7).tobytes()
@@ -72,6 +73,15 @@ def test_pool_lanes_and_devices(sim_lib, oracle):
         assert pool.compressFile(data, None, 1) == oracle.compress(data, 1)
         with pytest.raises(ValueError):
             pool.compressFile(data, None, 0)
+        pool.set_plan(0, 0.0)
+        oracle.set_block_cap(7001)
+        try:
+            exp = oracle.compress(data[:120_000], 9)
+            for per in (1, 3):
+                pool.debug(block_cap=7001, batch_blocks=per)
+                assert pool.compressFile(data[:120_000], None, 9, shard_bytes=30_000) == exp, per
+        finally:
+            oracle.set_block_cap(0)
     finally:
         pool.close()
 

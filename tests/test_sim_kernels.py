@@ -118,8 +118,29 @@ def test_cut_points_many_tiles_speculation(sim_engine, oracle):
         sim_engine.debug_set_block_cap(0)
 
 
+def _shards_stitched(eng, data, world, halo):
+    """the shard protocol driven in-process: `world` shards compressed one after the other, stitched on the host"""
+    n = len(data)
+    slice_len = (n + world - 1) // world
+    start, bitpos, segs, infos = 0, 32, [], []
+    for r in range(world):
+        base = r * slice_len
+        own = max(0, min(slice_len, n - base))
+        eng.shard_begin(data[base:min(n, base + own + halo)], 9)
+        info = eng.shard_cut(max(start - base, 0), own, r == world - 1)
+        assert info.complete
+        start = max(base + info.next_start, start)
+        eng.shard_compress(info)
+        segs.append(eng.shard_emit(info, bitpos & 7))
+        infos.append(info)
+        bitpos += info.bits
+    return eng.stitch_shards(9, segs, infos)
+
+
 def test_batched_blocks_same_stream(sim_engine, oracle):
-    """More blocks than one batch holds: the batches are stitched behind one another at the running bit offset."""
+    """More blocks than one batch holds: the batches are stitched behind one another at the running bit offset, for a
+    whole stream and for the shard segments of the shard protocol and of the stream compressor."""
+    import io
     data = fixture_bytes("sample5.ref")[:150_000] + bytes(3000) + b"ab" * 4000
     try:
         oracle.set_block_cap(9000)
@@ -130,6 +151,8 @@ def test_batched_blocks_same_stream(sim_engine, oracle):
             assert sim_engine.compressFile(data, None, 9) == exp, per
             starts, lens, crcs = oracle.cut_points(data, 9)
             assert [(r.s, r.n, r.crc) for r in sim_engine.block_table()] == list(zip(starts[:-1], lens, crcs))
+            assert sim_engine.compressStream(io.BytesIO(data), None, 9, chunk_bytes=60_000) == exp, per
+            assert _shards_stitched(sim_engine, data, 2, 20_000) == exp, per
     finally:
         oracle.set_block_cap(0)
         sim_engine.debug_set_block_cap(0)
