@@ -153,6 +153,9 @@ class Library:
                                                      C.POINTER(RangeResult)]
         L.bz2b200_debug_set_decode_batch.argtypes = [vp, vp, C.c_uint32]
         L.bz2b200_debug_set_rle1_threads.argtypes = [vp, vp, C.c_uint32]
+        L.bz2b200_pool_search.argtypes = [vp, vp, C.c_size_t, C.c_int, vp, vp, C.c_size_t, C.c_uint, C.c_uint64, C.c_size_t, C.POINTER(C.POINTER(Match)),
+                                          szp, C.POINTER(SearchTotals), u8pp, szp]
+        L.bz2b200_debug_set_pool_search_tile.argtypes = [vp, C.c_uint32]
         for name in ("zstream", "dstream"):
             getattr(L, f"bz2b200_{name}_open").argtypes = [vp, C.c_int, C.c_size_t, C.POINTER(vp)]
             getattr(L, f"bz2b200_{name}_feed").argtypes = [vp, vp, C.c_size_t, u8pp, szp]

@@ -92,6 +92,33 @@ def _patterns(patterns):
     return pats   # the largest block a stream can have: the buffer of Bzip2Engine.open
 
 
+def _search(owner, fn, handle, input, patterns, ignore_case, max_matches, multistream, lines, *extra):
+    """fn = bz2b200_search or bz2b200_pool_search on `handle` (extra: the arguments between max_matches and the
+    results), its arguments checked and packed and its results unpacked into a SearchResult; errors through owner._raise"""
+    pats = _patterns(patterns)
+    if max_matches is None:
+        max_matches = (1 << 64) - 1
+    elif max_matches < 0:
+        raise ValueError("max_matches must not be negative")
+    max_matches = min(int(max_matches), (1 << 64) - 1)
+    a = _coerce_input(input)
+    packed = np.frombuffer(b"".join(pats), dtype=np.uint8)
+    lens = np.array([len(p) for p in pats], dtype=np.uint32)
+    mp, nm, tot = C.POINTER(_native.Match)(), C.c_size_t(), _native.SearchTotals()
+    lp, nl = C.POINTER(C.c_uint8)(), C.c_size_t()
+    rc = fn(handle, a.ctypes.data, a.size, int(bool(multistream)), packed.ctypes.data, lens.ctypes.data, len(pats),
+            SEARCH_IGNORE_CASE if ignore_case else 0, int(max_matches), *extra, C.byref(mp), C.byref(nm), C.byref(tot),
+            C.byref(lp) if lines else None, C.byref(nl) if lines else None)
+    if rc:
+        owner._raise(rc)
+    try:
+        raw = _native.take_bytes(C.cast(mp, C.POINTER(C.c_uint8)), nm.value * MATCH_DTYPE.itemsize)
+    finally:
+        owner._L.bz2b200_free(mp)
+    text = owner._take(lp, nl.value) if lines else None
+    return SearchResult(np.frombuffer(raw, dtype=MATCH_DTYPE), tot.matches, tot.lines, tot.out_bytes, text)
+
+
 class Bzip2Index:
     """The blocks of a bzip2 file (Bzip2Engine.index): `entries` is a numpy structured array with the layout of
     bz2b200_block_entry -- bit_begin, bit_end, out_offset, out_bytes, crc, stream, level -- one row per block in stream order."""
@@ -469,28 +496,7 @@ class Bzip2Engine:
         holds the first max_matches (None: all) in (offset, pattern) order; total_matches and total_lines count them all.
         lines=True also returns the distinct lines holding a returned match, each ending in '\n' (grep -F's output).
         Decode errors raise Bzip2Error as decompressFile does."""
-        pats = _patterns(patterns)
-        if max_matches is None:
-            max_matches = (1 << 64) - 1
-        elif max_matches < 0:
-            raise ValueError("max_matches must not be negative")
-        max_matches = min(int(max_matches), (1 << 64) - 1)
-        a = _coerce_input(input)
-        packed = np.frombuffer(b"".join(pats), dtype=np.uint8)
-        lens = np.array([len(p) for p in pats], dtype=np.uint32)
-        mp, nm, tot = C.POINTER(_native.Match)(), C.c_size_t(), _native.SearchTotals()
-        lp, nl = C.POINTER(C.c_uint8)(), C.c_size_t()
-        rc = self._L.bz2b200_search(self._ctx, a.ctypes.data, a.size, int(bool(multistream)), packed.ctypes.data, lens.ctypes.data, len(pats),
-                                    SEARCH_IGNORE_CASE if ignore_case else 0, int(max_matches), C.byref(mp), C.byref(nm), C.byref(tot),
-                                    C.byref(lp) if lines else None, C.byref(nl) if lines else None)
-        if rc:
-            self._raise(rc)
-        try:
-            raw = _native.take_bytes(C.cast(mp, C.POINTER(C.c_uint8)), nm.value * MATCH_DTYPE.itemsize)
-        finally:
-            self._L.bz2b200_free(mp)
-        text = self._take(lp, nl.value) if lines else None
-        return SearchResult(np.frombuffer(raw, dtype=MATCH_DTYPE), tot.matches, tot.lines, tot.out_bytes, text)
+        return _search(self, self._L.bz2b200_search, self._ctx, input, patterns, ignore_case, max_matches, multistream, lines)
 
     def debug_set_search_tile(self, nbytes):
         """tests only: bytes per search tile (a multiple of 256 up to 8192; 0 restores the default)"""

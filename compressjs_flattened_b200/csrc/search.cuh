@@ -4,11 +4,16 @@
 // of a CTA owns the CH = tile / SEARCH_THREADS consecutive positions i*CH .. i*CH + CH - 1 of its tile, so that one
 // 32-bit mask per thread describes its newlines and the positions where a match starts.  A match belongs to the tile
 // where it starts; a tile reads up to 255 bytes past its end (the longest pattern), clamped at the output's end.
+// The kernels work on a SLICE of the output (SearchSlice): `own` bytes at global offset `base`, followed in the buffer by
+// what follows them, `avail` bytes in all.  Matches start and newlines count in the own bytes only; the verify may read
+// all of them.  Every position the kernels write is global.  One context searches one slice: base 0, own = avail = n.
 //   k_search_count  per tile: matches, newlines, first / last newline, the lines of its first and last match and the
 //                   distinct lines its matches start in; per thread: (mask of match positions, match count)
 //   k_search_scan   one CTA over the tiles: exclusive sums of matches and newlines, exclusive max of the last newline
 //                   (line_begin), suffix min of the first newline (line_end), exclusive max of the last match line and
-//                   from it the exclusive sum of lines that hold a first match (the rank of a line among those)
+//                   from it the exclusive sum of lines that hold a first match (the rank of a line among those); the
+//                   carries start at a seed (what the slices before and after hold), and the unseeded scan of a slice can
+//                   write the slice's own summary, composed by the host over the slices as this kernel composes tiles
 //   k_search_emit   per tile holding a match of rank < n_ret: the matches in (offset, pattern) order with their line
 //                   fields, and for every returned FIRST_IN_LINE match the piece [line_begin, line_end] of its line
 // The patterns come with a filter: a 65 536-bit table of the first two bytes of the patterns of two bytes or more and a
@@ -45,6 +50,15 @@ struct SearchBase {     // k_search_scan -> k_search_emit
   i64 prev_ml;             // line of the last match before the tile, -1 if none
 };
 struct SearchTotals { u64 matches, lines, pieces, pad; };
+struct SearchSlice {    // the bytes a launch searches: own bytes at global offset base, avail >= own readable, n = global output length
+  u64 base, own, avail, n;
+};
+struct SearchSum {      // a slice as a SearchTile: global first / last newline, 64-bit counts, slice-local lines of its first / last match
+  u64 first_nl;
+  i64 last_nl;
+  u64 matches, nl, lines;
+  i64 first_ml, last_ml;
+};
 struct SearchMatch {    // bz2b200_match, field for field
   u64 offset, line, line_begin, line_end;
   u32 pattern, flags;
@@ -85,7 +99,7 @@ __device__ __forceinline__ bool search_verify(const SearchPats &P, u32 j, const 
 __device__ __forceinline__ u32 search_line_of(u32 nlmask, u32 k) { return __popc(nlmask & ((1u << k) - 1u)); }
 
 // persistent: every CTA loads the filter once and takes tiles blockIdx.x, + gridDim.x, ... (4 CTAs per SM fit 64 registers)
-__global__ void __launch_bounds__(SEARCH_THREADS, 4) k_search_count(const u8 *__restrict__ src, u64 n, u32 tile, u32 n_tiles, SearchPats P,
+__global__ void __launch_bounds__(SEARCH_THREADS, 4) k_search_count(const u8 *__restrict__ src, SearchSlice S, u32 tile, u32 n_tiles, SearchPats P,
                                                                     SearchTile *__restrict__ tiles, uint2 *__restrict__ tsum) {
   __shared__ __align__(16) u8 s[SEARCH_TILE_MAX + SEARCH_HALO];
   __shared__ u32 bg[2048], one[8];
@@ -97,20 +111,20 @@ __global__ void __launch_bounds__(SEARCH_THREADS, 4) k_search_count(const u8 *__
   for (u32 t = blockIdx.x; t < n_tiles; t += gridDim.x) {
     const u64 t0 = (u64)t * tile;
     __syncthreads();  // the previous tile's text is no longer read (and the tables are in place)
-    search_stage(src, n, t0, tile, P.fold, s);
+    search_stage(src, S.avail, t0, tile, P.fold, s);
     const u32 k0 = threadIdx.x * CH;
     u32 nlmask = 0, mmask = 0, cnt = 0;
     for (u32 k = 0; k < CH; k++) {
-      const u64 p = t0 + k0 + k;
-      if (p >= n) break;
+      const u64 p = t0 + k0 + k;  // in the slice
+      if (p >= S.own) break;
       const u32 c = s[k0 + k];
       if (c == '\n') nlmask |= 1u << k;
       u32 m = 0;
       if ((one[c >> 5] >> (c & 31)) & 1u) m += P.one_off[c + 1] - P.one_off[c];
-      if (p + 1 < n) {
+      if (p + 1 < S.avail) {
         const u32 key = (c << 8) | s[k0 + k + 1];
         if ((bg[key >> 5] >> (key & 31)) & 1u)
-          for (u32 q = P.bg_off[key], qe = P.bg_off[key + 1]; q < qe; q++) m += search_verify(P, P.bg_list[q], s + k0 + k, n - p);
+          for (u32 q = P.bg_off[key], qe = P.bg_off[key + 1]; q < qe; q++) m += search_verify(P, P.bg_list[q], s + k0 + k, S.avail - p);
       }
       if (m) { mmask |= 1u << k; cnt += m; }
     }
@@ -130,8 +144,8 @@ __global__ void __launch_bounds__(SEARCH_THREADS, 4) k_search_count(const u8 *__
     }
     if (first_ml >= 0 && first_ml == prev_ml) lines--;  // that line was counted by an earlier chunk of the tile
     const u64 m_tile = block_sum<u64>(cnt, wsu), l_tile = block_sum<u64>(lines, wsu);
-    const i64 first_nl = nlmask ? (i64)(t0 + k0 + __ffs((int)nlmask) - 1) : (i64)n;
-    const i64 last_nl = nlmask ? (i64)(t0 + k0 + 31 - __clz((int)nlmask)) : -1;
+    const i64 first_nl = nlmask ? (i64)(S.base + t0 + k0 + __ffs((int)nlmask) - 1) : (i64)S.n;
+    const i64 last_nl = nlmask ? (i64)(S.base + t0 + k0 + 31 - __clz((int)nlmask)) : -1;
     const i64 fnl = block_min<i64>(first_nl, ws), lnl = block_max<i64>(last_nl, ws);
     const i64 fml = block_min<i64>(first_ml >= 0 ? first_ml : INT64_MAX, ws);
     if (threadIdx.x == 0) {
@@ -144,13 +158,14 @@ __global__ void __launch_bounds__(SEARCH_THREADS, 4) k_search_count(const u8 *__
 }
 
 // one CTA of 1024 threads over the tiles, in rounds of 1024 with carries: forward for the prefix quantities, backward for
-// the suffix min of the first newline
-__global__ void __launch_bounds__(1024) k_search_scan(const SearchTile *__restrict__ tiles, u32 n_tiles, u64 n, SearchBase *__restrict__ base,
-                                                      SearchTotals *__restrict__ tot) {
+// the suffix min of the first newline.  The carries start at `seed` (nothing before: 0, 0, 0, -1, n, -1).  sum != nullptr
+// (unseeded): the slice's summary; its lines are slice-local.  tot: the totals through the slice.
+__global__ void __launch_bounds__(1024) k_search_scan(const SearchTile *__restrict__ tiles, u32 n_tiles, u64 n, SearchBase seed,
+                                                      SearchBase *__restrict__ base, SearchTotals *__restrict__ tot, SearchSum *__restrict__ sum) {
   __shared__ u64 wsu[33];
   __shared__ i64 ws[33];
-  u64 c_match = 0, c_nl = 0, c_line = 0;
-  i64 c_prev_nl = -1, c_prev_ml = -1;
+  u64 c_match = seed.match0, c_nl = seed.nl0, c_line = seed.line0;
+  i64 c_prev_nl = seed.prev_nl, c_prev_ml = seed.prev_ml;
   for (u32 b = 0; b < n_tiles; b += blockDim.x) {
     const u32 t = b + threadIdx.x;
     const bool on = t < n_tiles;
@@ -168,6 +183,7 @@ __global__ void __launch_bounds__(1024) k_search_scan(const SearchTile *__restri
     prev_ml = prev_ml > c_prev_ml ? prev_ml : c_prev_ml;
     const u64 lines = r.lines - (r.first_ml >= 0 && (i64)nl0 + r.first_ml == prev_ml ? 1u : 0u);
     const u64 line0 = c_line + block_excl_sum<u64>(lines, s_line, wsu);
+    if (sum && r.matches && match0 == seed.match0) sum->first_ml = (i64)nl0 + r.first_ml;  // the first tile with a match
     if (on) {
       SearchBase o;
       o.match0 = match0; o.nl0 = nl0; o.line0 = line0; o.prev_nl = prev_nl; o.next_nl = n; o.prev_ml = prev_ml;
@@ -179,7 +195,7 @@ __global__ void __launch_bounds__(1024) k_search_scan(const SearchTile *__restri
   }
   __syncthreads();
   // suffix min as an exclusive max of the negated values with the tiles in descending order
-  i64 c_next = -(i64)n;
+  i64 c_next = -(i64)seed.next_nl;
   for (u32 b = 0; b < n_tiles; b += blockDim.x) {
     const bool on = b + threadIdx.x < n_tiles;
     const u32 t = on ? n_tiles - 1 - (b + threadIdx.x) : 0;
@@ -190,16 +206,24 @@ __global__ void __launch_bounds__(1024) k_search_scan(const SearchTile *__restri
     if (on) base[t].next_nl = (u64)(-e);
     if (m > c_next) c_next = m;
   }
-  if (threadIdx.x == 0) { tot->matches = c_match; tot->lines = c_line; tot->pieces = 0; tot->pad = 0; }
+  if (threadIdx.x == 0) {
+    tot->matches = c_match; tot->lines = c_line; tot->pieces = 0; tot->pad = 0;
+    if (sum) {  // first_ml: written above when the slice has a match
+      sum->first_nl = (u64)(-c_next); sum->last_nl = c_prev_nl; sum->matches = c_match; sum->nl = c_nl; sum->lines = c_line; sum->last_ml = c_prev_ml;
+      if (!c_match) sum->first_ml = -1;
+    }
+  }
 }
 
-// Matches of rank < n_ret, written at their rank; with piece_src != nullptr also the line of every returned FIRST_IN_LINE
-// match as piece (line rank): piece_src = line_begin, piece_len = through its '\n' (to n for a last line without one).
+// Matches of rank < n_ret, match of rank r written at out[r - rank0]; with piece_src != nullptr also the line of every
+// returned FIRST_IN_LINE match as piece (line rank lr at lr - lrank0), clipped to the own bytes: piece_src = its first
+// byte in the slice, piece_len = through its '\n' (to n for a last line without one).
 // tot->pieces = line rank of the match of rank n_ret - 1, plus one.
-__global__ void __launch_bounds__(SEARCH_THREADS) k_search_emit(const u8 *__restrict__ src, u64 n, u32 tile, u32 n_tiles, SearchPats P,
+__global__ void __launch_bounds__(SEARCH_THREADS) k_search_emit(const u8 *__restrict__ src, SearchSlice S, u32 tile, u32 n_tiles, SearchPats P,
                                                                 const SearchTile *__restrict__ tiles, const SearchBase *__restrict__ base,
-                                                                const uint2 *__restrict__ tsum, u64 n_ret, SearchMatch *__restrict__ out,
-                                                                u64 *__restrict__ piece_src, u64 *__restrict__ piece_len, SearchTotals *__restrict__ tot) {
+                                                                const uint2 *__restrict__ tsum, u64 n_ret, u64 rank0, u64 lrank0,
+                                                                SearchMatch *__restrict__ out, u64 *__restrict__ piece_src, u64 *__restrict__ piece_len,
+                                                                SearchTotals *__restrict__ tot) {
   __shared__ __align__(16) u8 s[SEARCH_TILE_MAX + SEARCH_HALO];
   __shared__ i64 ws[33], nxt[SEARCH_THREADS];
   __shared__ u64 wsu[33];
@@ -208,14 +232,14 @@ __global__ void __launch_bounds__(SEARCH_THREADS) k_search_emit(const u8 *__rest
   if (tiles[t].matches == 0 || B.match0 >= n_ret) return;
   const u32 CH = tile / SEARCH_THREADS;
   const u64 t0 = (u64)t * tile;
-  search_stage(src, n, t0, tile, P.fold, s);
+  search_stage(src, S.avail, t0, tile, P.fold, s);
   const u32 k0 = threadIdx.x * CH;
   u32 nlmask = 0;
-  for (u32 k = 0; k < CH && t0 + k0 + k < n; k++)
+  for (u32 k = 0; k < CH && t0 + k0 + k < S.own; k++)
     if (s[k0 + k] == '\n') nlmask |= 1u << k;
   const uint2 ts = tsum[(u64)t * SEARCH_THREADS + threadIdx.x];
   const u32 mmask = ts.x;
-  const u64 pos0 = t0 + k0;
+  const u64 pos0 = S.base + t0 + k0;
   // newlines around the chunk
   u64 nl_tot;
   const u64 line0 = B.nl0 + block_excl_sum<u64>((u64)__popc(nlmask), nl_tot, wsu);
@@ -258,26 +282,28 @@ __global__ void __launch_bounds__(SEARCH_THREADS) k_search_emit(const u8 *__rest
     const bool first = (i64)r.line != prev_ml;
     const u64 lr = first ? lrank : lrank - 1;  // rank of the match's line among the lines that hold a first match
     if (first && piece_src) {
-      piece_src[lr] = r.line_begin;
-      piece_len[lr] = (r.line_end < n ? r.line_end + 1 : n) - r.line_begin;
+      const u64 b = r.line_begin > S.base ? r.line_begin : S.base, e = r.line_end < S.n ? r.line_end + 1 : S.n;
+      piece_src[lr - lrank0] = b - S.base;
+      piece_len[lr - lrank0] = (e < S.base + S.own ? e : S.base + S.own) - b;
     }
     // the patterns at p in ascending index: merge the one-byte list and the list of the first two bytes
     const u8 *sp = s + k0 + k;
     const u32 c = sp[0];
     u32 q1 = P.one_off[c], e1 = P.one_off[c + 1], q2 = 0, e2 = 0;
-    if (p + 1 < n) { const u32 key = (c << 8) | sp[1]; q2 = P.bg_off[key]; e2 = P.bg_off[key + 1]; }
+    const u64 room = S.avail - (p - S.base);
+    if (room > 1) { const u32 key = (c << 8) | sp[1]; q2 = P.bg_off[key]; e2 = P.bg_off[key + 1]; }
     u32 flags = first ? 1u : 0u;
     while (rank < n_ret) {
       u32 j;
       if (q1 < e1 && (q2 >= e2 || P.one_list[q1] < P.bg_list[q2])) j = P.one_list[q1++];
       else if (q2 < e2) {
         j = P.bg_list[q2++];
-        if (!search_verify(P, j, sp, n - p)) continue;
+        if (!search_verify(P, j, sp, room)) continue;
       } else break;
       r.pattern = j;
       r.flags = flags;
       flags = 0;
-      out[rank] = r;
+      out[rank - rank0] = r;
       if (rank == n_ret - 1) tot->pieces = lr + 1;
       rank++;
     }

@@ -12,7 +12,7 @@ import ctypes as C
 import numpy as np
 
 from . import _native
-from .bzip2 import Bzip2Error, _coerce_input, _deliver
+from .bzip2 import Bzip2Error, _coerce_input, _deliver, _search
 
 
 def shard_plan(n, level=9, lanes=2, first_bytes=0, growth=0.0, library=None):
@@ -160,6 +160,17 @@ class Bzip2Pool:
         if rc:
             self._raise(rc)
         return out, n.value
+
+    def search(self, input, patterns, ignore_case=False, max_matches=None, multistream=False, lines=False, slice_bytes=0):
+        """Bzip2Engine.search of ONE stream, decoded and searched slice by slice over the lanes of the pool: the same
+        SearchResult, field for field.  slice_bytes: bytes of stream per slice (0 = as decompressFile picks them)."""
+        return _search(self, self._L.bz2b200_pool_search, self._p, input, patterns, ignore_case, max_matches, multistream, lines, int(slice_bytes))
+
+    def debug_set_search_tile(self, nbytes):
+        """tests only: bytes per search tile of every lane (a multiple of 256 up to 8192; 0 restores the default)"""
+        rc = self._L.bz2b200_debug_set_pool_search_tile(self._p, nbytes)
+        if rc:
+            self._raise(rc)
 
     def debug_decode_batch(self, candidates):
         self._L.bz2b200_debug_set_decode_batch(None, self._p, candidates)

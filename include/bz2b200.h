@@ -141,7 +141,9 @@ int bz2b200_decompress_ranges(bz2b200_ctx *ctx, const uint8_t *in, size_t n, con
  * (for patterns without '\n', what grep -F prints, -i with IGNORE_CASE in the C locale).  *matches and *lines are
  * released with bz2b200_free.  bz2b200_last_stats: n_blocks, in_bytes and out_bytes as bz2b200_decompress; ms_total =
  * device time up to the packed results (their copy to the host is not included); ms_stage[5] = device time of the
- * search kernels and the line gather alone. */
+ * search kernels and the line gather alone.
+ * bz2b200_pool_search (with the shard scheduler below) searches one stream over every lane of a pool and returns what
+ * bz2b200_search returns for the same arguments, byte for byte. */
 #define BZ2B200_SEARCH_IGNORE_CASE 1u      /* ASCII: A-Z equal a-z; every other byte compares as it is */
 #define BZ2B200_MATCH_FIRST_IN_LINE 1u     /* bz2b200_match.flags */
 typedef struct {
@@ -275,6 +277,16 @@ int bz2b200_pool_decompress_shards(bz2b200_pool *pool, bz2b200_group *grp, const
                                    uint64_t total_n, int first_level, int multistream, int keep_on_device, bz2b200_range_result *results);
 int bz2b200_pool_compress_shards(bz2b200_pool *pool, bz2b200_group *grp, const bz2b200_shard_job *jobs, int n_jobs, int total_shards, int level,
                                  int keep_on_device, bz2b200_shard_result *results);
+/* bz2b200_search of ONE stream over the lanes: the slices of bz2b200_pool_decompress (slice_bytes = 0 picks them) are
+ * decoded and searched on their lanes, and the host composes the per-slice counts into global ranks, line numbers and
+ * lines.  Matches, totals, lines, return codes and argument-error texts (bz2b200_pool_last_error) equal bz2b200_search's
+ * on one context; a damaged stream gives bz2b200_pool_decompress's error.  Each slice's decoded bytes stay on its lane's
+ * device until the call ends, so a device holds its lanes' share of the output (all of it with one device).
+ * bz2b200_pool_last_stats: n_blocks, in_bytes and out_bytes as bz2b200_pool_decompress, ms_total = host wall time of the
+ * call, ms_stage[5] = device time of the search kernels and line gathers, summed over the lanes. */
+int bz2b200_pool_search(bz2b200_pool *pool, const uint8_t *in, size_t n, int multistream, const uint8_t *patterns, const uint32_t *pattern_lens,
+                        size_t n_patterns, unsigned flags, uint64_t max_matches, size_t slice_bytes, bz2b200_match **matches, size_t *n_matches,
+                        bz2b200_search_totals *totals, uint8_t **lines, size_t *lines_len);
 /* tests/ only: block capacity, blocks per batch, first halo (0 = defaults) and forced staging for every lane of a pool;
  * and for a context: inputs of min_bytes or more go through its own two-lane pool in shards of shard_bytes (0 = auto). */
 int bz2b200_pool_debug(bz2b200_pool *pool, uint32_t block_cap, uint32_t batch_blocks, size_t first_halo, int force_staging);
@@ -283,6 +295,8 @@ int bz2b200_debug_set_decode_batch(bz2b200_ctx *ctx, bz2b200_pool *pool, uint32_
 /* tests/ only: threads per CTA of the RLE1 inverse, 512 or 1024 (0 = 1024 when the batch has no more blocks than the
  * device has SMs, else 512) for a context / every lane of a pool, so that one input reaches both strip widths */
 int bz2b200_debug_set_rle1_threads(bz2b200_ctx *ctx, bz2b200_pool *pool, uint32_t threads);
+/* tests/ only: bz2b200_debug_set_search_tile for every lane of a pool */
+int bz2b200_debug_set_pool_search_tile(bz2b200_pool *pool, uint32_t bytes);
 int bz2b200_debug_set_pool(bz2b200_ctx *ctx, size_t min_bytes, size_t shard_bytes, size_t first_halo, int force_staging);
 
 /* ---- the stream flavour (SURVEY.md 8f N2; csrc/stream_abi.inl) ----
