@@ -4,6 +4,8 @@
   python -m compressjs_flattened_b200 -d|-z [-1 .. -9] [-b <bits>] [-t bzip2] [infile] [outfile]
   python -m compressjs_flattened_b200 -d --list [--multistream] [infile]
   python -m compressjs_flattened_b200 -d --range START:LEN [--index FILE] [--multistream] [infile] [outfile]
+  python -m compressjs_flattened_b200 -d --line-index [--multistream] [infile]
+  python -m compressjs_flattened_b200 -d --lines FIRST:COUNT [--index FILE] [--multistream] [infile] [outfile]
   python -m compressjs_flattened_b200 -d --grep PATTERN [--grep PATTERN ...] [--ignore-case] [--line-number] [--count]
       [--multistream] [infile] [outfile]
 
@@ -22,12 +24,17 @@
       for several), searched on the GPU (Bzip2Engine.search), like bzgrep -F; --ignore-case folds ASCII letters,
       --line-number puts "N:" (1-based) before each line, --count prints the number of matching lines instead.  Exit
       status 0 when a line matched, 1 when none did, as with grep
+  --line-index  print the line index (Bzip2LineIndex.to_text: the --list columns plus the '\n' bytes of every block, under a
+      "# lines" total) to stdout; with --multistream it covers every stream
+  --lines FIRST:COUNT  write COUNT lines from line FIRST (1-based, the numbers --grep --line-number prints), clipped to the
+      output, decoding only the blocks that hold them; --index FILE takes the index from --line-index output, otherwise it
+      is built first (a full decode)
 Usage errors (flags that contradict each other) exit with status 1.
 If <infile> is omitted, reads from stdin; if <outfile> is omitted, writes to stdout.  Needs a CUDA device: no CPU fallback."""
 import argparse
 import sys
 
-from .bzip2 import MATCH_FIRST_IN_LINE, NO_SIGNATURE, Bzip2Index, Err
+from .bzip2 import MATCH_FIRST_IN_LINE, NO_SIGNATURE, Bzip2Index, Bzip2LineIndex, Err
 
 
 def main(argv=None, engine=None):
@@ -47,7 +54,9 @@ def main(argv=None, engine=None):
     ap.add_argument("--recover", action="store_true", help="write the intact blocks of a damaged file, report the damage")
     ap.add_argument("--list", action="store_true", help="with -d: print the block index")
     ap.add_argument("--range", default=None, metavar="START:LEN", help="with -d: write only these decompressed bytes")
-    ap.add_argument("--index", default=None, metavar="FILE", help="with --range: the block index (--list output)")
+    ap.add_argument("--index", default=None, metavar="FILE", help="with --range: the block index (--list output); with --lines: the line index")
+    ap.add_argument("--line-index", action="store_true", help="with -d: print the line index")
+    ap.add_argument("--lines", default=None, metavar="FIRST:COUNT", help="with -d: write COUNT lines from line FIRST (1-based)")
     ap.add_argument("--grep", action="append", default=None, metavar="PATTERN", help="with -d: write the lines that contain PATTERN")
     ap.add_argument("--ignore-case", action="store_true", help="with --grep: ASCII letters match either case")
     ap.add_argument("--line-number", action="store_true", help="with --grep: prefix each line with its 1-based number and ':'")
@@ -57,7 +66,9 @@ def main(argv=None, engine=None):
         if on and not a.grep:
             print(f"{flag} can only be used with --grep", file=sys.stderr)
             return 1
-    for flag, on, verb in (("--list", a.list, "listing"), ("--range", a.range is not None, "reading a range"), ("--grep", bool(a.grep), "searching")):
+    modes = (("--list", a.list, "listing"), ("--range", a.range is not None, "reading a range"), ("--grep", bool(a.grep), "searching"),
+             ("--line-index", a.line_index, "listing lines"), ("--lines", a.lines is not None, "reading lines"))
+    for flag, on, verb in modes:
         if not on:
             continue
         if a.compress:
@@ -73,14 +84,11 @@ def main(argv=None, engine=None):
             print(f"Compression level has no effect when {verb}.", file=sys.stderr)
             return 1
         a.decompress = True
-    if a.list and a.range is not None:
-        print("--list and --range can't be used together", file=sys.stderr)
+    chosen = [flag for flag, on, _ in modes if on]
+    if len(chosen) > 1:
+        print(f"{chosen[0]} and {chosen[1]} can't be used together", file=sys.stderr)
         return 1
-    for flag, on in (("--list", a.list), ("--range", a.range is not None)):
-        if on and a.grep:
-            print(f"{flag} and --grep can't be used together", file=sys.stderr)
-            return 1
-    if a.index is not None and a.range is None:
+    if a.index is not None and a.range is None and a.lines is None:
         print("--index can only be used with --range", file=sys.stderr)
         return 1
     if a.range is not None:
@@ -88,6 +96,14 @@ def main(argv=None, engine=None):
             start, length = (int(v) for v in a.range.split(":"))
         except ValueError:
             print(f"--range takes START:LEN, not {a.range}", file=sys.stderr)
+            return 1
+    if a.lines is not None:
+        try:
+            first, count = (int(v) for v in a.lines.split(":"))
+        except ValueError:
+            first = 0
+        if first < 1:
+            print(f"--lines takes FIRST:COUNT with FIRST from 1, not {a.lines}", file=sys.stderr)
             return 1
     if a.recover:
         if a.compress:
@@ -148,6 +164,20 @@ def main(argv=None, engine=None):
             else:
                 index = Bzip2.index(data, a.multistream)
             dst.write(Bzip2.decompressRange(data, index, start, length))
+        elif a.line_index:
+            dst.write(Bzip2.lineIndex(src.read(), a.multistream).to_text().encode())
+        elif a.lines is not None:
+            data = src.read()
+            if a.index is not None:
+                with open(a.index) as fh:
+                    text = fh.read()
+                if text.startswith(Bzip2Index.HEADER):
+                    print(f"--lines needs a line index (--line-index output), and {a.index} is a block index", file=sys.stderr)
+                    return 1
+                index = Bzip2LineIndex.from_text(text)
+            else:
+                index = Bzip2.lineIndex(data, a.multistream)
+            dst.write(b"".join(Bzip2.decompressLines(data, index, [(first - 1, count)])))
         elif a.grep:
             r = Bzip2.search(src.read(), a.grep, ignore_case=a.ignore_case, max_matches=0 if a.count else None, multistream=a.multistream,
                              lines=not a.count)

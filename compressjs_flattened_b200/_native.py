@@ -105,6 +105,9 @@ class Library:
         L.bz2b200_recover.argtypes = [vp, vp, C.c_size_t, u8pp, szp, C.POINTER(C.POINTER(Region)), szp]
         L.bz2b200_index.argtypes = [vp, vp, C.c_size_t, C.c_int, C.POINTER(C.POINTER(BlockEntry)), szp]
         L.bz2b200_decompress_ranges.argtypes = [vp, vp, C.c_size_t, vp, C.c_size_t, vp, vp, C.c_size_t, u8pp, szp]
+        L.bz2b200_line_index.argtypes = [vp, vp, C.c_size_t, C.c_int, C.POINTER(C.POINTER(BlockEntry)), C.POINTER(C.POINTER(C.c_uint32)), szp,
+                                         C.POINTER(C.c_uint64)]
+        L.bz2b200_decompress_lines.argtypes = [vp, vp, C.c_size_t, vp, vp, C.c_size_t, C.c_uint64, vp, vp, C.c_size_t, u8pp, szp, vp]
         L.bz2b200_search.argtypes = [vp, vp, C.c_size_t, C.c_int, vp, vp, C.c_size_t, C.c_uint, C.c_uint64, C.POINTER(C.POINTER(Match)), szp,
                                      C.POINTER(SearchTotals), u8pp, szp]
         L.bz2b200_free.argtypes = [vp]
@@ -124,6 +127,7 @@ class Library:
         L.bz2b200_debug_set_batch_blocks.argtypes = [vp, C.c_uint32]
         L.bz2b200_debug_set_ignore_block_crc.argtypes = [vp, C.c_int]
         L.bz2b200_debug_set_search_tile.argtypes = [vp, C.c_uint32]
+        L.bz2b200_debug_set_line_tile.argtypes = [vp, C.c_uint32]
         L.bz2b200_debug_huffman_lengths.argtypes = [vp, vp, C.c_int, C.c_int]
         L.bz2b200_shard_begin.argtypes = [vp, vp, C.c_size_t, C.c_int, C.c_int]
         L.bz2b200_shard_cut.argtypes = [vp, C.c_uint64, C.c_uint64, C.c_int, C.POINTER(ShardInfo)]

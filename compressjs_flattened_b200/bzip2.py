@@ -6,6 +6,7 @@
     Bzip2.table(input, callback, multistream=False)           BJ:1823-1863
 
 Random access (no counterpart in the reference): Bzip2Engine.index, decompressRanges, decompressRange and open.
+Lines by number (no counterpart in the reference): Bzip2Engine.lineIndex, decompressLines and lineSpans.
 Search (bzgrep -F, no counterpart in the reference): Bzip2Engine.search.
 
 Same names, argument meaning and error behaviour as the JavaScript API; the work is done by
@@ -141,10 +142,11 @@ class Bzip2Index:
 
     def to_text(self):
         """One line per block under a header line: stream, level, bit_begin, bit_end, out_offset, out_bytes, crc (hex), tab-separated."""
-        lines = [self.HEADER]
+        return "\n".join([self.HEADER] + ["\t".join(r) for r in self._text_rows()]) + "\n"
+
+    def _text_rows(self):
         for e in self.entries:
-            lines.append("\t".join([str(int(e[f])) for f in self._TEXT_FIELDS[:-1]] + [f"{int(e['crc']):08x}"]))
-        return "\n".join(lines) + "\n"
+            yield [str(int(e[f])) for f in self._TEXT_FIELDS[:-1]] + [f"{int(e['crc']):08x}"]
 
     @classmethod
     def from_text(cls, text):
@@ -152,23 +154,79 @@ class Bzip2Index:
         lines = text.splitlines()
         if not lines or lines[0] != cls.HEADER:
             raise ValueError(f"not a block index: the first line must be {cls.HEADER!r}")
-        rows = []
-        for no, line in enumerate(lines[1:], 2):
-            parts = line.split("\t")
-            if len(parts) != len(cls._TEXT_FIELDS):
-                raise ValueError(f"line {no}: {len(parts)} fields, expected {len(cls._TEXT_FIELDS)}")
-            vals = []
-            for name, p in zip(cls._TEXT_FIELDS, parts):
-                digits = "0123456789abcdefABCDEF" if name == "crc" else "0123456789"
-                if not p or any(ch not in digits for ch in p):
-                    raise ValueError(f"line {no}: bad {name} {p!r}")
-                v = int(p, 16 if name == "crc" else 10)
-                if v >= 1 << (INDEX_DTYPE[name].itemsize * 8):
-                    raise ValueError(f"line {no}: {name} {p} out of range")
-                vals.append(v)
-            rec = dict(zip(cls._TEXT_FIELDS, vals))
-            rows.append(tuple(rec[f] for f in INDEX_DTYPE.names))
-        return cls(np.array(rows, dtype=INDEX_DTYPE))
+        return cls(_parse_rows(lines[1:], 2, cls._TEXT_FIELDS)[0])
+
+
+def _parse_rows(lines, first_no, fields):
+    """tab-separated rows of `fields` (those of Bzip2Index._TEXT_FIELDS, then optionally "newlines", a u32), numbered from
+    line first_no -> (the block columns as an INDEX_DTYPE array, the newlines column as uint32 or None); ValueError on
+    anything else"""
+    rows, extra = [], []
+    for no, line in enumerate(lines, first_no):
+        parts = line.split("\t")
+        if len(parts) != len(fields):
+            raise ValueError(f"line {no}: {len(parts)} fields, expected {len(fields)}")
+        vals = []
+        for name, p in zip(fields, parts):
+            digits = "0123456789abcdefABCDEF" if name == "crc" else "0123456789"
+            if not p or any(ch not in digits for ch in p):
+                raise ValueError(f"line {no}: bad {name} {p!r}")
+            v = int(p, 16 if name == "crc" else 10)
+            if v >= 1 << ((INDEX_DTYPE[name].itemsize if name in INDEX_DTYPE.names else 4) * 8):
+                raise ValueError(f"line {no}: {name} {p} out of range")
+            vals.append(v)
+        rec = dict(zip(fields, vals))
+        rows.append(tuple(rec[f] for f in INDEX_DTYPE.names))
+        extra.append(rec.get("newlines", 0))
+    return np.array(rows, dtype=INDEX_DTYPE), (np.array(extra, dtype=np.uint32) if "newlines" in fields else None)
+
+
+class Bzip2LineIndex:
+    """The blocks of a bzip2 file and the '\n' bytes of each (Bzip2Engine.lineIndex): `blocks` is a Bzip2Index,
+    `newlines` a uint32 array with one count per block, `total_lines` the number of lines of the decompressed output (the
+    '\n' bytes, plus one when the output does not end with '\n') and `total` its bytes."""
+    HEADER = "# bzip2 line index v1"
+    _TEXT_FIELDS = Bzip2Index._TEXT_FIELDS + ("newlines",)
+
+    def __init__(self, blocks, newlines, total_lines):
+        self.blocks = blocks if isinstance(blocks, Bzip2Index) else Bzip2Index(blocks)
+        self.newlines = np.ascontiguousarray(newlines, dtype=np.uint32)
+        self.total_lines = int(total_lines)
+        if len(self.newlines) != len(self.blocks):
+            raise ValueError(f"{len(self.newlines)} newline counts for {len(self.blocks)} blocks")
+
+    @property
+    def total(self):
+        """decompressed bytes the index covers"""
+        return self.blocks.total
+
+    def __len__(self):
+        return len(self.blocks)
+
+    def to_text(self):
+        """The header line, "# lines <total_lines>", then one line per block: the columns of Bzip2Index.to_text and the
+        block's '\n' bytes, tab-separated."""
+        rows = (r + [str(int(k))] for r, k in zip(self.blocks._text_rows(), self.newlines))
+        return "\n".join([self.HEADER, f"# lines {self.total_lines}"] + ["\t".join(r) for r in rows]) + "\n"
+
+    @classmethod
+    def from_text(cls, text):
+        """The inverse of to_text; ValueError on anything else, and on counts that do not add up (a count above its
+        block's bytes, or total_lines other than the '\n' bytes, or those + 1 when the last line has no '\n')."""
+        lines = text.splitlines()
+        if not lines or lines[0] != cls.HEADER:
+            raise ValueError(f"not a line index: the first line must be {cls.HEADER!r}")
+        head = lines[1].split(" ") if len(lines) > 1 else []
+        if len(head) != 3 or head[:2] != ["#", "lines"] or not head[2].isascii() or not head[2].isdigit():
+            raise ValueError("line 2: expected '# lines <total_lines>'")
+        entries, newlines = _parse_rows(lines[2:], 3, cls._TEXT_FIELDS)
+        ix = cls(entries, newlines, int(head[2]))
+        nl = int(newlines.sum(dtype=np.uint64))
+        if (newlines > entries["out_bytes"]).any():
+            raise ValueError("a block's newlines exceed its bytes")
+        if ix.total_lines not in ((nl, nl + 1) if nl and ix.total else (1,) if ix.total else (0,)):
+            raise ValueError(f"# lines {ix.total_lines} does not match {nl} '\\n' bytes in {ix.total} bytes")
+        return ix
 
 
 class _RangeReader(io.RawIOBase):
@@ -487,6 +545,59 @@ class Bzip2Engine:
         if index is None:
             index = self.index(a, multistream)
         return io.BufferedReader(_RangeReader(self, a, index), buffer_size=LEVEL9_BLOCK)
+
+    # -- lines by number (include/bz2b200.h, bz2b200_line_index / bz2b200_decompress_lines) --
+    def lineIndex(self, input, multistream=False):
+        """The block index of `input` with the '\n' bytes of every block (a Bzip2LineIndex).  The input is decoded as
+        decompressFile decodes it, with the same errors; the '\n' bytes are counted on the GPU."""
+        a = _coerce_input(input)
+        ptr, nlp, n, lines = C.POINTER(_native.BlockEntry)(), C.POINTER(C.c_uint32)(), C.c_size_t(), C.c_uint64()
+        rc = self._L.bz2b200_line_index(self._ctx, a.ctypes.data, a.size, int(bool(multistream)), C.byref(ptr), C.byref(nlp), C.byref(n), C.byref(lines))
+        if rc:
+            self._raise(rc)
+        try:
+            raw = _native.take_bytes(C.cast(ptr, C.POINTER(C.c_uint8)), n.value * INDEX_DTYPE.itemsize)
+            nl = _native.take_bytes(C.cast(nlp, C.POINTER(C.c_uint8)), n.value * 4)
+        finally:
+            self._L.bz2b200_free(ptr)
+            self._L.bz2b200_free(nlp)
+        return Bzip2LineIndex(Bzip2Index(np.frombuffer(raw, dtype=INDEX_DTYPE)), np.frombuffer(nl, dtype=np.uint32), lines.value)
+
+    def _lines(self, input, index, requests, want_bytes):
+        """bz2b200_decompress_lines over the clipped requests -> (bytes or None, (k, 2) uint64 spans)"""
+        a = _coerce_input(input)
+        ix = index.blocks.entries
+        se = [slice(int(f), int(f) + int(k)).indices(index.total_lines)[:2] for f, k in requests]
+        firsts = np.array([f for f, _ in se], dtype=np.uint64)
+        counts = np.array([max(0, e - f) for f, e in se], dtype=np.uint64)
+        spans = np.zeros((len(se), 2), dtype=np.uint64)
+        out, n = C.POINTER(C.c_uint8)(), C.c_size_t()
+        rc = self._L.bz2b200_decompress_lines(self._ctx, a.ctypes.data, a.size, ix.ctypes.data, index.newlines.ctypes.data, len(ix), index.total_lines,
+                                              firsts.ctypes.data, counts.ctypes.data, len(se), C.byref(out) if want_bytes else None,
+                                              C.byref(n) if want_bytes else None, spans.ctypes.data)
+        if rc:
+            self._raise(rc)
+        return (self._take(out, n.value) if want_bytes else None), spans
+
+    def decompressLines(self, input, index, requests):
+        """The lines of every (first, count) of the decompressed output, 0-based, as a list of bytes in request order.  A
+        request is clipped the way slicing clips lines[first:first + count]; the bytes are as in the output (a last line
+        without '\n' comes back without one).  index: a Bzip2LineIndex.  One call decodes every block that holds a
+        requested line, once, and nothing else (include/bz2b200.h)."""
+        data, spans = self._lines(input, index, requests, True)
+        ends = np.cumsum(spans[:, 1], dtype=np.uint64).tolist()
+        return [data[e - int(ln):e] for e, ln in zip(ends, spans[:, 1].tolist())]
+
+    def lineSpans(self, input, index, requests):
+        """The byte (start, length) of every (first, count) of decompressLines, as a (k, 2) uint64 array: what
+        decompressRanges takes.  Decodes what decompressLines decodes and returns no bytes."""
+        return self._lines(input, index, requests, False)[1]
+
+    def debug_set_line_tile(self, nbytes):
+        """tests only: bytes per newline-directory tile (a multiple of 256 up to 8192; 0 restores the default)"""
+        rc = self._L.bz2b200_debug_set_line_tile(self._ctx, nbytes)
+        if rc:
+            self._raise(rc)
 
     # -- search (include/bz2b200.h, bz2b200_search) --
     def search(self, input, patterns, ignore_case=False, max_matches=None, multistream=False, lines=False):

@@ -12,6 +12,7 @@
 #include "huff.cuh"
 #include "decode.cuh"
 #include "search.cuh"
+#include "lines.cuh"
 
 #include <algorithm>
 #include <atomic>
@@ -140,6 +141,7 @@ struct Ctx {
   DevBuf d_in, cand, ncand, dmeta, dsyms, dL, dtt, dwalk, dblk, dout, dmisc, dsel, doff, dperm, dmap;
   DevBuf dpieces, dgather;  // range reads: the pieces and the packed bytes (search: the lines)
   DevBuf dspat, dstile, dsbase, dstsum, dsmatch, dspart, dstot;  // search: patterns and filter, per-tile and per-thread summaries, matches
+  DevBuf dnltile, dnlpart, dnlq;  // newline directory: tile counts then their prefix, scan partials, queries and their results
   // last compress, for debug_fetch
   struct Pipe {
     const u8 *d_in = nullptr;
@@ -171,6 +173,7 @@ struct Ctx {
   std::vector<u32> dec_last_chain;
   i64 dec_last_bs = 0;
   u32 search_tile = 0;     // tests only: bytes per search tile (0 = SEARCH_TILE_DEFAULT)
+  u32 line_tile = 0;       // tests only: bytes per newline-directory tile (0 = LINE_TILE_DEFAULT)
   u64 shard_bits = 0;      // bit length of the last shard segment (phase 0 in `out`)
   int cand_n = 0, cand_max_blocks = 0, cand_nb[64];  // speculated cut walks of the last shard_cut_g
   i64 cand_s[64];
@@ -188,7 +191,7 @@ struct Ctx {
                      &gbounds, &key2, &big_cnt, &big_old, &big_rank, &big_tile0, &big_tblk, &totals2,
                      &recs_cand, &cand_first, &out2, &blksort, &r2_status, &hfreq, &hlens, &hplen, &hcodes, &hsel, &hcost, &hgoff, &hblk,
                      &d_in, &cand, &ncand, &dmeta, &dsyms, &dL, &dtt, &dwalk, &dblk, &dout, &dmisc, &dsel, &doff, &dperm, &dmap,
-                     &dpieces, &dgather, &dspat, &dstile, &dsbase, &dstsum, &dsmatch, &dspart, &dstot};
+                     &dpieces, &dgather, &dspat, &dstile, &dsbase, &dstsum, &dsmatch, &dspart, &dstot, &dnltile, &dnlpart, &dnlq};
     for (DevBuf *b : all) pool.push_back(b);
   }
 };
@@ -1129,6 +1132,13 @@ int bz2b200_debug_set_search_tile(bz2b200_ctx *ctx, uint32_t bytes) {
   Ctx *c = reinterpret_cast<Ctx *>(ctx);
   if (!c || bytes % SEARCH_THREADS || bytes > SEARCH_TILE_MAX) return BZ2B200_E_ARG;
   c->search_tile = bytes;
+  return BZ2B200_OK;
+}
+
+int bz2b200_debug_set_line_tile(bz2b200_ctx *ctx, uint32_t bytes) {
+  Ctx *c = reinterpret_cast<Ctx *>(ctx);
+  if (!c || bytes % 256 || bytes > LINE_TILE_MAX) return BZ2B200_E_ARG;
+  c->line_tile = bytes;
   return BZ2B200_OK;
 }
 

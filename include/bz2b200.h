@@ -17,6 +17,7 @@
  *   (bzip2recover: no counterpart in BJ)   bz2b200_recover
  *   (random access: no counterpart in BJ)  bz2b200_index / bz2b200_decompress_ranges
  *   (bzgrep: no counterpart in BJ)         bz2b200_search
+ *   (sed -n by line: no counterpart in BJ) bz2b200_line_index / bz2b200_decompress_lines
  */
 #ifndef BZ2B200_H
 #define BZ2B200_H
@@ -127,6 +128,32 @@ typedef struct {
 int bz2b200_index(bz2b200_ctx *ctx, const uint8_t *in, size_t n, int multistream, bz2b200_block_entry **entries, size_t *count);
 int bz2b200_decompress_ranges(bz2b200_ctx *ctx, const uint8_t *in, size_t n, const bz2b200_block_entry *index, size_t count,
                               const uint64_t *starts, const uint64_t *lens, size_t n_ranges, uint8_t **out, size_t *out_len);
+
+/* Lines by number.  Line i (0-based) of the decompressed output (streams concatenated) runs from just after the i-th '\n'
+ * (or from byte 0) through the next '\n', or to the output's end for a last line without one; only '\n' ends a line.
+ * total_lines = the '\n' bytes, plus 1 when the output is not empty and its last byte is not '\n' (0 for an empty output).
+ * bz2b200_line_index decodes the input exactly as bz2b200_decompress(ctx, in, n, multistream) decodes it -- same walk,
+ * block and stream CRC checks, error codes -- so the whole output must fit in device memory, as for bz2b200_search.  It
+ * returns the block index (*entries equals bz2b200_index's for an intact input) and, in a parallel array, the '\n' bytes of
+ * every block; *entries and *newlines are released with bz2b200_free.  The '\n' bytes are counted on the GPU where the
+ * decode leaves the output, by a newline directory (per-tile counts and their prefix, rank and select queries).
+ * bz2b200_decompress_lines returns the lines [firsts[i], firsts[i] + counts[i]) for every i, concatenated in request order,
+ * byte for byte as they are in the output (no '\n' is added to a last line without one).  Requests may overlap, repeat,
+ * come in any order, be empty or cover every line.  Only the blocks from the one that holds '\n' firsts[i] - 1 to the one
+ * that holds '\n' firsts[i] + counts[i] - 1 are decoded, each once, as bz2b200_decompress_ranges decodes its covering
+ * blocks (same uploads, checks and error codes).  out == NULL: nothing is gathered or returned (out_len may be NULL too).
+ * spans (NULL: skipped): 2 * n_requests u64, the byte start and length of each request in the output -- what
+ * bz2b200_decompress_ranges takes.  BZ2B200_E_ARG: an entry bz2b200_decompress_ranges rejects, a newlines[i] above
+ * out_bytes, a total_lines other than the sum of newlines[] (or that sum + 1 for a non-empty output; 1 when the sum is 0),
+ * a request past total_lines.  A covered block whose '\n' count differs from newlines[], or a last byte that disagrees with
+ * total_lines, is DATA_ERROR "index does not match the input".  bz2b200_last_stats: n_blocks = blocks decoded, in_bytes =
+ * bytes uploaded, out_bytes = bytes of the requested lines, ms_total as bz2b200_decompress_ranges, ms_stage[5] = device time
+ * of the newline-directory kernels alone (also for bz2b200_line_index). */
+int bz2b200_line_index(bz2b200_ctx *ctx, const uint8_t *in, size_t n, int multistream, bz2b200_block_entry **entries, uint32_t **newlines,
+                       size_t *count, uint64_t *total_lines);
+int bz2b200_decompress_lines(bz2b200_ctx *ctx, const uint8_t *in, size_t n, const bz2b200_block_entry *index, const uint32_t *newlines, size_t count,
+                             uint64_t total_lines, const uint64_t *firsts, const uint64_t *counts, size_t n_requests, uint8_t **out, size_t *out_len,
+                             uint64_t *spans);
 
 /* Fixed-string search of the decompressed output (what bzgrep -F does, without bringing the decoded bytes back).  The
  * input is decoded exactly as bz2b200_decompress(ctx, in, n, multistream) decodes it -- same walk, CRC checks and error
@@ -343,6 +370,8 @@ int bz2b200_debug_set_batch_blocks(bz2b200_ctx *ctx, uint32_t blocks);
 /* tests/ only: bytes per tile of the search kernels, a multiple of 256 up to 8192 (0 = 8192), so that small outputs
  * span many tiles. */
 int bz2b200_debug_set_search_tile(bz2b200_ctx *ctx, uint32_t bytes);
+/* tests/ only: bytes per newline-directory tile (a multiple of 256 up to 8192; 0 = the default, 8192) */
+int bz2b200_debug_set_line_tile(bz2b200_ctx *ctx, uint32_t bytes);
 /* tests/ only: skip the block-CRC comparison of the decoder (BJ:1756-1761), so that what a damaged stream decodes TO
  * can be compared with the oracle.  Not reachable from the environment. */
 int bz2b200_debug_set_ignore_block_crc(bz2b200_ctx *ctx, int on);
