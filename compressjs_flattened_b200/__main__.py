@@ -2,6 +2,7 @@
 (NPM/bin/compressjs:7-33,58,163-180):
 
   python -m compressjs_flattened_b200 -d|-z [-1 .. -9] [-b <bits>] [-t bzip2] [infile] [outfile]
+  python -m compressjs_flattened_b200 -z [-1 .. -9] --index-out FILE [infile] [outfile]
   python -m compressjs_flattened_b200 -d --list [--multistream] [infile]
   python -m compressjs_flattened_b200 -d --range START:LEN [--index FILE] [--multistream] [infile] [outfile]
   python -m compressjs_flattened_b200 -d --line-index [--multistream] [infile]
@@ -10,6 +11,8 @@
       [--multistream] [infile] [outfile]
 
   -z  compress (the default), stream flavour: the input is read piece by piece (bz2b200_zstream_*), level 7 by default
+  --index-out FILE  with -z: also write the line index of the stream being written (the --line-index text) to FILE, built
+      while compressing, with no decode; --range and --lines take it as --index.  The stream itself is unchanged
   -d  decompress the FIRST stream of the input, stream flavour (bz2b200_dstream_*); --multistream decodes all of them
       (an extension: the reference's command line never passes the flag, NPM/bin/compressjs:166)
   -b  with -d: extract the single block whose signature starts at bit <bits> (Bzip2.decompressBlock)
@@ -19,7 +22,8 @@
       stdout; with --multistream it covers every stream
   --range START:LEN  write the decompressed bytes [START, START+LEN), clipped like a slice, decoding only the blocks that
       hold them; --index FILE takes the index from --list output, otherwise it is built first (a full decode).  A negative
-      START (counted from the end, like a slice) must be written --range=START:LEN, since -1 .. -9 are flags
+      START (counted from the end, like a slice) must be written --range=START:LEN, since -1 .. -9 are flags; a line index
+      (--line-index or --index-out output) is accepted as --index too
   --grep PATTERN  write the lines of the decompressed output that contain PATTERN (a fixed string, UTF-8; repeat the flag
       for several), searched on the GPU (Bzip2Engine.search), like bzgrep -F; --ignore-case folds ASCII letters,
       --line-number puts "N:" (1-based) before each line, --count prints the number of matching lines instead.  Exit
@@ -54,7 +58,9 @@ def main(argv=None, engine=None):
     ap.add_argument("--recover", action="store_true", help="write the intact blocks of a damaged file, report the damage")
     ap.add_argument("--list", action="store_true", help="with -d: print the block index")
     ap.add_argument("--range", default=None, metavar="START:LEN", help="with -d: write only these decompressed bytes")
-    ap.add_argument("--index", default=None, metavar="FILE", help="with --range: the block index (--list output); with --lines: the line index")
+    ap.add_argument("--index", default=None, metavar="FILE",
+                    help="with --range: the block index (--list output) or a line index; with --lines: the line index")
+    ap.add_argument("--index-out", default=None, metavar="FILE", help="with -z: write the line index of the stream to FILE")
     ap.add_argument("--line-index", action="store_true", help="with -d: print the line index")
     ap.add_argument("--lines", default=None, metavar="FIRST:COUNT", help="with -d: write COUNT lines from line FIRST (1-based)")
     ap.add_argument("--grep", action="append", default=None, metavar="PATTERN", help="with -d: write the lines that contain PATTERN")
@@ -62,6 +68,12 @@ def main(argv=None, engine=None):
     ap.add_argument("--line-number", action="store_true", help="with --grep: prefix each line with its 1-based number and ':'")
     ap.add_argument("--count", action="store_true", help="with --grep: print the number of matching lines")
     a = ap.parse_args(argv)
+    if a.index_out is not None:
+        for flag, on in (("-d", a.decompress), ("--list", a.list), ("--range", a.range is not None), ("--grep", bool(a.grep)),
+                         ("--line-index", a.line_index), ("--lines", a.lines is not None), ("--recover", a.recover), ("-b", a.block >= 0)):
+            if on:
+                print(f"--index-out can only be used with -z, not with {flag}", file=sys.stderr)
+                return 1
     for flag, on in (("--ignore-case", a.ignore_case), ("--line-number", a.line_number), ("--count", a.count)):
         if on and not a.grep:
             print(f"{flag} can only be used with --grep", file=sys.stderr)
@@ -160,7 +172,8 @@ def main(argv=None, engine=None):
             data = src.read()
             if a.index is not None:
                 with open(a.index) as fh:
-                    index = Bzip2Index.from_text(fh.read())
+                    text = fh.read()
+                index = Bzip2LineIndex.from_text(text).blocks if text.startswith(Bzip2LineIndex.HEADER) else Bzip2Index.from_text(text)
             else:
                 index = Bzip2.index(data, a.multistream)
             dst.write(Bzip2.decompressRange(data, index, start, length))
@@ -193,6 +206,10 @@ def main(argv=None, engine=None):
             dst.write(Bzip2.decompressBlock(src.read(), a.block))
         elif a.decompress:
             Bzip2.decompressStream(src, dst, a.multistream)
+        elif a.index_out is not None:
+            _, index = Bzip2.compressStream(src, dst, level, chunk_bytes=a.chunk_mb << 20, index=True)
+            with open(a.index_out, "w") as fh:
+                fh.write(index.to_text())
         else:
             Bzip2.compressStream(src, dst, level, chunk_bytes=a.chunk_mb << 20)
     finally:

@@ -108,6 +108,11 @@ class Library:
         L.bz2b200_line_index.argtypes = [vp, vp, C.c_size_t, C.c_int, C.POINTER(C.POINTER(BlockEntry)), C.POINTER(C.POINTER(C.c_uint32)), szp,
                                          C.POINTER(C.c_uint64)]
         L.bz2b200_decompress_lines.argtypes = [vp, vp, C.c_size_t, vp, vp, C.c_size_t, C.c_uint64, vp, vp, C.c_size_t, u8pp, szp, vp]
+        ixp = [C.POINTER(C.POINTER(BlockEntry)), C.POINTER(C.POINTER(C.c_uint32)), szp, C.POINTER(C.c_uint64)]   # the line index outputs
+        L.bz2b200_compress_indexed.argtypes = [vp, vp, C.c_size_t, C.c_int, u8pp, szp] + ixp
+        L.bz2b200_pool_compress_indexed.argtypes = [vp, vp, C.c_size_t, C.c_int, C.c_size_t, u8pp, szp] + ixp
+        L.bz2b200_zstream_open_indexed.argtypes = [vp, C.c_int, C.c_size_t, C.POINTER(vp)]
+        L.bz2b200_zstream_index.argtypes = [vp] + ixp
         L.bz2b200_search.argtypes = [vp, vp, C.c_size_t, C.c_int, vp, vp, C.c_size_t, C.c_uint, C.c_uint64, C.POINTER(C.POINTER(Match)), szp,
                                      C.POINTER(SearchTotals), u8pp, szp]
         L.bz2b200_free.argtypes = [vp]

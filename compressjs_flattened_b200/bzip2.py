@@ -7,6 +7,7 @@
 
 Random access (no counterpart in the reference): Bzip2Engine.index, decompressRanges, decompressRange and open.
 Lines by number (no counterpart in the reference): Bzip2Engine.lineIndex, decompressLines and lineSpans.
+The same line index while compressing, with no decode: Bzip2Engine.compressIndexed and compressStream(..., index=True).
 Search (bzgrep -F, no counterpart in the reference): Bzip2Engine.search.
 
 Same names, argument meaning and error behaviour as the JavaScript API; the work is done by
@@ -91,6 +92,39 @@ def _patterns(patterns):
         if not 1 <= len(p) <= SEARCH_MAX_LEN:
             raise ValueError(f"pattern {i}: length must be 1..{SEARCH_MAX_LEN}, not {len(p)}")
     return pats   # the largest block a stream can have: the buffer of Bzip2Engine.open
+
+
+def _level(props):
+    """the level of compressFile's props (BJ:2204-2210): a number 1..9, 9 when props is not a number"""
+    level = props if isinstance(props, (int, float)) and not isinstance(props, bool) else 9
+    if level < 1 or level > 9 or int(level) != level:
+        raise ValueError("Invalid block size multiplier")
+    return int(level)
+
+
+def _line_index_call(owner, fn, *args):
+    """fn(*args, entries, newlines, count, total_lines) -> a Bzip2LineIndex of what it returned; errors through owner._raise"""
+    ptr, nlp, n, lines = C.POINTER(_native.BlockEntry)(), C.POINTER(C.c_uint32)(), C.c_size_t(), C.c_uint64()
+    rc = fn(*args, C.byref(ptr), C.byref(nlp), C.byref(n), C.byref(lines))
+    if rc:
+        owner._raise(rc)
+    try:
+        raw = _native.take_bytes(C.cast(ptr, C.POINTER(C.c_uint8)), n.value * INDEX_DTYPE.itemsize)
+        nl = _native.take_bytes(C.cast(nlp, C.POINTER(C.c_uint8)), n.value * 4)
+    finally:
+        owner._L.bz2b200_free(ptr)
+        owner._L.bz2b200_free(nlp)
+    return Bzip2LineIndex(Bzip2Index(np.frombuffer(raw, dtype=INDEX_DTYPE)), np.frombuffer(nl, dtype=np.uint32), lines.value)
+
+
+def _compress_indexed(owner, fn, handle, input, props, *extra):
+    """fn = bz2b200_compress_indexed or bz2b200_pool_compress_indexed on `handle` (extra: the arguments after the level)
+    -> (stream bytes, Bzip2LineIndex)"""
+    level = _level(props)
+    a = _coerce_input(input)
+    out, n = C.POINTER(C.c_uint8)(), C.c_size_t()
+    index = _line_index_call(owner, fn, handle, a.ctypes.data, a.size, level, *extra, C.byref(out), C.byref(n))
+    return owner._take(out, n.value), index
 
 
 def _search(owner, fn, handle, input, patterns, ignore_case, max_matches, multistream, lines, *extra):
@@ -348,15 +382,18 @@ class Bzip2Engine:
 
     # -- the four methods of the reference object --
     def compressFile(self, input, output=None, props=None):
-        level = props if isinstance(props, (int, float)) and not isinstance(props, bool) else 9  # BJ:2204-2206
-        if level < 1 or level > 9 or int(level) != level:
-            raise ValueError("Invalid block size multiplier")
+        level = _level(props)
         a = _coerce_input(input)
         out, n = C.POINTER(C.c_uint8)(), C.c_size_t()
-        rc = self._L.bz2b200_compress(self._ctx, a.ctypes.data, a.size, int(level), C.byref(out), C.byref(n))
+        rc = self._L.bz2b200_compress(self._ctx, a.ctypes.data, a.size, level, C.byref(out), C.byref(n))
         if rc:
             self._raise(rc)
         return _deliver(self._take(out, n.value), output)
+
+    def compressIndexed(self, input, props=None):
+        """compressFile that also returns the stream's line index, computed while compressing (no decode):
+        (stream bytes, Bzip2LineIndex), the index equal to lineIndex(stream).  The stream is compressFile's."""
+        return _compress_indexed(self, self._L.bz2b200_compress_indexed, self._ctx, input, props)
 
     # -- the stream flavour (SURVEY 8f N2; what NPM/bin/compressjs:163-180 does with {readByte}/{writeByte} streams) --
     @staticmethod
@@ -381,8 +418,10 @@ class Bzip2Engine:
             return b
         return read
 
-    def _pump(self, kind, handle, source, sink, piece):
-        """read pieces, feed them, hand on what comes back; the C stream object does the work (csrc/stream_abi.inl)"""
+    def _pump(self, kind, handle, source, sink, piece, finished=None):
+        """read pieces, feed them, hand on what comes back; the C stream object does the work (csrc/stream_abi.inl).
+        finished: called with the handle after finish succeeded, before the handle is closed; the result is then
+        (what is returned without it, what finished returned)"""
         L = self._L
         feed, finish = getattr(L, f"bz2b200_{kind}_feed"), getattr(L, f"bz2b200_{kind}_finish")
         read = self._reader(source, piece)
@@ -417,27 +456,31 @@ class Bzip2Engine:
             if rc:
                 self._raise(rc)
             put(out, n.value)
+            extra = finished(handle) if finished else None
         finally:
             getattr(L, f"bz2b200_{kind}_close")(handle)
         if sink is None:
-            return bytes(collected)
-        if hasattr(sink, "flush"):
-            sink.flush()
-        return sink
+            result = bytes(collected)
+        else:
+            if hasattr(sink, "flush"):
+                sink.flush()
+            result = sink
+        return (result, extra) if finished else result
 
-    def compressStream(self, source, sink=None, props=None, chunk_bytes=64 << 20, piece_bytes=None):
+    def compressStream(self, source, sink=None, props=None, chunk_bytes=64 << 20, piece_bytes=None, index=False):
         """Stream flavour of compressFile: the source is read piece by piece and whole blocks are compressed as soon as the
         bytes after them (their halo) have arrived, so neither the input nor the output is ever held in full.
         Byte-identical to compressFile on the concatenated input.  source: .read(n) -> bytes, {readByte}, or bytes-like;
-        sink: .write(bytes), {writeByte}, or None (the stream is returned as bytes)."""
-        level = props if isinstance(props, (int, float)) and not isinstance(props, bool) else 9  # BJ:2204-2206
-        if level < 1 or level > 9 or int(level) != level:
-            raise ValueError("Invalid block size multiplier")                                    # BJ:2208-2210
+        sink: .write(bytes), {writeByte}, or None (the stream is returned as bytes).  index=True: returns (what it
+        returns otherwise, the stream's Bzip2LineIndex), built while compressing as compressIndexed builds it."""
+        level = _level(props)
         h = C.c_void_p()
-        rc = self._L.bz2b200_zstream_open(self._ctx, int(level), int(chunk_bytes), C.byref(h))
+        open_ = self._L.bz2b200_zstream_open_indexed if index else self._L.bz2b200_zstream_open
+        rc = open_(self._ctx, level, int(chunk_bytes), C.byref(h))
         if rc:
             self._raise(rc)
-        return self._pump("zstream", h, source, sink, int(piece_bytes or max(1, chunk_bytes // 4)))
+        finished = (lambda handle: _line_index_call(self, self._L.bz2b200_zstream_index, handle)) if index else None
+        return self._pump("zstream", h, source, sink, int(piece_bytes or max(1, chunk_bytes // 4)), finished)
 
     def decompressStream(self, source, sink=None, multistream=False, chunk_bytes=16 << 20, piece_bytes=None):
         """Stream flavour of decompressFile: blocks are decoded as soon as they are complete; the bytes of the blocks before
@@ -512,7 +555,10 @@ class Bzip2Engine:
     def decompressRanges(self, input, index, ranges):
         """The bytes of every (start, length) of the decompressed output, as a list in request order.  Each range is clipped
         to the output the way slicing clips output[start:start + length].  One call decodes every block that covers a
-        range, once, and nothing else; the stream CRC is not checked (include/bz2b200.h)."""
+        range, once, and nothing else; the stream CRC is not checked (include/bz2b200.h).  index: a Bzip2Index or a
+        Bzip2LineIndex (its blocks are used)."""
+        if isinstance(index, Bzip2LineIndex):
+            index = index.blocks
         a = _coerce_input(input)
         ix = index.entries
         total = index.total
@@ -534,8 +580,8 @@ class Bzip2Engine:
 
     def open(self, input, index=None, multistream=False):
         """A seekable, read-only binary file over the decompressed bytes of `input` (bytes-like, or a path, which is
-        memory-mapped).  Every read decodes only the blocks it needs.  Without `index` one is built first: that is a full
-        decode of the input.  The buffer holds one level-9 block, so small sequential reads do not decode a block each;
+        memory-mapped).  Every read decodes only the blocks it needs.  index: a Bzip2Index or a Bzip2LineIndex (what
+        compressIndexed returns); without it one is built first: that is a full decode of the input.  The buffer holds one level-9 block, so small sequential reads do not decode a block each;
         read() to the end is one call."""
         if isinstance(input, (str, os.PathLike)):
             with builtins.open(input, "rb") as fh:
@@ -544,24 +590,17 @@ class Bzip2Engine:
         a = _coerce_input(input)
         if index is None:
             index = self.index(a, multistream)
+        elif isinstance(index, Bzip2LineIndex):
+            index = index.blocks
         return io.BufferedReader(_RangeReader(self, a, index), buffer_size=LEVEL9_BLOCK)
 
     # -- lines by number (include/bz2b200.h, bz2b200_line_index / bz2b200_decompress_lines) --
     def lineIndex(self, input, multistream=False):
         """The block index of `input` with the '\n' bytes of every block (a Bzip2LineIndex).  The input is decoded as
-        decompressFile decodes it, with the same errors; the '\n' bytes are counted on the GPU."""
+        decompressFile decodes it, with the same errors; the '\n' bytes are counted on the GPU.  A stream compressed here
+        can have the same index without a decode: compressIndexed."""
         a = _coerce_input(input)
-        ptr, nlp, n, lines = C.POINTER(_native.BlockEntry)(), C.POINTER(C.c_uint32)(), C.c_size_t(), C.c_uint64()
-        rc = self._L.bz2b200_line_index(self._ctx, a.ctypes.data, a.size, int(bool(multistream)), C.byref(ptr), C.byref(nlp), C.byref(n), C.byref(lines))
-        if rc:
-            self._raise(rc)
-        try:
-            raw = _native.take_bytes(C.cast(ptr, C.POINTER(C.c_uint8)), n.value * INDEX_DTYPE.itemsize)
-            nl = _native.take_bytes(C.cast(nlp, C.POINTER(C.c_uint8)), n.value * 4)
-        finally:
-            self._L.bz2b200_free(ptr)
-            self._L.bz2b200_free(nlp)
-        return Bzip2LineIndex(Bzip2Index(np.frombuffer(raw, dtype=INDEX_DTYPE)), np.frombuffer(nl, dtype=np.uint32), lines.value)
+        return _line_index_call(self, self._L.bz2b200_line_index, self._ctx, a.ctypes.data, a.size, int(bool(multistream)))
 
     def _lines(self, input, index, requests, want_bytes):
         """bz2b200_decompress_lines over the clipped requests -> (bytes or None, (k, 2) uint64 spans)"""

@@ -142,6 +142,7 @@ struct Ctx {
   DevBuf dpieces, dgather;  // range reads: the pieces and the packed bytes (search: the lines)
   DevBuf dspat, dstile, dsbase, dstsum, dsmatch, dspart, dstot;  // search: patterns and filter, per-tile and per-thread summaries, matches
   DevBuf dnltile, dnlpart, dnlq;  // newline directory: tile counts then their prefix, scan partials, queries and their results
+  DevBuf ixtab;  // indexed compress: a bz2b200_block_entry row per block of the call, then the blocks' '\n' counts (u32)
   // last compress, for debug_fetch
   struct Pipe {
     const u8 *d_in = nullptr;
@@ -173,7 +174,9 @@ struct Ctx {
   std::vector<u32> dec_last_chain;
   i64 dec_last_bs = 0;
   u32 search_tile = 0;     // tests only: bytes per search tile (0 = SEARCH_TILE_DEFAULT)
-  u32 line_tile = 0;       // tests only: bytes per newline-directory tile (0 = LINE_TILE_DEFAULT)
+  u32 line_tile = 0;       // tests only: bytes per newline-directory tile (0 = LINE_TILE_DEFAULT), also per k_index_rows segment
+  bool index_on = false;   // pipe_run also builds the line index of its blocks (the indexed compress calls set it for one call)
+  std::vector<u8> ix_host; // that index after pipe_run: pipe.nb rows, then pipe.nb '\n' counts, as in ixtab
   u64 shard_bits = 0;      // bit length of the last shard segment (phase 0 in `out`)
   int cand_n = 0, cand_max_blocks = 0, cand_nb[64];  // speculated cut walks of the last shard_cut_g
   i64 cand_s[64];
@@ -191,7 +194,7 @@ struct Ctx {
                      &gbounds, &key2, &big_cnt, &big_old, &big_rank, &big_tile0, &big_tblk, &totals2,
                      &recs_cand, &cand_first, &out2, &blksort, &r2_status, &hfreq, &hlens, &hplen, &hcodes, &hsel, &hcost, &hgoff, &hblk,
                      &d_in, &cand, &ncand, &dmeta, &dsyms, &dL, &dtt, &dwalk, &dblk, &dout, &dmisc, &dsel, &doff, &dperm, &dmap,
-                     &dpieces, &dgather, &dspat, &dstile, &dsbase, &dstsum, &dsmatch, &dspart, &dstot, &dnltile, &dnlpart, &dnlq};
+                     &dpieces, &dgather, &dspat, &dstile, &dsbase, &dstsum, &dsmatch, &dspart, &dstot, &dnltile, &dnlpart, &dnlq, &ixtab};
     for (DevBuf *b : all) pool.push_back(b);
   }
 };
@@ -680,12 +683,35 @@ int batch_limit(Ctx *c) {
   return (int)(lim < 1 ? 1 : lim);
 }
 
+// k_index_rows over blocks first .. first + nb - 1 of the table (the batch pipe_run is stitching), timed by ev[6] / ev[7]
+int index_rows(Ctx *c, int first, int nb) {
+  const BlockRec *h = c->pipe.hrecs.data() + first;
+  i64 span = 0;
+  for (int k = 0; k < nb; k++) span = std::max(span, h[k].p - (h[k].s & ~(i64)15));
+  const u32 seg = c->line_tile ? c->line_tile : IX_SEG_DEFAULT;
+  bz2b200_block_entry *rows = P<bz2b200_block_entry>(c->ixtab);
+  u32 *counts = reinterpret_cast<u32 *>(rows + c->pipe.nb);
+  RC(mark(c, 6));
+  LAUNCH(k_index_rows, dim3((unsigned)((span + seg - 1) / seg), (unsigned)std::min(nb, 65535)), IX_THREADS, 0, c->pipe.d_in, P<BlockRec>(c->recs) + first,
+         P<u64>(c->bit_off), nb, seg, (u32)c->pipe.level, rows + first, counts + first);
+  return mark(c, 7);
+}
+
 // stages + emission of every block in the table, batch by batch.  base_bits: 32 for a whole stream (then header and
 // footer are written too), 0..7 for a shard segment.  The stats of the batches add up in c->st, which pipe_begin cleared.
+// With c->index_on, k_index_rows also runs on every batch and the rows and counts come back to c->ix_host with the
+// last batch's read-back; ms_stage[5] is then its device time.
 int pipe_run(Ctx *c, u64 base_bits, bool whole, u32 *d_out, size_t out_cap, bool own_out, size_t *out_len, u64 *bits_out, u32 *crc_fold) {
   Ctx::Pipe &P_ = c->pipe;
   const int nb = P_.nb, maxb = batch_limit(c);
   const bool batched = nb > maxb;
+  const bool ix = c->index_on;
+  const size_t ix_bytes = (sizeof(bz2b200_block_entry) + 4) * (size_t)nb;
+  if (ix) {
+    c->ix_host.resize(ix_bytes);
+    ENS(c->ixtab, ix_bytes);
+    if (nb) CK(cudaMemsetAsync(P<u8>(c->ixtab) + sizeof(bz2b200_block_entry) * (size_t)nb, 0, 4 * (size_t)nb, c->stream));
+  }
   if (own_out && batched) {  // sized once: growing it later would drop the bits of the earlier batches
     out_cap = bz2b200_compress_bound((size_t)P_.N, P_.level) + 64;
     ENS(c->out, out_cap);
@@ -700,6 +726,7 @@ int pipe_run(Ctx *c, u64 base_bits, bool whole, u32 *d_out, size_t out_cap, bool
     if ((rc = pipe_stages(c, b0, bn))) return rc;
     const u64 base = end_bits;
     LAUNCH(k_stitch_offsets, 1, 1024, 0, P<BlockMeta>(c->meta), P<BlockRec>(c->recs) + b0, bn, P<u64>(c->bit_off), P<u32>(c->scrc), base, fold);
+    if (ix && bn) RC(index_rows(c, b0, bn));
     RC(rb_add(c, &end_bits, P<u64>(c->bit_off) + bn, 8));
     RC(rb_add(c, &fold, c->scrc.p, 4));
     RC(rb_sync(c));
@@ -720,6 +747,7 @@ int pipe_run(Ctx *c, u64 base_bits, bool whole, u32 *d_out, size_t out_cap, bool
       LAUNCH(k_stream_ends, 1, 32, 0, d_out, P<u64>(c->bit_off), bn, P<u32>(c->scrc), P_.level, P<u64>(c->out_len));
       RC(rb_add(c, &olen, c->out_len.p, 8));
     }
+    if (ix && nb && b0 + bn == nb) CK(cudaMemcpyAsync(c->ix_host.data(), c->ixtab.p, ix_bytes, cudaMemcpyDeviceToHost, c->stream));
     if ((rc = mark(c, 5))) return rc;
     RC(rb_sync(c));
     CK(cudaGetLastError());
@@ -734,6 +762,7 @@ int pipe_run(Ctx *c, u64 base_bits, bool whole, u32 *d_out, size_t out_cap, bool
       CK(cudaEventElapsedTime(&t, c->ev[0], c->ev[5]));
       c->st.ms_total += t;
       for (size_t i = 0; i + 1 < c->dom_used; i += 2) { CK(cudaEventElapsedTime(&t, c->dom_ev[i], c->dom_ev[i + 1])); c->st.dom_ms += t; }
+      if (ix && bn) { CK(cudaEventElapsedTime(&t, c->ev[6], c->ev[7])); c->st.ms_stage[5] += t; }
     }
     b0 += bn;
   } while (b0 < nb);
@@ -751,6 +780,39 @@ int compress_device(Ctx *c, const u8 *d_in, size_t n_, int level, u32 *d_out, si
   rc = pipe_run(c, 32, true, d_out, out_cap, own_out, out_len, nullptr, nullptr);
   trace_report(c);
   return rc;
+}
+
+// ---- the line index of an indexed compress call: the rows and '\n' counts of its blocks in stream order ----------------
+struct LineIx {
+  std::vector<bz2b200_block_entry> rows;
+  std::vector<u32> nl;
+  u64 total_lines = 0;
+};
+// the rows and counts pipe_run left in c->ix_host, appended with their bits moved by bit_add and their out_offset by in_add
+// (where the bits and the input of the segment pipe_run compressed start in the stream)
+void ix_append(Ctx *c, LineIx &ix, u64 bit_add, u64 in_add) {
+  const size_t nb = (size_t)c->pipe.nb, at = ix.rows.size();
+  const bz2b200_block_entry *r = reinterpret_cast<const bz2b200_block_entry *>(c->ix_host.data());
+  const u32 *k = reinterpret_cast<const u32 *>(r + nb);
+  ix.rows.insert(ix.rows.end(), r, r + nb);
+  ix.nl.insert(ix.nl.end(), k, k + nb);
+  for (size_t i = at; i < ix.rows.size(); i++) { ix.rows[i].bit_begin += bit_add; ix.rows[i].bit_end += bit_add; ix.rows[i].out_offset += in_add; }
+}
+// total_lines of an input of n bytes whose last byte is `last`: its '\n' bytes, plus 1 when it does not end with one
+void ix_total(LineIx &ix, u64 n, u8 last) {
+  u64 t = 0;
+  for (u32 k : ix.nl) t += k;
+  ix.total_lines = t + (n && last != '\n' ? 1 : 0);
+}
+// ix as the caller's arrays (malloc'ed, released with bz2b200_free); nothing is returned on failure
+int ix_out(const LineIx &ix, bz2b200_block_entry **entries, uint32_t **newlines, size_t *count, uint64_t *total_lines) {
+  const size_t k = ix.rows.size();
+  bz2b200_block_entry *e = (bz2b200_block_entry *)malloc((k ? k : 1) * sizeof(bz2b200_block_entry));
+  uint32_t *h = (uint32_t *)malloc((k ? k : 1) * sizeof(uint32_t));
+  if (!e || !h) { free(e); free(h); return BZ2B200_E_OUT_OF_MEMORY; }
+  if (k) { memcpy(e, ix.rows.data(), k * sizeof(bz2b200_block_entry)); memcpy(h, ix.nl.data(), k * sizeof(uint32_t)); }
+  *entries = e; *newlines = h; *count = k; *total_lines = ix.total_lines;
+  return BZ2B200_OK;
 }
 
 // the segment of `bits` bits that pipe_run left in c->out, moved to start at bit `phase` of its first byte (into
@@ -814,6 +876,42 @@ void ctx_delete(Ctx *c) {
   delete c;
 }
 
+// bz2b200_compress of valid arguments; ix != nullptr: also the line index of the stream (without total_lines)
+int compress_host(Ctx *c, const uint8_t *in, size_t n, int level, uint8_t **out, size_t *out_len, LineIx *ix) {
+  if (n >= c->pool_min_bytes) {
+    // large input: shards over two lanes of this device, so that the copies in both directions hide under the kernels
+    if (!c->own_pool) {
+      const int dev = c->device;
+      int prc = pool_new(&dev, 1, 2, &c->own_pool);
+      if (prc) { c->err = "cannot create the lanes of the context's pool"; return prc; }
+    }
+    Pool *p = c->own_pool;
+    p->cap_override = c->cap_override; p->batch_override = c->batch_override;
+    p->halo0 = c->pool_halo0; p->force_staging = c->pool_force_staging;
+    p->line_tile = c->line_tile;
+    p->plan_first = n / 5 * 2 + 1;  // one device, two lanes: two shards of 40 / 60 % measured best (profiles/r02_pool_two_shard_plans_n1.log)
+    p->plan_growth = 1000.0;
+    int prc = pool_compress_whole(p, in, n, level, c->pool_shard_bytes, out, out_len, ix);
+    c->st = p->st;
+    c->err = p->err;
+    return prc;
+  }
+  ENS(c->in, n + 64);
+  if (n) CK(cudaMemcpyAsync(c->in.p, in, n, cudaMemcpyHostToDevice, c->stream));
+  size_t olen = 0;
+  c->index_on = ix != nullptr;
+  int rc = compress_device(c, P<u8>(c->in), n, level, nullptr, 0, &olen, true);
+  c->index_on = false;
+  if (rc) return rc;
+  uint8_t *res = (uint8_t *)result_pool().get(olen);
+  if (!res) return BZ2B200_E_OUT_OF_MEMORY;
+  CK(cudaMemcpy(res, c->out.p, olen, cudaMemcpyDeviceToHost));
+  if (ix) ix_append(c, *ix, 0, 0);
+  *out = res;
+  *out_len = olen;
+  return BZ2B200_OK;
+}
+
 }  // namespace
 
 // ------------------------------------------------------------------------------------ C ABI
@@ -843,34 +941,31 @@ int bz2b200_compress(bz2b200_ctx *ctx, const uint8_t *in, size_t n, int level, u
   if (!c || !out || !out_len || (n && !in)) return BZ2B200_E_ARG;
   if (level < 1 || level > 9) return BZ2B200_E_LEVEL;
   CK(cudaSetDevice(c->device));
-  if (n >= c->pool_min_bytes) {
-    // large input: shards over two lanes of this device, so that the copies in both directions hide under the kernels
-    if (!c->own_pool) {
-      const int dev = c->device;
-      int prc = pool_new(&dev, 1, 2, &c->own_pool);
-      if (prc) { c->err = "cannot create the lanes of the context's pool"; return prc; }
-    }
-    Pool *p = c->own_pool;
-    p->cap_override = c->cap_override; p->batch_override = c->batch_override;
-    p->halo0 = c->pool_halo0; p->force_staging = c->pool_force_staging;
-    p->plan_first = n / 5 * 2 + 1;  // one device, two lanes: two shards of 40 / 60 % measured best (profiles/r02_pool_two_shard_plans_n1.log)
-    p->plan_growth = 1000.0;
-    int prc = pool_compress_whole(p, in, n, level, c->pool_shard_bytes, out, out_len);
-    c->st = p->st;
-    c->err = p->err;
-    return prc;
+  return compress_host(c, in, n, level, out, out_len, nullptr);
+}
+
+int bz2b200_compress_indexed(bz2b200_ctx *ctx, const uint8_t *in, size_t n, int level, uint8_t **out, size_t *out_len, bz2b200_block_entry **entries,
+                             uint32_t **newlines, size_t *count, uint64_t *total_lines) {
+  Ctx *c = reinterpret_cast<Ctx *>(ctx);
+  if (!c || !out || !out_len || (n && !in) || !entries || !newlines || !count || !total_lines) return BZ2B200_E_ARG;
+  if (level < 1 || level > 9) return BZ2B200_E_LEVEL;
+  CK(cudaSetDevice(c->device));
+  try {
+    LineIx ix;
+    uint8_t *res = nullptr;
+    size_t olen = 0;
+    int rc = compress_host(c, in, n, level, &res, &olen, &ix);
+    if (rc) return rc;
+    ix_total(ix, n, n ? in[n - 1] : 0);
+    if ((rc = ix_out(ix, entries, newlines, count, total_lines))) { result_pool().put(res); return rc; }
+    *out = res;
+    *out_len = olen;
+    return BZ2B200_OK;
+  } catch (...) {
+    c->index_on = false;
+    c->err = "host exception (memory)";
+    return BZ2B200_E_OUT_OF_MEMORY;
   }
-  ENS(c->in, n + 64);
-  if (n) CK(cudaMemcpyAsync(c->in.p, in, n, cudaMemcpyHostToDevice, c->stream));
-  size_t olen = 0;
-  int rc = compress_device(c, P<u8>(c->in), n, level, nullptr, 0, &olen, true);
-  if (rc) return rc;
-  uint8_t *res = (uint8_t *)result_pool().get(olen);
-  if (!res) return BZ2B200_E_OUT_OF_MEMORY;
-  CK(cudaMemcpy(res, c->out.p, olen, cudaMemcpyDeviceToHost));
-  *out = res;
-  *out_len = olen;
-  return BZ2B200_OK;
 }
 
 int bz2b200_shard_begin(bz2b200_ctx *ctx, const void *in, size_t n_avail, int on_device, int level) {

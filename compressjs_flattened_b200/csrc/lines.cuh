@@ -9,7 +9,8 @@
 //                then the warp walks the tile 512 bytes at a time (one word per lane, a warp scan of the counts) and the
 //                lane that holds the k-th '\n' takes it from its word's 16-bit mask with __fns
 // A word is read whole even where it runs past n (a decode sink keeps 64 bytes of slack after its bytes); what lies past
-// n or past the tile is masked off and never counted.
+// n or past the tile is masked off and never counted.  k_index_rows (below) counts the input of the compressor's blocks
+// with the same helpers.
 #define LINE_TILE_DEFAULT 8192u
 #define LINE_TILE_MAX 8192u
 #define NL_THREADS 256              // 8 warps per CTA: 8 tiles or 8 queries
@@ -103,5 +104,58 @@ __global__ void __launch_bounds__(NL_THREADS) k_nl_select(const u8 *__restrict__
       return;
     }
     r -= total;
+  }
+}
+
+// ---- the line index of a compress call (bz2b200_compress_indexed and friends) ----------------------------------------
+// Launched once per batch of the compressor, right after k_stitch_offsets.  For block b of the batch it writes the
+// bz2b200_block_entry row rows[b] -- bits from bit_off (absolute for a whole stream, from 0 for a shard segment: the caller
+// moves them), out_offset = the block's first input byte s (the caller adds the offset of the input buffer), out_bytes =
+// p - s, since the block decodes to exactly the input bytes [s, p) -- and adds the '\n' bytes of [s, p) into counts[b]
+// (zeroed by the caller).  A run-heavy block spans up to ~46 MB of input, so the grid is (segments, blocks): CTA (x, y)
+// counts segment x -- `seg` bytes from the 16-byte word that holds s -- of blocks y, y + gridDim.y, ..., one atomicAdd per
+// CTA.  Every word is loaded once with a 16-byte load (the word a block boundary cuts is loaded by both blocks); the bytes
+// before s and from p on are masked off.  A word read past p stays inside the input buffer's 64 bytes of slack.
+#define IX_THREADS 256
+#define IX_SEG_DEFAULT 32768u  // bytes per segment (bz2b200_debug_set_line_tile sets it for tests)
+
+// m without its first k bytes
+__device__ __forceinline__ uint4 nl_drop16(uint4 m, u32 k) {
+  m.x &= ~nl_keep(k, 0); m.y &= ~nl_keep(k, 1); m.z &= ~nl_keep(k, 2); m.w &= ~nl_keep(k, 3);
+  return m;
+}
+
+__global__ void __launch_bounds__(IX_THREADS) k_index_rows(const u8 *__restrict__ in, const BlockRec *__restrict__ recs, const u64 *__restrict__ bit_off,
+                                                           int nb, u32 seg, u32 level, bz2b200_block_entry *__restrict__ rows, u32 *__restrict__ counts) {
+  __shared__ u32 part[IX_THREADS / 32];
+  const u32 lane = threadIdx.x & 31, warp = threadIdx.x / 32;
+  for (int b = blockIdx.y; b < nb; b += gridDim.y) {
+    const u64 s = (u64)recs[b].s, p = (u64)recs[b].p;
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+      bz2b200_block_entry e;
+      e.bit_begin = bit_off[b]; e.bit_end = bit_off[b + 1];
+      e.out_offset = s; e.out_bytes = (u32)(p - s);
+      e.crc = recs[b].crc; e.stream = 0; e.level = level;
+      rows[b] = e;
+    }
+    const u64 a = (s & ~(u64)15) + (u64)blockIdx.x * seg;
+    if (a >= p) continue;  // the same for the whole CTA
+    const u64 e = p - a < seg ? p : a + seg;
+    u32 cnt = 0;
+#pragma unroll 4
+    for (u64 w = a + 16 * (u64)threadIdx.x; w < e; w += 16 * IX_THREADS) {
+      uint4 m = nl_marks16(*reinterpret_cast<const uint4 *>(in + w), e - w < 16 ? (u32)(e - w) : 16u);
+      if (w < s) m = nl_drop16(m, (u32)(s - w));
+      cnt += nl_count16(m);
+    }
+    cnt = (u32)nl_warp_sum(cnt);
+    if (lane == 0) part[warp] = cnt;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      u32 t = 0;
+      for (int i = 0; i < IX_THREADS / 32; i++) t += part[i];
+      if (t) atomicAdd(&counts[b], t);
+    }
+    __syncthreads();
   }
 }

@@ -12,7 +12,7 @@ import ctypes as C
 import numpy as np
 
 from . import _native
-from .bzip2 import Bzip2Error, _coerce_input, _deliver, _search
+from .bzip2 import Bzip2Error, _coerce_input, _compress_indexed, _deliver, _level, _search
 
 
 def shard_plan(n, level=9, lanes=2, first_bytes=0, growth=0.0, library=None):
@@ -122,15 +122,18 @@ class Bzip2Pool:
             self._raise(rc)
 
     def compressFile(self, input, output=None, props=None, shard_bytes=0):
-        level = props if isinstance(props, (int, float)) and not isinstance(props, bool) else 9  # BJ:2204-2206
-        if level < 1 or level > 9 or int(level) != level:
-            raise ValueError("Invalid block size multiplier")
+        level = _level(props)
         a = _coerce_input(input)
         out, n = C.POINTER(C.c_uint8)(), C.c_size_t()
-        rc = self._L.bz2b200_pool_compress(self._p, a.ctypes.data, a.size, int(level), shard_bytes, C.byref(out), C.byref(n))
+        rc = self._L.bz2b200_pool_compress(self._p, a.ctypes.data, a.size, level, shard_bytes, C.byref(out), C.byref(n))
         if rc:
             self._raise(rc)
         return _deliver(self._take(out, n.value), output)
+
+    def compressIndexed(self, input, props=None, shard_bytes=0):
+        """compressFile that also returns the stream's line index, built by every lane for its shards while compressing
+        (no decode): (stream bytes, Bzip2LineIndex), as Bzip2Engine.compressIndexed returns them."""
+        return _compress_indexed(self, self._L.bz2b200_pool_compress_indexed, self._p, input, props, int(shard_bytes))
 
     def compress_raw(self, ptr, nbytes, level, shard_bytes=0):
         """(pointer, length) of the stream in the library's page-locked result memory; release with free_raw."""

@@ -18,6 +18,8 @@
  *   (random access: no counterpart in BJ)  bz2b200_index / bz2b200_decompress_ranges
  *   (bzgrep: no counterpart in BJ)         bz2b200_search
  *   (sed -n by line: no counterpart in BJ) bz2b200_line_index / bz2b200_decompress_lines
+ *   (an index while compressing: none)     bz2b200_compress_indexed / bz2b200_pool_compress_indexed /
+ *                                          bz2b200_zstream_open_indexed + bz2b200_zstream_index
  */
 #ifndef BZ2B200_H
 #define BZ2B200_H
@@ -154,6 +156,27 @@ int bz2b200_line_index(bz2b200_ctx *ctx, const uint8_t *in, size_t n, int multis
 int bz2b200_decompress_lines(bz2b200_ctx *ctx, const uint8_t *in, size_t n, const bz2b200_block_entry *index, const uint32_t *newlines, size_t count,
                              uint64_t total_lines, const uint64_t *firsts, const uint64_t *counts, size_t n_requests, uint8_t **out, size_t *out_len,
                              uint64_t *spans);
+/* The line index as a by-product of compression, with no decode.  bz2b200_compress_indexed returns what
+ * bz2b200_compress(ctx, in, n, level) returns -- the same stream bytes, return codes and errors, also through the two-lane
+ * route of inputs of 32 MB or more -- and the line index of that stream: *entries, *newlines, *count and *total_lines equal
+ * what bz2b200_line_index(stream, multistream = 0) returns for it (stream = 0 and the call's level in every entry).  The
+ * compressor knows every field: block i decodes to exactly its input bytes [s, p), its bits are where the stitch puts
+ * them and its CRC is the one it writes; the '\n' bytes of each block are counted on the GPU in the input it already holds
+ * (k_index_rows, once per batch of blocks).  The index describes the input and the emitted bits: when a block reproduces
+ * defect D1 (DESIGN.md section 2, a stream the reference's own decoder rejects) the stream is still the reference's and
+ * the index is still the one computed from the input (stats d1_triggered set); nothing is decoded to check it.  An empty
+ * input gives count 0 and total_lines 0.  The four index outputs are required (NULL: BZ2B200_E_ARG); they are released
+ * with bz2b200_free.  On any error nothing is returned.  bz2b200_last_stats: as for bz2b200_compress, except that
+ * kernel_launches also counts the index kernel (one launch per batch of blocks) and ms_stage[5] is its device time, summed
+ * over the batches (and over the lanes for a pool).
+ * bz2b200_pool_compress_indexed is bz2b200_pool_compress with the same index.  The stream flavour: a zstream opened with
+ * bz2b200_zstream_open_indexed feeds and finishes exactly as one from bz2b200_zstream_open; once bz2b200_zstream_finish
+ * has succeeded, bz2b200_zstream_index returns the index of the whole stream (BZ2B200_E_ARG, with a message in
+ * bz2b200_last_error of the zstream's context, before that or on a zstream opened without an index).
+ * Not indexed: bz2b200_compress_device, the ranked and group shard calls (bz2b200_pool_compress_shards, bz2b200_shard_*;
+ * bz2b200_shard_result keeps its layout), and the JavaScript addon and shim. */
+int bz2b200_compress_indexed(bz2b200_ctx *ctx, const uint8_t *in, size_t n, int level, uint8_t **out, size_t *out_len, bz2b200_block_entry **entries,
+                             uint32_t **newlines, size_t *count, uint64_t *total_lines);
 
 /* Fixed-string search of the decompressed output (what bzgrep -F does, without bringing the decoded bytes back).  The
  * input is decoded exactly as bz2b200_decompress(ctx, in, n, multistream) decodes it -- same walk, CRC checks and error
@@ -249,6 +272,9 @@ typedef struct bz2b200_group bz2b200_group;
 int bz2b200_pool_create(const int *devices, int n_devices, int lanes_per_device, bz2b200_pool **pool);
 void bz2b200_pool_destroy(bz2b200_pool *pool);
 int bz2b200_pool_compress(bz2b200_pool *pool, const uint8_t *in, size_t n, int level, size_t shard_bytes, uint8_t **out, size_t *out_len);
+/* pool_compress that also returns the stream's line index (see bz2b200_compress_indexed) */
+int bz2b200_pool_compress_indexed(bz2b200_pool *pool, const uint8_t *in, size_t n, int level, size_t shard_bytes, uint8_t **out, size_t *out_len,
+                                  bz2b200_block_entry **entries, uint32_t **newlines, size_t *count, uint64_t *total_lines);
 /* shard plan of pool_compress when shard_bytes == 0: the first shard of every lane has first_bytes (0 = six blocks), every
  * following wave is `growth` times larger (0 = 2.5): only the first upload is exposed, large batches do most of the work */
 int bz2b200_pool_set_plan(bz2b200_pool *pool, size_t first_bytes, double growth);
@@ -337,6 +363,9 @@ int bz2b200_debug_set_pool(bz2b200_ctx *ctx, size_t min_bytes, size_t shard_byte
 typedef struct bz2b200_zstream bz2b200_zstream;
 typedef struct bz2b200_dstream bz2b200_dstream;
 int bz2b200_zstream_open(bz2b200_ctx *ctx, int level, size_t chunk_bytes, bz2b200_zstream **zs);
+/* a zstream that also builds the stream's line index; bz2b200_zstream_index after finish (see bz2b200_compress_indexed) */
+int bz2b200_zstream_open_indexed(bz2b200_ctx *ctx, int level, size_t chunk_bytes, bz2b200_zstream **zs);
+int bz2b200_zstream_index(bz2b200_zstream *zs, bz2b200_block_entry **entries, uint32_t **newlines, size_t *count, uint64_t *total_lines);
 int bz2b200_zstream_feed(bz2b200_zstream *zs, const uint8_t *in, size_t n, uint8_t **out, size_t *out_len);
 int bz2b200_zstream_finish(bz2b200_zstream *zs, uint8_t **out, size_t *out_len);
 void bz2b200_zstream_close(bz2b200_zstream *zs);
@@ -370,7 +399,8 @@ int bz2b200_debug_set_batch_blocks(bz2b200_ctx *ctx, uint32_t blocks);
 /* tests/ only: bytes per tile of the search kernels, a multiple of 256 up to 8192 (0 = 8192), so that small outputs
  * span many tiles. */
 int bz2b200_debug_set_search_tile(bz2b200_ctx *ctx, uint32_t bytes);
-/* tests/ only: bytes per newline-directory tile (a multiple of 256 up to 8192; 0 = the default, 8192) */
+/* tests/ only: bytes per newline-directory tile (a multiple of 256 up to 8192; 0 = the default, 8192), and per segment of the
+ * indexed compress calls' '\n' count (0 = the default, 32768; a context's own two-lane pool takes it too) */
 int bz2b200_debug_set_line_tile(bz2b200_ctx *ctx, uint32_t bytes);
 /* tests/ only: skip the block-CRC comparison of the decoder (BJ:1756-1761), so that what a damaged stream decodes TO
  * can be compared with the oracle.  Not reachable from the environment. */
