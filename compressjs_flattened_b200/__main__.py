@@ -3,6 +3,7 @@
 
   python -m compressjs_flattened_b200 -d|-z [-1 .. -9] [-b <bits>] [-t bzip2] [infile] [outfile]
   python -m compressjs_flattened_b200 -z [-1 .. -9] --index-out FILE [infile] [outfile]
+  python -m compressjs_flattened_b200 -z --append FILE [--index FILE] [--index-out FILE] [infile]
   python -m compressjs_flattened_b200 -d --list [--multistream] [infile]
   python -m compressjs_flattened_b200 -d --range START:LEN [--index FILE] [--multistream] [infile] [outfile]
   python -m compressjs_flattened_b200 -d --line-index [--multistream] [infile]
@@ -13,6 +14,11 @@
   -z  compress (the default), stream flavour: the input is read piece by piece (bz2b200_zstream_*), level 7 by default
   --index-out FILE  with -z: also write the line index of the stream being written (the --line-index text) to FILE, built
       while compressing, with no decode; --range and --lines take it as --index.  The stream itself is unchanged
+  --append FILE  with -z: append infile (or stdin) to the bzip2 file FILE in place, recompressing only the last block of its
+      last stream (Bzip2Engine.append): FILE then holds what compressing the old and the new bytes together gives, at FILE's
+      level.  --index takes FILE's line index (--line-index or --index-out output; without it one is built first, a full
+      decode), --index-out writes the new one (it may be the same file).  The new tail is written to a temporary file next to
+      FILE first; FILE is changed only once that has succeeded, so an error leaves it as it was
   -d  decompress the FIRST stream of the input, stream flavour (bz2b200_dstream_*); --multistream decodes all of them
       (an extension: the reference's command line never passes the flag, NPM/bin/compressjs:166)
   -b  with -d: extract the single block whose signature starts at bit <bits> (Bzip2.decompressBlock)
@@ -36,9 +42,31 @@
 Usage errors (flags that contradict each other) exit with status 1.
 If <infile> is omitted, reads from stdin; if <outfile> is omitted, writes to stdout.  Needs a CUDA device: no CPU fallback."""
 import argparse
+import os
+import shutil
 import sys
+import tempfile
 
 from .bzip2 import MATCH_FIRST_IN_LINE, NO_SIGNATURE, Bzip2Index, Bzip2LineIndex, Err
+
+
+def _append_in_place(engine, path, src, index, chunk_bytes):
+    """engine.append of src to the file at `path`: the tail goes to a temporary file next to it, and only once the append
+    has succeeded is the file overwritten from `keep`, truncated and synced.  Returns the new line index."""
+    fd, tmp = tempfile.mkstemp(prefix=".append-", dir=os.path.dirname(os.path.abspath(path)))
+    try:
+        with os.fdopen(fd, "w+b") as t:
+            keep, _, index = engine.append(path, src, index, sink=t, chunk_bytes=chunk_bytes)
+            t.seek(0)
+            with open(path, "r+b") as fh:
+                fh.seek(keep)
+                shutil.copyfileobj(t, fh, 1 << 20)
+                fh.truncate()
+                fh.flush()
+                os.fsync(fh.fileno())
+    finally:
+        os.unlink(tmp)
+    return index
 
 
 def main(argv=None, engine=None):
@@ -61,6 +89,7 @@ def main(argv=None, engine=None):
     ap.add_argument("--index", default=None, metavar="FILE",
                     help="with --range: the block index (--list output) or a line index; with --lines: the line index")
     ap.add_argument("--index-out", default=None, metavar="FILE", help="with -z: write the line index of the stream to FILE")
+    ap.add_argument("--append", default=None, metavar="FILE", help="with -z: append the input to the bzip2 file FILE in place")
     ap.add_argument("--line-index", action="store_true", help="with -d: print the line index")
     ap.add_argument("--lines", default=None, metavar="FIRST:COUNT", help="with -d: write COUNT lines from line FIRST (1-based)")
     ap.add_argument("--grep", action="append", default=None, metavar="PATTERN", help="with -d: write the lines that contain PATTERN")
@@ -68,12 +97,22 @@ def main(argv=None, engine=None):
     ap.add_argument("--line-number", action="store_true", help="with --grep: prefix each line with its 1-based number and ':'")
     ap.add_argument("--count", action="store_true", help="with --grep: print the number of matching lines")
     a = ap.parse_args(argv)
-    if a.index_out is not None:
-        for flag, on in (("-d", a.decompress), ("--list", a.list), ("--range", a.range is not None), ("--grep", bool(a.grep)),
-                         ("--line-index", a.line_index), ("--lines", a.lines is not None), ("--recover", a.recover), ("-b", a.block >= 0)):
+    not_z = (("-d", a.decompress), ("--list", a.list), ("--range", a.range is not None), ("--grep", bool(a.grep)),
+             ("--line-index", a.line_index), ("--lines", a.lines is not None), ("--recover", a.recover), ("-b", a.block >= 0))
+    for opt in ("--append", "--index-out"):
+        if getattr(a, opt[2:].replace("-", "_")) is None:
+            continue
+        for flag, on in not_z:
             if on:
-                print(f"--index-out can only be used with -z, not with {flag}", file=sys.stderr)
+                print(f"{opt} can only be used with -z, not with {flag}", file=sys.stderr)
                 return 1
+    if a.append is not None:
+        if any(getattr(a, f"l{lv}") for lv in range(1, 10)):
+            print("--append keeps the level of the file it appends to: a compression level has no effect", file=sys.stderr)
+            return 1
+        if a.outfile is not None:
+            print("--append changes FILE in place and takes no outfile", file=sys.stderr)
+            return 1
     for flag, on in (("--ignore-case", a.ignore_case), ("--line-number", a.line_number), ("--count", a.count)):
         if on and not a.grep:
             print(f"{flag} can only be used with --grep", file=sys.stderr)
@@ -100,7 +139,7 @@ def main(argv=None, engine=None):
     if len(chosen) > 1:
         print(f"{chosen[0]} and {chosen[1]} can't be used together", file=sys.stderr)
         return 1
-    if a.index is not None and a.range is None and a.lines is None:
+    if a.index is not None and a.range is None and a.lines is None and a.append is None:
         print("--index can only be used with --range", file=sys.stderr)
         return 1
     if a.range is not None:
@@ -206,6 +245,19 @@ def main(argv=None, engine=None):
             dst.write(Bzip2.decompressBlock(src.read(), a.block))
         elif a.decompress:
             Bzip2.decompressStream(src, dst, a.multistream)
+        elif a.append is not None:
+            index = None
+            if a.index is not None:
+                with open(a.index) as fh:
+                    text = fh.read()
+                if text.startswith(Bzip2Index.HEADER):
+                    print(f"--append needs a line index (--line-index or --index-out output), and {a.index} is a block index", file=sys.stderr)
+                    return 1
+                index = Bzip2LineIndex.from_text(text)
+            index = _append_in_place(Bzip2, a.append, src, index, a.chunk_mb << 20)
+            if a.index_out is not None:
+                with open(a.index_out, "w") as fh:
+                    fh.write(index.to_text())
         elif a.index_out is not None:
             _, index = Bzip2.compressStream(src, dst, level, chunk_bytes=a.chunk_mb << 20, index=True)
             with open(a.index_out, "w") as fh:

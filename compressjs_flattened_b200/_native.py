@@ -113,6 +113,8 @@ class Library:
         L.bz2b200_pool_compress_indexed.argtypes = [vp, vp, C.c_size_t, C.c_int, C.c_size_t, u8pp, szp] + ixp
         L.bz2b200_zstream_open_indexed.argtypes = [vp, C.c_int, C.c_size_t, C.POINTER(vp)]
         L.bz2b200_zstream_index.argtypes = [vp] + ixp
+        L.bz2b200_zstream_open_append.argtypes = [vp, vp, C.c_size_t, vp, vp, C.c_size_t, C.c_uint64, C.c_size_t, C.POINTER(vp),
+                                                  C.POINTER(C.c_uint64)]
         L.bz2b200_search.argtypes = [vp, vp, C.c_size_t, C.c_int, vp, vp, C.c_size_t, C.c_uint, C.c_uint64, C.POINTER(C.POINTER(Match)), szp,
                                      C.POINTER(SearchTotals), u8pp, szp]
         L.bz2b200_free.argtypes = [vp]

@@ -8,6 +8,7 @@
 Random access (no counterpart in the reference): Bzip2Engine.index, decompressRanges, decompressRange and open.
 Lines by number (no counterpart in the reference): Bzip2Engine.lineIndex, decompressLines and lineSpans.
 The same line index while compressing, with no decode: Bzip2Engine.compressIndexed and compressStream(..., index=True).
+Appending to a stream and its line index, recompressing only the last block: Bzip2Engine.append.
 Search (bzgrep -F, no counterpart in the reference): Bzip2Engine.search.
 
 Same names, argument meaning and error behaviour as the JavaScript API; the work is done by
@@ -320,6 +321,15 @@ def _coerce_input(inp):
     return np.asarray(list(inp), dtype=np.uint8)
 
 
+def _map_path(input):
+    """a path -> the file's bytes, memory-mapped read-only (b"" for an empty file); anything else as it is"""
+    if isinstance(input, (str, os.PathLike)):
+        with builtins.open(input, "rb") as fh:
+            size = os.fstat(fh.fileno()).st_size
+            return np.frombuffer(mmap.mmap(fh.fileno(), 0, access=mmap.ACCESS_READ), dtype=np.uint8) if size else b""
+    return input
+
+
 def _deliver(data, output):
     """Util.coerceOutputStream + BufferStream.getBuffer (BJ:222-272)."""
     if output is None or output is False:
@@ -482,6 +492,30 @@ class Bzip2Engine:
         finished = (lambda handle: _line_index_call(self, self._L.bz2b200_zstream_index, handle)) if index else None
         return self._pump("zstream", h, source, sink, int(piece_bytes or max(1, chunk_bytes // 4)), finished)
 
+    def append(self, stream, source, index=None, sink=None, chunk_bytes=64 << 20, piece_bytes=None):
+        """Append the bytes of `source` to the last stream of `stream`, recompressing only its last block: returns (keep,
+        tail, Bzip2LineIndex).  The new stream is stream[:keep] + tail; for a stream written from input A (by this library
+        or the reference) it is byte for byte compressFile(A + B) at the stream's level, and the index is that of the new
+        stream (include/bz2b200.h, bz2b200_zstream_open_append).  stream: bytes-like, or a path, which is memory-mapped as
+        open() maps it; only its last block and footer are read.  source: what compressStream takes.  sink: as for
+        compressStream, the tail goes there and the sink is returned in its place.  index: the Bzip2LineIndex of `stream`
+        (compressIndexed, compressStream(..., index=True), lineIndex or a previous append); without it one is built first
+        with lineIndex(stream, multistream=True): that is a full decode of the stream."""
+        if isinstance(index, Bzip2Index):
+            raise TypeError("append needs a line index (Bzip2LineIndex: compressIndexed, lineIndex), not a block index")
+        a = _coerce_input(_map_path(stream))
+        if index is None:
+            index = self.lineIndex(a, multistream=True)
+        ix = index.blocks.entries
+        h, keep = C.c_void_p(), C.c_uint64()
+        rc = self._L.bz2b200_zstream_open_append(self._ctx, a.ctypes.data, a.size, ix.ctypes.data, index.newlines.ctypes.data, len(ix),
+                                                 index.total_lines, int(chunk_bytes), C.byref(h), C.byref(keep))
+        if rc:
+            self._raise(rc)
+        finished = lambda handle: _line_index_call(self, self._L.bz2b200_zstream_index, handle)  # noqa: E731
+        tail, li = self._pump("zstream", h, source, sink, int(piece_bytes or max(1, chunk_bytes // 4)), finished)
+        return keep.value, tail, li
+
     def decompressStream(self, source, sink=None, multistream=False, chunk_bytes=16 << 20, piece_bytes=None):
         """Stream flavour of decompressFile: blocks are decoded as soon as they are complete; the bytes of the blocks before
         an error have been delivered when it is raised (like the reference, which writes as it goes)."""
@@ -583,11 +617,7 @@ class Bzip2Engine:
         memory-mapped).  Every read decodes only the blocks it needs.  index: a Bzip2Index or a Bzip2LineIndex (what
         compressIndexed returns); without it one is built first: that is a full decode of the input.  The buffer holds one level-9 block, so small sequential reads do not decode a block each;
         read() to the end is one call."""
-        if isinstance(input, (str, os.PathLike)):
-            with builtins.open(input, "rb") as fh:
-                size = os.fstat(fh.fileno()).st_size
-                input = np.frombuffer(mmap.mmap(fh.fileno(), 0, access=mmap.ACCESS_READ), dtype=np.uint8) if size else b""
-        a = _coerce_input(input)
+        a = _coerce_input(_map_path(input))
         if index is None:
             index = self.index(a, multistream)
         elif isinstance(index, Bzip2LineIndex):

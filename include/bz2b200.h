@@ -366,6 +366,25 @@ int bz2b200_zstream_open(bz2b200_ctx *ctx, int level, size_t chunk_bytes, bz2b20
 /* a zstream that also builds the stream's line index; bz2b200_zstream_index after finish (see bz2b200_compress_indexed) */
 int bz2b200_zstream_open_indexed(bz2b200_ctx *ctx, int level, size_t chunk_bytes, bz2b200_zstream **zs);
 int bz2b200_zstream_index(bz2b200_zstream *zs, bz2b200_block_entry **entries, uint32_t **newlines, size_t *count, uint64_t *total_lines);
+/* Appending to a stream and its line index, without recompressing it.  Opens an indexed zstream that continues the LAST
+ * stream of `in` (n bytes: caller-owned, only read, may be a memory map) whose line index is index / newlines / count /
+ * total_lines (what bz2b200_compress_indexed, bz2b200_zstream_index or bz2b200_line_index return).  The new bytes then go
+ * through bz2b200_zstream_feed and bz2b200_zstream_finish; the stream to keep is in[0, *keep) followed by every byte they
+ * return, and bz2b200_zstream_index returns the line index of that whole stream.  For a stream the reference (or this
+ * library) wrote from input A, appending B gives byte for byte bz2b200_compress(A + B) at the stream's level: every block
+ * before the last keeps its bits, and the last block L is decoded and compressed again together with B (DESIGN.md
+ * section 8, "Appending").  Any valid stream can be continued (one from libbz2 too); the result then decodes to A + B.  The call reads
+ * only L's bytes, the footer after it and the byte at *keep = L.bit_begin / 8 (its bits before L are carried over).  Rows
+ * the append writes carry L's stream and level.  Checks, before anything is returned: the index passes the checks of
+ * bz2b200_decompress_lines (BZ2B200_E_ARG); the end-of-stream magic sits at L.bit_end and the stream CRC after it equals
+ * the fold of the stored CRCs of L's stream's entries, L decodes (the verdicts of bz2b200_decompress_ranges) to
+ * newlines[count - 1] '\n' bytes and ends as total_lines says (DATA_ERROR "index does not match the input" otherwise);
+ * the stream ends the input, (L.bit_end + 87) / 8 == n (BZ2B200_E_ARG otherwise: the bytes after it, another stream or
+ * trailing data, would be dropped).  count == 0 is accepted only for one empty stream (14 bytes; *keep = 4).  Blocks
+ * before L are neither read nor checked, as range reads do not check the blocks they do not decode.  newlines is required.
+ * bz2b200_last_stats after the call describes the decode of L, as bz2b200_decompress_lines would.  On error *zs is NULL. */
+int bz2b200_zstream_open_append(bz2b200_ctx *ctx, const uint8_t *in, size_t n, const bz2b200_block_entry *index, const uint32_t *newlines, size_t count,
+                                uint64_t total_lines, size_t chunk_bytes, bz2b200_zstream **zs, uint64_t *keep);
 int bz2b200_zstream_feed(bz2b200_zstream *zs, const uint8_t *in, size_t n, uint8_t **out, size_t *out_len);
 int bz2b200_zstream_finish(bz2b200_zstream *zs, uint8_t **out, size_t *out_len);
 void bz2b200_zstream_close(bz2b200_zstream *zs);
