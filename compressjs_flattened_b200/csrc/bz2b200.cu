@@ -140,7 +140,7 @@ struct Ctx {
   // decode-side buffers
   DevBuf d_in, cand, ncand, dmeta, dsyms, dL, dtt, dwalk, dblk, dout, dmisc, dsel, doff, dperm, dmap;
   DevBuf dpieces, dgather;  // range reads: the pieces and the packed bytes (search: the lines)
-  DevBuf dspat, dstile, dsbase, dstsum, dsmatch, dspart, dstot;  // search: patterns and filter, per-tile and per-thread summaries, matches
+  DevBuf dspat, dstile, dstsum, dsmatch, dspart, dstot;  // search: patterns and filter, per-tile and per-thread summaries (then the tiles' bases), matches
   DevBuf dnltile, dnlpart, dnlq;  // newline directory: tile counts then their prefix, scan partials, queries and their results
   DevBuf ixtab;  // indexed compress: a bz2b200_block_entry row per block of the call, then the blocks' '\n' counts (u32)
   // last compress, for debug_fetch
@@ -194,7 +194,7 @@ struct Ctx {
                      &gbounds, &key2, &big_cnt, &big_old, &big_rank, &big_tile0, &big_tblk, &totals2,
                      &recs_cand, &cand_first, &out2, &blksort, &r2_status, &hfreq, &hlens, &hplen, &hcodes, &hsel, &hcost, &hgoff, &hblk,
                      &d_in, &cand, &ncand, &dmeta, &dsyms, &dL, &dtt, &dwalk, &dblk, &dout, &dmisc, &dsel, &doff, &dperm, &dmap,
-                     &dpieces, &dgather, &dspat, &dstile, &dsbase, &dstsum, &dsmatch, &dspart, &dstot, &dnltile, &dnlpart, &dnlq, &ixtab};
+                     &dpieces, &dgather, &dspat, &dstile, &dstsum, &dsmatch, &dspart, &dstot, &dnltile, &dnlpart, &dnlq, &ixtab};
     for (DevBuf *b : all) pool.push_back(b);
   }
 };
